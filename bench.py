@@ -25,7 +25,7 @@ The same line also carries, at every N (strong scaling: the total work is fixed,
 and, for N > 1, `gather` (the weak-scaled terrain built into rank 0's buffer, checked against a local
 build), plus `single_polygon_us` (N = 1): Polygon.create_polygon's own call shape.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 """
 from __future__ import annotations
 
@@ -243,6 +243,56 @@ def run_reference_arm(args):
     emit(line)
 
 
+DUMP_SEED = 0x5EED00D0
+# sample sizes of --dump-outputs (rows of each buffer), divided among the ranks: at most 52 MiB of .npy in all
+DUMP_VERTICES, DUMP_QUADS, DUMP_TRIANGLES, DUMP_POLYGONS = 1 << 19, 1 << 18, 1 << 18, 1 << 17
+
+
+def dump_sample(count: int, k: int, *key) -> np.ndarray:
+    """Sorted ids of k of the `count` rows (all of them when k >= count); fixed by DUMP_SEED and `key`."""
+    if k >= count:
+        return np.arange(count, dtype=np.int64)
+    return np.sort(np.random.default_rng([DUMP_SEED, *key]).choice(count, size=k, replace=False))
+
+
+def dump_outputs(out_dir, rank, world, rows, qrows, n, vtx, idx, tlayout, ptri_base, pvtx, pbbox, pstat, pntri, player,
+                 poly_base):
+    """Writes what one step of the timed path produced, as a caller receives it, to out_dir/<name>.npy
+    (<name>.rank<r>.npy at N > 1): the terrain's vertex attributes and index buffer, the polygon batch's vertex
+    attributes, bounding boxes, status words and triangle counts.  Buffers with more rows than the sample size are
+    represented by a seeded sample of their rows; `*_ids` holds the global row numbers of what was kept (a
+    terrain vertex is row-major r * n + c, a terrain quad r * (n - 1) + c with 6 indices each)."""
+    import torch
+
+    def rows_of(buf, dtype, width, ids):
+        return buf.view(dtype).view(-1, width)[torch.from_numpy(ids).to(buf.device)].cpu().numpy()
+
+    def attribute_columns(layout):  # the float components of every attribute, in attribute order
+        return [off // 4 + c for off, ncomp in layout.attributes for c in range(ncomp)]
+
+    out = {}
+    (r0, r1), (q0, q1) = rows, qrows
+    vids = dump_sample((r1 - r0) * n, DUMP_VERTICES // world, rank, 0)
+    out["terrain_vertex_ids"] = (r0 * n + vids).astype(np.float64)
+    out["terrain_vertices"] = rows_of(vtx, torch.float32, tlayout.stride // 4, vids)[:, attribute_columns(tlayout)]
+    qids = dump_sample((q1 - q0) * (n - 1), DUMP_QUADS // world, rank, 1)
+    out["terrain_quad_ids"] = (q0 * (n - 1) + qids).astype(np.float64)
+    out["terrain_indices"] = rows_of(idx[:(q1 - q0) * 6 * (n - 1)], torch.int32, 6, qids).view(np.uint32).astype(np.float64)
+    tids = dump_sample(pvtx.numel() // (3 * player.stride), DUMP_TRIANGLES // world, rank, 2)
+    out["polygon_triangle_ids"] = (ptri_base + tids).astype(np.float64)
+    tri = rows_of(pvtx, torch.float32, 3 * player.stride // 4, tids).reshape(-1, 3, player.stride // 4)
+    out["polygon_vertices"] = tri[:, :, attribute_columns(player)]
+    pids = dump_sample(pstat.numel(), DUMP_POLYGONS // world, rank, 3)
+    out["polygon_ids"] = (poly_base + pids).astype(np.float64)
+    out["polygon_bbox"] = rows_of(pbbox, torch.float32, 4, pids)
+    out["polygon_status"] = rows_of(pstat, torch.int32, 1, pids).view(np.uint32)[:, 0].astype(np.float64)
+    out["polygon_ntri"] = rows_of(pntri, torch.int32, 1, pids).view(np.uint32)[:, 0].astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = "" if world == 1 else f".rank{rank}"
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), np.ascontiguousarray(a))
+
+
 _STDOUT_FD = None
 
 
@@ -267,7 +317,12 @@ def main():
     ap.add_argument("--no-gather", action="store_true", help="N>1: skip the NVLink gather legs (they are on by default)")
     ap.add_argument("--no-configs45", action="store_true", help="skip the BASELINE config 4 / config 5 legs")
     ap.add_argument("--gather", action="store_true", help="(accepted for compatibility: the gather is on by default)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (a seeded sample "
+                         "of the large buffers, 52 MiB at most) so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     # stdout carries exactly one JSON line: anything a library prints there (NCCL's version banner, ...) goes to stderr
     global _STDOUT_FD
@@ -453,6 +508,10 @@ def main():
     ok_star = int((pstat == 0).sum().item())
     tiers = (C.c_uint32 * 8)()
     lib.mr_triangulate_tier_counts(ctx.handle, tiers)  # how the star batch was spread over the arena tiers
+    if args.dump_outputs:  # before the convex batch below reuses the polygon output buffers
+        ptri_base = int(mr.polygon_offsets_host(fp_all[:pa + 1])[-1])
+        dump_outputs(args.dump_outputs, rank, world, (r0, r1), (q0, q1), n, vtx, idx, T.layout, ptri_base, pvtx, pbbox,
+                     pstat, pntri, P.layout, pa)
 
     # ---- convex batch, same protocol -----------------------------------------------------------------
     for _ in range(2):

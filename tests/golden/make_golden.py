@@ -2,6 +2,9 @@
 
   heightmap_100.npy       u16[100][100] decoded from the reference's App/HEIGHTMAP.png
                           (sha256 of the PNG checked against SURVEY 4); a data fixture, not source
+  heightmap_100.png       the same pixels as a 16-bit grayscale PNG written by write_png_u16 below (not by the
+                          loader's library), the input of the PNG loader's test; `make_golden.py png` rewrites it
+                          from the committed heightmap_100.npy alone
   app_polygons.json       the two literal polygons of App/App.zig:68-83 (f32 values)
   kat.json                oracle outputs (known-answer vectors):
       polygon2 / linear order  -> the hand-derived answer of SURVEY 8-a
@@ -11,7 +14,9 @@
 import hashlib
 import json
 import os
+import struct
 import sys
+import zlib
 
 import numpy as np
 
@@ -27,6 +32,23 @@ POLYGON1 = [[62.742857, 106.97143], [93.085712, 65.828571], [147.08571, 85.62857
 POLYGON2 = [[10.0, 10.0], [40.0, 10.0], [40.0, 40.0], [10.0, 40.0]]
 
 
+def write_png_u16(path, a):
+    """Minimal PNG writer: 16-bit grayscale, no interlace, filter type 0 on every row, one IDAT chunk."""
+    h, w = a.shape
+    raw = b"".join(b"\x00" + np.ascontiguousarray(a[r], dtype=">u2").tobytes() for r in range(h))
+
+    def chunk(tag, data):
+        return struct.pack(">I", len(data)) + tag + data + struct.pack(">I", zlib.crc32(tag + data))
+
+    with open(path, "wb") as f:
+        f.write(b"\x89PNG\r\n\x1a\n" + chunk(b"IHDR", struct.pack(">IIBBBBB", w, h, 16, 0, 0, 0, 0))
+                + chunk(b"IDAT", zlib.compress(raw, 9)) + chunk(b"IEND", b""))
+
+
+def write_heightmap_png():
+    write_png_u16(os.path.join(HERE, "heightmap_100.png"), np.load(os.path.join(HERE, "heightmap_100.npy")))
+
+
 def main():
     from PIL import Image
 
@@ -35,6 +57,7 @@ def main():
     h = np.ascontiguousarray(np.asarray(Image.open(png)).astype(np.uint16))
     assert h.shape == (100, 100)
     np.save(os.path.join(HERE, "heightmap_100.npy"), h)
+    write_heightmap_png()
     json.dump({"polygon1": POLYGON1, "polygon2": POLYGON2}, open(os.path.join(HERE, "app_polygons.json"), "w"))
 
     kat = {}
@@ -67,4 +90,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    write_heightmap_png() if sys.argv[1:] == ["png"] else main()

@@ -4,6 +4,7 @@ import ctypes as C
 import os
 import re
 import subprocess
+import sys
 import tempfile
 
 import numpy as np
@@ -63,23 +64,36 @@ int main(void){
     assert vals[10:] == [8 * 64 + 64, 16 * 64 + 64]
 
 
-def test_no_cpu_fallback(lib):
-    import torch
+_NO_DEVICE_CHECKS = r'''
+import ctypes as C
+import sys
 
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    import myrenderer_b200 as mr
+sys.path.insert(0, sys.argv[1])
+import myrenderer_b200 as mr
+from myrenderer_b200._capi import MrTerrainJob
 
-    h = C.c_void_p()
-    assert lib.mr_context_create(0, C.byref(h)) == -2 and not h.value  # MR_E_CUDA
-    with pytest.raises(mr.MrError):
-        mr.Context(0)
-    n = C.c_int(-1)
-    assert lib.mr_device_count(C.byref(n)) in (0, -2) and n.value == 0
-    # null context is rejected, not dereferenced
-    from myrenderer_b200._capi import MrTerrainJob
+lib = mr.load()
+h = C.c_void_p()
+assert lib.mr_context_create(0, C.byref(h)) == -2 and not h.value  # MR_E_CUDA
+try:
+    mr.Context(0)
+    raise SystemExit("mr.Context(0) did not raise MrError")
+except mr.MrError:
+    pass
+n = C.c_int(-1)
+assert lib.mr_device_count(C.byref(n)) in (0, -2) and n.value == 0
+# null context is rejected, not dereferenced
+assert lib.mr_terrain_build(None, C.byref(MrTerrainJob())) == -1
+print("no-device checks ok")
+'''
 
-    assert lib.mr_terrain_build(None, C.byref(MrTerrainJob())) == -1
+
+def test_no_cpu_fallback():
+    """No device visible (none installed, or all hidden through CUDA_VISIBLE_DEVICES): every entry point fails with an
+    error code, nothing computes on the CPU.  Runs in a child process so that the devices can be hidden from it."""
+    r = subprocess.run([sys.executable, "-c", _NO_DEVICE_CHECKS, ROOT], capture_output=True, text=True, timeout=300,
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert r.returncode == 0 and "no-device checks ok" in r.stdout, r.stdout[-2000:] + r.stderr[-2000:]
 
 
 def test_layout_presets_and_describe(lib):
