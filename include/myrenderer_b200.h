@@ -146,7 +146,8 @@ int mr_fill_zero(mr_context* ctx, void* dev, size_t bytes);
  * Grid mesh of an n x n heightmap.
  *   height texel (r,c), row-major r*n+c:
  *       MR_HEIGHT_U16: raw PNG grayscale16 value v; h = 1.0f - (float)v / 65535.0f   (Terrain.zig:120)
- *       MR_HEIGHT_F32: h itself
+ *       MR_HEIGHT_F32: h itself.  Any float: NaN, +-inf, +-0 and subnormals are computed with IEEE
+ *                      semantics, with no flush to zero of inputs or results.
  *   position(r,c) = ( grid_step*(float)r - origin_scale*(float)n,
  *                     height_scale*h,
  *                     grid_step*(float)c - origin_scale*(float)n )                  (Terrain.zig:24-48, indexed form)
@@ -158,6 +159,10 @@ int mr_fill_zero(mr_context* ctx, void* dev, size_t bytes);
  *       len = sqrtf(((gx*gx)+1.0f)+(gz*gz));  inv = 1.0f/len;  normal = (-gx*inv, inv, -gz*inv)
  *     IEEE round-to-nearest for every operation, no FMA; n==1 gives gx=gz=0.  (One reciprocal and
  *     two products instead of three quotients: at most 1 ulp from the quotient form.)
+ *   NaN outputs (of the mesh, the tile boxes and anything else this header calls bit-exact): where an
+ *     output float is NaN, its sign and payload are unspecified (the GPU writes a canonical NaN, a CPU
+ *     may carry an input's payload).  Every other output, signed zeros and infinities included, is
+ *     bit-exact as specified.
  *   indices [NEW SPEC]: u32, 6 per quad, quads (r,c) r,c in [0,n-1) row-major, corner order of
  *       Terrain.zig:28-35 under cw front faces (Pipeline.zig:145-149):
  *       (r+1,c) (r,c) (r+1,c+1) (r+1,c+1) (r,c) (r,c+1)   with i(r,c)=r*n+c
@@ -224,7 +229,9 @@ int mr_heightmap_normalize(mr_context* ctx, const uint16_t* in, uint64_t count, 
  * over the tile's vertices, positions as defined for mr_terrain_build (x from the row, z from the
  * column, y = height_scale * h).  min/max are exact (comparisons only), so the boxes are bit-exact;
  * a y bound that is zero is written as +0.0f (with height_scale == 0, or a float map holding both
- * zeros, the sign of a zero bound would otherwise depend on the order of the reduction).
+ * zeros, the sign of a zero bound would otherwise depend on the order of the reduction).  NaN heights
+ * are skipped by the min/max; a tile of NaNs only has min +inf and max -inf, so its y bounds are
+ * height_scale*(+-inf) in order (-inf, +inf at height_scale 5; NaN at height_scale 0).
  *
  * mr_terrain_cull applies the reference's visibility test (SceneNode.zig:96-110) to every tile box:
  *     q0 = M * p0 unless some component of p0 is -inf;  q1 = M * p1 unless some component of p1 is +inf
@@ -233,6 +240,9 @@ int mr_heightmap_normalize(mr_context* ctx, const uint16_t* in, uint64_t count, 
  * xform[4*col + row]) and M * p evaluated like mach's Mat4x4.mulVec: result[i] starts at 0 and adds
  * xform[4*j + i] * p[j] for j = 0..3 in order, every operation separately rounded.  (mach is not
  * vendored in the reference tree: mulVec is restated from the mach source -- parity unpinned.)
+ * bbox may hold any floats.  "Some component is -inf" is fminf over the four components == -inf (and
+ * fmaxf == +inf for p1), so the skip rule ignores NaN components; a NaN that reaches a comparison makes
+ * it false.  Subnormal inputs and products are not flushed to zero.
  * Outputs, each optional (NULL to skip), device or host pointers:
  *     visible_out[t]      1 / 0 per tile
  *     visible_ids_out[k]  the visible tiles in ascending order, k < counts_out[0]

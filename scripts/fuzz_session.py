@@ -1,8 +1,8 @@
-"""Session fuzz: ONE context, a long random sequence of calls -- terrain builds, tile boxes, culls, polygon batches of
-every shape, deliberately invalid calls (which must fail with an error code and leave the context usable), scratch
-trims and tier-count queries in between -- every result compared with the CPU oracle.  Looks for state that leaks
-from one call into the next (scratch growth and trim, the cached launch plan, side streams, staging buffers).
-Test infrastructure: the oracle is the checker.
+"""Session fuzz: ONE context, a long random sequence of calls -- terrain builds (on the heights of fuzz_terrain, NaN and
+infinite texels among them), tile boxes, culls, polygon batches of every shape, deliberately invalid calls (which must
+fail with an error code and leave the context usable), scratch trims and tier-count queries in between -- every result
+compared with the CPU oracle.  Looks for state that leaks from one call into the next (scratch growth and trim, the
+cached launch plan, side streams, staging buffers).  Test infrastructure: the oracle is the checker.
 
     python scripts/fuzz_session.py --steps 400 --seed 1 --out gpurun_out/fuzz_session.json     # on a GPU box
 
@@ -22,6 +22,7 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 sys.path.insert(0, os.path.join(ROOT, "scripts"))
+import _float_edges as E  # noqa: E402
 
 
 def main():
@@ -69,7 +70,8 @@ def main():
                 vbytes, icount = n * n * lay_t[0], 6 * max(n - 1, 0) ** 2
                 gv, gi = FT.run_build(ctx, t, torch, h, n, host, 0, n, 0, max(n - 1, 0), 0, n, 0, 0, vbytes, icount)
                 ovtx, oidx = orc.terrain_build(h, n, layout=lay_t, params=params, nthreads=0)
-                if not np.array_equal(gv[:vbytes], ovtx) or (icount and not np.array_equal(gi[:icount], oidx)):
+                vbad = vbytes and E.float_mismatch(gv[:vbytes], ovtx, E.vertex_float_mask(vbytes, lay_t)) is not None
+                if vbad or (icount and not np.array_equal(gi[:icount], oidx)):
                     fail(step, "terrain n=%d differs" % n)
                 counts["terrain"] += 1
             elif kind == "polygons":

@@ -1,8 +1,11 @@
 """Terrain fuzz: mr_terrain_build / mr_terrain_tile_bounds / mr_terrain_cull through the C ABI vs the CPU oracle, byte
 for byte, on drawn cases -- sizes 1..1600 (odd, even, multiples of 8 and of 256), u16 and f32 heights (noise, constant,
-extremes, steps), terrain parameters (the reference's constants, other grid steps, negative and zero scales), vertex
-layouts (strides 12..64, position / normal at any 4-byte offset, with and without a normal), row bands written into
-larger buffers, device and host pointers, tilings and cull matrices.  Test infrastructure: the oracle is the checker.
+extremes, steps, maps of NaN / +-inf / +-0 / subnormal / +-FLT_MAX texels), terrain parameters (the reference's
+constants, other grid steps, negative and zero scales), vertex layouts (strides 12..64, position / normal at any 4-byte
+offset, with and without a normal), row bands written into larger buffers, device and host pointers, tilings, cull
+matrices, and the near-threshold and non-finite cull boxes of tests/_float_edges.py.  Any two NaN floats compare equal
+(the header leaves a NaN's sign and payload unspecified); every other word, padding included, must be bit-equal.  Test
+infrastructure: the oracle is the checker.
 
     python scripts/fuzz_terrain.py --rounds 300 --seed 1 --out gpurun_out/fuzz_terrain.json     # on a GPU box
 
@@ -21,6 +24,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 sys.path.insert(0, os.path.join(ROOT, "tests"))
+import _float_edges as E  # noqa: E402
 
 
 def draw_n(rng):
@@ -39,7 +43,9 @@ def draw_n(rng):
 
 
 def draw_height(rng, orc, n):
-    k = int(rng.integers(0, 7))
+    k = int(rng.integers(0, 8))
+    if k == 7:
+        return E.special_heightmap(rng, n, ((int(rng.choice([1, 8, 33])), int(rng.choice([2, 24, 600]))),))
     if k <= 2:
         return orc.synth_heightmap_u16(int(rng.integers(1, 2 ** 62)), n)
     if k == 3:
@@ -120,6 +126,7 @@ def main():
     import myrenderer_b200 as mr
     from test_terrain_cull_cpu import camera_matrix, mat_image
 
+    edge_cases = E.cull_cases(seed=a.seed)
     ctx = mr.Context(0)
     lib = ctx.lib
     rng = np.random.default_rng(a.seed)
@@ -183,7 +190,8 @@ def main():
             continue
         if not np.array_equal(gi, want_i):
             fail(desc, "index buffer (or the words around the band) differs")
-        if not np.array_equal(gv, want_v):
+        if (E.float_mismatch(gv, want_v, E.vertex_float_mask(vbytes, lay_t)) is not None if vbytes
+                else not np.array_equal(gv, want_v)):
             fail(desc, "vertex bytes (or the bytes around the band) differ")
         totals["vertices"] += (re - rb) * n
         totals["indices"] += oidx.size
@@ -198,12 +206,12 @@ def main():
             ctx.check(lib.mr_terrain_tile_bounds(ctx.handle, hd.data_ptr(), 0 if h.dtype == np.uint16 else 1, n, tr, tc, C.byref(t.params),
                                                  box_d.data_ptr()), "tile bounds")
             ctx.sync()
-            if not np.array_equal(box_d.cpu().numpy().view(np.uint32), want_box.reshape(-1).view(np.uint32)):
+            if E.float_mismatch(box_d.cpu().numpy(), want_box) is not None:
                 fail(dict(desc, tile=[tr, tc]), "tile boxes differ")
             totals["tiles"] += ntiles
-            box_d = torch.from_numpy(want_box.reshape(-1)).cuda()  # the cull is checked on the oracle's boxes
             for _ in range(2):
-                k = int(rng.integers(0, 4))
+                k = int(rng.integers(0, 5))
+                boxes = want_box  # the cull is checked on the oracle's boxes
                 if k == 0:
                     m = camera_matrix()
                 elif k == 1:
@@ -211,9 +219,13 @@ def main():
                     m = camera_matrix(eye, tuple(float(x) for x in rng.uniform(-40, 40, 3)))
                 elif k == 2:
                     m = rng.uniform(-1, 1, 16).astype(np.float32)
-                else:
+                elif k == 3:
                     m = mat_image(np.array([[0, 0, 0, 1]] * 4, dtype=np.float32))
-                ref = orc.terrain_cull(want_box, n, tr, tc, m)
+                else:  # boxes near the thresholds of the test, or with +-inf / NaN components, under their matrix
+                    _, m, pool = edge_cases[int(rng.integers(0, len(edge_cases)))]
+                    boxes = pool[rng.integers(0, len(pool), ntiles)]
+                box_d = torch.from_numpy(np.ascontiguousarray(boxes).reshape(-1)).cuda()
+                ref = orc.terrain_cull(boxes, n, tr, tc, m)
                 vis = torch.empty(ntiles, dtype=torch.int32, device="cuda")
                 ids = torch.empty(ntiles, dtype=torch.int32, device="cuda")
                 idx = torch.full((6 * (n - 1) * (n - 1),), -1, dtype=torch.int32, device="cuda")
