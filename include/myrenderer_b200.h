@@ -272,7 +272,14 @@ int mr_terrain_cull(mr_context* ctx, const float* bbox /* tiles * 8 */, uint32_t
  * Edge insertion order (unirand.zig): either explicit per-polygon (offset,prime)
  * pairs, or drawn on the device by the port of unirand_seed from the documented
  * stream  R_k(i) = splitmix64 stream keyed by (seed, poly_index0+i)  -- see mr_rng_u32.
- * Output triangles are bit-identical to the reference's for the same (offset,prime). */
+ * Output triangles are bit-identical to the reference's for the same (offset,prime).
+ * Float semantics, on every path (all size classes, the small-batch path, the general path):
+ *   - coordinates are compared and the side test is evaluated with IEEE f32 semantics, each operation rounded on
+ *     its own, with no flush to zero: subnormal coordinates, differences and products keep their values
+ *   - in the (y, x) order of point_is_above -0 equals +0; two points equal in both coordinates up to the sign of
+ *     zero are coincident
+ *   - finiteness is checked on both coordinates of every point: a NaN or +-inf anywhere gives MR_POLY_NONFINITE
+ *   - a bbox component that is zero is always +0 (the accumulators start at +0 and a tie keeps the accumulator) */
 typedef struct mr_polygon_job {
     const float* xy;
     const uint64_t* first_point; /* npoly+1 entries */

@@ -81,6 +81,39 @@ uint32_t mr_o_tri_create_polygon(mr_o_tri* t, const float* xy, uint32_t n, mr_o_
                                  void* ctx, mr_o_emit_fn emit, mr_o_stats* stats);
 /* Test-only: multiply the contract caps MR_NODE_CAP / MR_STACK_CAP (1 = contract; safety valve 2^27). */
 void mr_o_test_lift_caps(uint32_t multiplier);
+/* Test-only: replace one float rule of the reference by a plausible wrong restatement of it (a "mutant"), so that the
+ * tests can show that their inputs tell the two apart (tests/_poly_float_edges.py).  0 restores the reference rules.
+ * Set it only while no oracle call is running; it applies to every thread. */
+enum {
+    MR_O_MUT_NONE = 0,
+    /* is_left_of, Triangulation.zig:117-126 */
+    MR_O_MUT_SIDE_FMA,       /* fmaf(bx-ax, py-ay, -mul2): mul1 unrounded */
+    MR_O_MUT_SIDE_F64,       /* every operation in double */
+    MR_O_MUT_SIDE_EXACTDIFF, /* f32 differences, exact products and a correctly signed difference in double */
+    MR_O_MUT_SIDE_REFORM,    /* (ax-px)*(by-py) - (ay-py)*(bx-px): same exact sign, other roundings */
+    MR_O_MUT_SIDE_FTZ,       /* inputs, differences, products and result flushed to +-0 when subnormal */
+    MR_O_MUT_SIDE_GE,        /* d >= 0 */
+    /* point_is_above, Triangulation.zig:128-136 */
+    MR_O_MUT_ORDER_RAWZERO,  /* -0 before +0 (the sort key without its zero normalisation) */
+    MR_O_MUT_ORDER_SIGNFLIP, /* key = bits ^ sign bit only: negative coordinates sort backwards */
+    MR_O_MUT_ORDER_DAZ,      /* subnormal coordinates compare as zero */
+    MR_O_MUT_ORDER_TIE_LE,   /* ly == ry && lx <= rx */
+    /* push_triangle_if_acute, Triangulation.zig:398-425 */
+    MR_O_MUT_ACUTE_CR_ATAN2, /* correctly rounded atan2 (double atan2 rounded to f32) */
+    MR_O_MUT_ACUTE_PI_DOWN,  /* compare with 0x40490fda */
+    MR_O_MUT_ACUTE_LE,       /* diff <= pi */
+    MR_O_MUT_ACUTE_ALWAYS,   /* every corner acute */
+    MR_O_MUT_ACUTE_DAZ_ATAN2,/* atan2 arguments and result flushed to +-0 when subnormal */
+    /* render_point bbox, Polygon.zig:73-76 */
+    MR_O_MUT_BBOX_TIE_REPLACES, /* v <= acc ? v : acc (a hardware fminf/fmaxf on +-0) */
+    MR_O_MUT_BBOX_OWN_Y,        /* p1.y / p2.y accumulate their own min / max */
+    /* non-finite rejection */
+    MR_O_MUT_NONFINITE_X_ONLY,  /* only x coordinates are checked */
+    MR_O_MUT_NONFINITE_NAN_ONLY,/* infinities pass */
+    MR_O_MUT_COUNT
+};
+void mr_o_test_mutant(uint32_t id);
+uint32_t mr_o_mutant(void);
 /* Introspection for tests: node arena after the last create_polygon. */
 uint32_t mr_o_tri_node_count(const mr_o_tri* t);
 const mr_o_node* mr_o_tri_nodes(const mr_o_tri* t);

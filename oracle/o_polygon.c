@@ -42,17 +42,23 @@ typedef struct sink { /* RenderContext, Polygon.zig:59-63 */
 } sink;
 
 /* @min/@max for finite floats; ties (+0 vs -0) keep the accumulator */
-static float fmin_acc(float acc, float v) { return v < acc ? v : acc; }
-static float fmax_acc(float acc, float v) { return v > acc ? v : acc; }
+static float fmin_acc(float acc, float v) {
+    if (mr_o_mutant() == MR_O_MUT_BBOX_TIE_REPLACES) return v <= acc ? v : acc;
+    return v < acc ? v : acc;
+}
+static float fmax_acc(float acc, float v) {
+    if (mr_o_mutant() == MR_O_MUT_BBOX_TIE_REPLACES) return v >= acc ? v : acc;
+    return v > acc ? v : acc;
+}
 
 /* render_point, Polygon.zig:65-79 -- including the bbox rule exactly as written:
  * p1.y = min(p1.x, y) and p2.y = max(p2.x, y) use the *x* accumulators. */
 static void render_point(void* vctx, uint32_t id, float x, float y) {
     sink* s = (sink*)vctx;
     s->b1x = fmin_acc(s->b1x, x);
-    s->b1y = fmin_acc(s->b1x, y);
+    s->b1y = fmin_acc(mr_o_mutant() == MR_O_MUT_BBOX_OWN_Y ? s->b1y : s->b1x, y);
     s->b2x = fmax_acc(s->b2x, x);
-    s->b2y = fmax_acc(s->b2x, y);
+    s->b2y = fmax_acc(mr_o_mutant() == MR_O_MUT_BBOX_OWN_Y ? s->b2y : s->b2x, y);
     if (s->len >= s->cap) { /* appendAssumeCapacity past capacity is UB in the reference */
         s->dropped++;
         return;
@@ -108,8 +114,11 @@ static void run_range(work* w) {
         } else if (n > MR_MAX_POLYGON_POINTS) {
             status = MR_POLY_TOO_LARGE;
         } else {
-            for (k = 0; k < 2u * n; ++k)
-                if (!isfinite(xy[k])) status = MR_POLY_NONFINITE;
+            const uint32_t mut = mr_o_mutant();
+            for (k = 0; k < 2u * n; ++k) {
+                if (mut == MR_O_MUT_NONFINITE_X_ONLY && (k & 1u)) continue;
+                if (mut == MR_O_MUT_NONFINITE_NAN_ONLY ? isnan(xy[k]) : !isfinite(xy[k])) status = MR_POLY_NONFINITE;
+            }
         }
         if (status == MR_POLY_OK) {
             mr_o_unirand rng;

@@ -17,6 +17,7 @@
  *   - the contract's resource caps MR_NODE_CAP(n) / MR_STACK_CAP(n) abandon the polygon
  *     with MR_POLY_ARENA (the reference would keep allocating)
  */
+#include <math.h>
 #include <stdlib.h>
 #include <string.h>
 #include "mr_oracle.h"
@@ -55,6 +56,13 @@ static uint32_t lifted(uint32_t cap) {
     const uint64_t v = (uint64_t)cap * g_caps_mult;
     return v > (1u << 27) ? (1u << 27) : (uint32_t)v;
 }
+
+/* Test-only switch (tests/_poly_float_edges.py): one float rule replaced by a wrong restatement; 0 = the reference. */
+static uint32_t g_mutant = MR_O_MUT_NONE;
+void mr_o_test_mutant(uint32_t id) { g_mutant = id < MR_O_MUT_COUNT ? id : MR_O_MUT_NONE; }
+uint32_t mr_o_mutant(void) { return g_mutant; }
+
+static float ftz(float v) { return fpclassify(v) == FP_SUBNORMAL ? copysignf(0.0f, v) : v; }
 
 mr_o_tri* mr_o_tri_new(void) { /* :427-435 */
     return (mr_o_tri*)calloc(1, sizeof(mr_o_tri));
@@ -103,21 +111,70 @@ static uint32_t clone_node(mr_o_tri* t, uint32_t node) { /* :109-115 */
     return id;
 }
 
+static int is_left_of_mutant(const float* p, const float* a, const float* b) {
+    switch (g_mutant) {
+        case MR_O_MUT_SIDE_FMA:
+            return fmaf(b[0] - a[0], p[1] - a[1], -((b[1] - a[1]) * (p[0] - a[0]))) > 0.0f;
+        case MR_O_MUT_SIDE_F64:
+            return ((double)b[0] - a[0]) * ((double)p[1] - a[1]) - ((double)b[1] - a[1]) * ((double)p[0] - a[0]) > 0.0;
+        case MR_O_MUT_SIDE_EXACTDIFF: /* a product of two floats is exact in double; the difference keeps its sign */
+            return (double)(b[0] - a[0]) * (double)(p[1] - a[1]) - (double)(b[1] - a[1]) * (double)(p[0] - a[0]) > 0.0;
+        case MR_O_MUT_SIDE_REFORM:
+            return (a[0] - p[0]) * (b[1] - p[1]) - (a[1] - p[1]) * (b[0] - p[0]) > 0.0f;
+        case MR_O_MUT_SIDE_FTZ: {
+            const float m1 = ftz(ftz(ftz(b[0]) - ftz(a[0])) * ftz(ftz(p[1]) - ftz(a[1])));
+            const float m2 = ftz(ftz(ftz(b[1]) - ftz(a[1])) * ftz(ftz(p[0]) - ftz(a[0])));
+            return ftz(m1 - m2) > 0.0f;
+        }
+        default: /* MR_O_MUT_SIDE_GE */
+            return (b[0] - a[0]) * (p[1] - a[1]) - (b[1] - a[1]) * (p[0] - a[0]) >= 0.0f;
+    }
+}
+
+/* sort key of one coordinate: order-preserving u32, -0 mapped to +0 unless `rawzero`; `signflip` flips the sign bit only */
+static uint32_t order_key(float v, int rawzero, int signflip) {
+    uint32_t u;
+    if (!rawzero && v == 0.0f) v = 0.0f;
+    memcpy(&u, &v, 4);
+    if (signflip) return u ^ 0x80000000u;
+    return u ^ ((u >> 31) ? 0xFFFFFFFFu : 0x80000000u);
+}
+
+static int point_is_above_mutant(float lx, float ly, float rx, float ry) {
+    switch (g_mutant) {
+        case MR_O_MUT_ORDER_RAWZERO:
+        case MR_O_MUT_ORDER_SIGNFLIP: {
+            const int raw = g_mutant == MR_O_MUT_ORDER_RAWZERO, flip = g_mutant == MR_O_MUT_ORDER_SIGNFLIP;
+            const uint32_t kly = order_key(ly, raw, flip), kry = order_key(ry, raw, flip);
+            return kly < kry || (kly == kry && order_key(lx, raw, flip) < order_key(rx, raw, flip));
+        }
+        case MR_O_MUT_ORDER_DAZ:
+            lx = ftz(lx), ly = ftz(ly), rx = ftz(rx), ry = ftz(ry);
+            return ly < ry || (ly == ry && lx < rx);
+        default: /* MR_O_MUT_ORDER_TIE_LE */
+            return ly < ry || (ly == ry && lx <= rx);
+    }
+}
+
 /* :117-126 -- two separately rounded products, one rounded difference (compile with
  * -ffp-contract=off; the volatile-free form is safe on x86-64 SSE2, FLT_EVAL_METHOD 0) */
 static int is_left_of(const mr_o_tri* t, uint32_t pid, uint32_t s1, uint32_t s2) {
     const float* p = &t->points[2u * pid];
     const float* a = &t->points[2u * s1];
     const float* b = &t->points[2u * s2];
-    float mul1 = (b[0] - a[0]) * (p[1] - a[1]);
-    float mul2 = (b[1] - a[1]) * (p[0] - a[0]);
-    float d = mul1 - mul2;
+    float mul1, mul2, d;
+    if (g_mutant >= MR_O_MUT_SIDE_FMA && g_mutant <= MR_O_MUT_SIDE_GE) return is_left_of_mutant(p, a, b);
+    mul1 = (b[0] - a[0]) * (p[1] - a[1]);
+    mul2 = (b[1] - a[1]) * (p[0] - a[0]);
+    d = mul1 - mul2;
     return d > 0.0f;
 }
 
 /* :128-136 -- lexicographic (y, x); smaller y is "above" */
 static int point_is_above(const mr_o_tri* t, uint32_t lhs, uint32_t rhs) {
     float ly = t->points[2u * lhs + 1u], ry = t->points[2u * rhs + 1u];
+    if (g_mutant >= MR_O_MUT_ORDER_RAWZERO && g_mutant <= MR_O_MUT_ORDER_TIE_LE)
+        return point_is_above_mutant(t->points[2u * lhs], ly, t->points[2u * rhs], ry);
     if (ly < ry) return 1;
     if (ly == ry) return t->points[2u * lhs] < t->points[2u * rhs];
     return 0;
@@ -381,11 +438,20 @@ static int push_triangle_if_acute(mr_o_tri* t, uint32_t point, uint32_t axis1, u
     float ny1 = P[2u * point + 1u] - P[2u * axis1 + 1u];
     float nx2 = P[2u * point] - P[2u * axis2];
     float ny2 = P[2u * point + 1u] - P[2u * axis2 + 1u];
-    float diff = mr_o_atan2f(ny1, nx1) - mr_o_atan2f(ny2, nx2);
+    float diff;
     const float pi_f32 = 3.14159274101257324f; /* std.math.pi coerced to f32 */
     int is_acute;
+    if (g_mutant == MR_O_MUT_ACUTE_CR_ATAN2)
+        diff = (float)atan2((double)ny1, (double)nx1) - (float)atan2((double)ny2, (double)nx2);
+    else if (g_mutant == MR_O_MUT_ACUTE_DAZ_ATAN2)
+        diff = ftz(mr_o_atan2f(ftz(ny1), ftz(nx1))) - ftz(mr_o_atan2f(ftz(ny2), ftz(nx2)));
+    else
+        diff = mr_o_atan2f(ny1, nx1) - mr_o_atan2f(ny2, nx2);
     if (diff < 0.0f) diff = -diff; /* @abs; NaN stays NaN and compares false */
     is_acute = diff < pi_f32;
+    if (g_mutant == MR_O_MUT_ACUTE_PI_DOWN) is_acute = diff < 3.14159250259399414f; /* 0x40490fda */
+    if (g_mutant == MR_O_MUT_ACUTE_LE) is_acute = diff <= pi_f32;
+    if (g_mutant == MR_O_MUT_ACUTE_ALWAYS) is_acute = 1;
 #define EMIT(id) emit(ctx, (id), P[2u * (id)], P[2u * (id) + 1u])
     if (is_acute) {
         EMIT(point);

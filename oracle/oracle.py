@@ -90,6 +90,8 @@ def lib() -> C.CDLL:
                                                  C.c_void_p]
         L.mr_o_test_lift_caps.restype = None
         L.mr_o_test_lift_caps.argtypes = [C.c_uint32]
+        L.mr_o_test_mutant.restype = None
+        L.mr_o_test_mutant.argtypes = [C.c_uint32]
         L.mr_o_terrain_tile_bounds.restype = C.c_int
         L.mr_o_terrain_tile_bounds.argtypes = [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32,
                                                C.POINTER(MrTerrainParams), C.c_void_p]
@@ -325,6 +327,29 @@ def time_create_polygon(xy, offset, prime, reps=20000) -> float:
 def lift_caps(multiplier: int):
     """Test-only: multiply the contract caps of the oracle (1 restores them)."""
     lib().mr_o_test_lift_caps(multiplier)
+
+
+# Test-only mutants of the float rules (mr_oracle.h, MR_O_MUT_*): name -> (id, rule).  Same order as the C enum.
+MUTANTS = {name: (i + 1, rule) for i, (name, rule) in enumerate((
+    ("fma", "side"), ("f64", "side"), ("exactdiff", "side"), ("reform", "side"), ("ftz", "side"), ("ge", "side"),
+    ("rawzero", "order"), ("signflip", "order"), ("daz", "order"), ("tie_le", "order"),
+    ("cr_atan2", "acute"), ("pi_down", "acute"), ("le", "acute"), ("always", "acute"), ("daz_atan2", "acute"),
+    ("tie_replaces", "bbox"), ("own_y", "bbox"),
+    ("x_only", "nonfinite"), ("nan_only", "nonfinite")))}
+
+
+class mutant:
+    """Test-only: `with mutant("ftz"): ...` runs the oracle with one float rule replaced (None = the reference)."""
+
+    def __init__(self, name):
+        self.id = 0 if name is None else MUTANTS[name][0]
+
+    def __enter__(self):
+        lib().mr_o_test_mutant(self.id)
+        return self
+
+    def __exit__(self, *exc):
+        lib().mr_o_test_mutant(0)
 
 
 def atan2f(y, x) -> float:

@@ -93,8 +93,17 @@ def transform(rng, xy, fp, how):
         return per_polygon(xy, fp, mid)
     if how == "scale_huge":  # products overflow to inf in the acute test and the side tests
         return xy * np.float32(2.0 ** 100)
+    if how == "float_edges":  # signed zeros, subnormal coordinates / products, overflowing differences, mirrors
+        def edge(p, i):
+            k = int(rng.integers(0, 4))
+            c = p.astype(np.float64) - p.astype(np.float64).mean(0)
+            c = c * np.array([1.0 if rng.random() < 0.5 else -1.0, 1.0 if rng.random() < 0.5 else -1.0])
+            if k == 0:  # quarter grid: small negative coordinates round to -0
+                return (np.round(c * 4.0) / 4.0).astype(np.float32)
+            return (c * (2.0 ** -140, 2.0 ** -75, 2.0 ** 121)[k - 1]).clip(-3.4e38, 3.4e38).astype(np.float32)
+        return per_polygon(xy, fp, edge)
     if how == "mixed":
-        pool = ["identity", "reverse", "quantise", "noise", "duplicate", "collinear"]
+        pool = ["identity", "reverse", "quantise", "noise", "duplicate", "collinear", "float_edges"]
         out = xy.copy()
         for i in range(len(fp) - 1):
             a, z = int(fp[i]), int(fp[i + 1])
@@ -109,7 +118,7 @@ def transform(rng, xy, fp, how):
 
 
 TRANSFORMS = ["identity", "reverse", "rotate_start", "swap_axes", "negate_y", "negate_x", "scale_up", "scale_down", "quantise",
-              "duplicate", "noise", "noise_grid", "same_y", "collinear", "scale_huge", "mixed"]
+              "duplicate", "noise", "noise_grid", "same_y", "collinear", "scale_huge", "float_edges", "mixed"]
 MIXES = ["small", "small", "tiny", "loguniform", "loguniform", "boundaries", "xl", "few"]
 
 

@@ -1,4 +1,4 @@
-"""The polygon parity cases once more against the BOUNDS-CHECKED build of the library (-DMR_CHECKED: every workspace
+"""The polygon parity and float-edge cases once more against the BOUNDS-CHECKED build of the library (-DMR_CHECKED: every workspace
 array of the fast path carries its length and traps on an index out of range).  compute-sanitizer is not available on
 the GPU pool; this is the memory-safety evidence for the shared-memory overlays of triangulate_fast.cuh."""
 import os
@@ -21,9 +21,10 @@ def test_polygon_parity_under_the_checked_build():
     probe = subprocess.run([sys.executable, "-c", "import myrenderer_b200 as m; print('flags', m.load().mr_build_flags())"],
                            capture_output=True, text=True, cwd=ROOT, env=env)
     assert "flags 1" in probe.stdout, probe.stdout + probe.stderr  # the checked build is the one that gets loaded
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.join(ROOT, "tests", "test_gpu_parity.py"), "-x", "-q", "-k", CASES],
-                       capture_output=True, text=True, timeout=1700, cwd=ROOT, env=env)
-    tail = r.stdout[-3000:] + r.stderr[-2000:]
-    assert r.returncode == 0, tail
-    assert "MR_CHECKED" not in r.stdout + r.stderr, tail
-    assert " passed" in r.stdout and "skipped" not in r.stdout.splitlines()[-1], tail
+    for args in (["test_gpu_parity.py", "-k", CASES], ["test_gpu_poly_float_edges.py"]):
+        r = subprocess.run([sys.executable, "-m", "pytest", os.path.join(ROOT, "tests", args[0]), "-x", "-q"] + args[1:],
+                           capture_output=True, text=True, timeout=1700, cwd=ROOT, env=env)
+        tail = r.stdout[-3000:] + r.stderr[-2000:]
+        assert r.returncode == 0, tail
+        assert "MR_CHECKED" not in r.stdout + r.stderr, tail
+        assert " passed" in r.stdout and "skipped" not in r.stdout.splitlines()[-1], tail
