@@ -250,6 +250,9 @@ int mr_heightmap_normalize(mr_context* ctx, const uint16_t* in, uint64_t count, 
  *                         row-major, six indices per quad exactly as mr_terrain_build writes them --
  *                         one drawIndexed(counts_out[1]) draws what survives the cull
  *     counts_out[2]       {visible tiles, indices written} as uint64
+ * Any tile size is accepted, up to and beyond the terrain (one tile may hold all (n-1)^2 quads); with idx_out
+ * the tile count is at most 2^31-1 (only 1 x 1 tiles of an n > 46341 terrain exceed it).  The arguments are checked
+ * before any kernel runs, so a rejected call writes no output.
  * Alignment (MR_E_BADARG otherwise): bbox_out of mr_terrain_tile_bounds 16 bytes (a box is two float4),
  * idx_out of mr_terrain_cull 8 bytes. */
 int mr_terrain_tile_count(uint32_t n, uint32_t tile_rows, uint32_t tile_cols, uint32_t* tiles_r_out,

@@ -574,9 +574,10 @@ __global__ void __launch_bounds__(1024) terrain_cull_k(const CullArgs a) {
     }
 }
 
-// compacted index buffer: CTA (k, chunk) writes TI_QUADS quads of visible tile k -- the tile's quads are one contiguous
-// run of the output -- built in shared memory and shipped with one bulk async copy, like terrain_indices_k (CTAs beyond
-// the visible count leave at once)
+// compacted index buffer: CTA (k, y) writes chunks y, y + gridDim.y, ... of TI_QUADS quads of visible tile k -- the tile's
+// quads are one contiguous run of the output -- each built in shared memory and shipped with one bulk async copy, like
+// terrain_indices_k (CTAs beyond the visible count leave at once).  A tile may hold up to (n-1)^2 < 2^32 quads, more chunks
+// than gridDim.y can count, hence the stride; the chunk offset is 64-bit because it steps past 2^32 on the way out.
 __global__ void __launch_bounds__(TI_THREADS) terrain_cull_indices_k(const CullArgs a, uint32_t* __restrict__ idx_out) {
     __shared__ __align__(16) uint32_t buf[TI_QUADS * 6 + 4];
     if (blockIdx.x >= a.counts[0]) return;
@@ -584,42 +585,47 @@ __global__ void __launch_bounds__(TI_THREADS) terrain_cull_indices_k(const CullA
     const uint32_t tr = t / a.tiles_c, tc = t - tr * a.tiles_c;
     const uint32_t r0 = tr * a.tile_rows, c0 = tc * a.tile_cols;
     const uint32_t qr = min(a.tile_rows, a.n - 1u - r0), qc = min(a.tile_cols, a.n - 1u - c0);
-    const uint32_t q0 = blockIdx.y * TI_QUADS;
-    if (q0 >= qr * qc) return;
-    const uint32_t nq = min((uint32_t)TI_QUADS, qr * qc - q0);
-    uint32_t* dst = idx_out + a.first_index[blockIdx.x] + (size_t)q0 * 6;  // 24-byte quads: 8-byte aligned
-    const uint32_t mis = (uint32_t)((reinterpret_cast<uintptr_t>(dst) >> 2) & 3u);
-    uint32_t* sbuf = buf + mis;
+    const uint64_t tile_quads = (uint64_t)qr * qc;
     const uint32_t n = a.n;
+    for (uint64_t q0 = (uint64_t)blockIdx.y * TI_QUADS; q0 < tile_quads; q0 += (uint64_t)gridDim.y * TI_QUADS) {
+        if (q0 != (uint64_t)blockIdx.y * TI_QUADS) {  // the previous chunk's bulk copy must have read buf before it is refilled
+            if (threadIdx.x == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+            __syncthreads();
+        }
+        const uint32_t nq = (uint32_t)min((uint64_t)TI_QUADS, tile_quads - q0);
+        uint32_t* dst = idx_out + a.first_index[blockIdx.x] + q0 * 6;  // 24-byte quads: 8-byte aligned
+        const uint32_t mis = (uint32_t)((reinterpret_cast<uintptr_t>(dst) >> 2) & 3u);
+        uint32_t* sbuf = buf + mis;
 #pragma unroll
-    for (int k = 0; k < TI_QPT; ++k) {
-        const uint32_t ql = k * TI_THREADS + threadIdx.x;
-        if (ql < nq) {
-            const uint32_t q = q0 + ql;
-            const uint32_t lr = q / qc, lc = q - lr * qc;
-            const uint32_t i00 = (r0 + lr) * n + c0 + lc;
-            uint2* sm = reinterpret_cast<uint2*>(sbuf + ql * 6);
-            sm[0] = make_uint2(i00 + n, i00);
-            sm[1] = make_uint2(i00 + n + 1, i00 + n + 1);
-            sm[2] = make_uint2(i00, i00 + 1);
+        for (int k = 0; k < TI_QPT; ++k) {
+            const uint32_t ql = k * TI_THREADS + threadIdx.x;
+            if (ql < nq) {
+                const uint32_t q = (uint32_t)q0 + ql;  // < qr * qc < 2^32
+                const uint32_t lr = q / qc, lc = q - lr * qc;
+                const uint32_t i00 = (r0 + lr) * n + c0 + lc;
+                uint2* sm = reinterpret_cast<uint2*>(sbuf + ql * 6);
+                sm[0] = make_uint2(i00 + n, i00);
+                sm[1] = make_uint2(i00 + n + 1, i00 + n + 1);
+                sm[2] = make_uint2(i00, i00 + 1);
+            }
+        }
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        __syncthreads();
+        const uint32_t words = nq * 6;
+        const uint32_t head = mis ? 2u : 0u;
+        const uint32_t body = ((words - head) / 4u) * 4u;
+        if (threadIdx.x == 0 && body) {
+            const uint32_t saddr = (uint32_t)__cvta_generic_to_shared(sbuf + head);
+            asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst + head), "r"(saddr), "r"(body * 4u)
+                         : "memory");
+            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+        }
+        if (threadIdx.x == 32) {
+            if (head) *reinterpret_cast<uint2*>(dst) = *reinterpret_cast<uint2*>(sbuf);
+            if (words - head - body) *reinterpret_cast<uint2*>(dst + head + body) = *reinterpret_cast<uint2*>(sbuf + head + body);
         }
     }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    __syncthreads();
-    const uint32_t words = nq * 6;
-    const uint32_t head = mis ? 2u : 0u;
-    const uint32_t body = ((words - head) / 4u) * 4u;
-    if (threadIdx.x == 0 && body) {
-        const uint32_t saddr = (uint32_t)__cvta_generic_to_shared(sbuf + head);
-        asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst + head), "r"(saddr), "r"(body * 4u)
-                     : "memory");
-        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-    }
-    if (threadIdx.x == 32) {
-        if (head) *reinterpret_cast<uint2*>(dst) = *reinterpret_cast<uint2*>(sbuf);
-        if (words - head - body) *reinterpret_cast<uint2*>(dst + head + body) = *reinterpret_cast<uint2*>(sbuf + head + body);
-    }
-    if (threadIdx.x == 0 && body) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+    if (threadIdx.x == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
 }
 
 // exhaustive check of div_const against __fdiv_rn over all 2^32 dividends
@@ -776,13 +782,14 @@ int mr_terrain_cull_impl(mr_context* ctx, const float* bbox_dev, uint32_t n, uin
     a.visible_ids = ids_dev;
     a.first_index = first_index_dev;
     a.counts = counts_dev;
+    // one CTA column per tile: checked before anything runs, so that an error leaves every output untouched
+    if (idx_dev && a.ntiles > 0x7FFFFFFFu) return mr_fail(ctx, MR_E_BADARG, "cull: more than 2^31-1 tiles with idx_out");
     terrain_cull_k<<<1, 1024, 0, ctx->stream>>>(a);
     MR_LAUNCH_CHECK(ctx, "terrain_cull_k");
     if (idx_dev) {
         const uint64_t tile_quads = (uint64_t)std::min(tile_rows, n - 1u) * std::min(tile_cols, n - 1u);
-        const uint64_t chunks = (tile_quads + TI_QUADS - 1) / TI_QUADS;
-        if (chunks > 65535u) return mr_fail(ctx, MR_E_BADARG, "cull: tiles too large for one launch");
-        terrain_cull_indices_k<<<dim3(a.ntiles, (unsigned)chunks), TI_THREADS, 0, ctx->stream>>>(a, idx_dev);
+        const uint64_t chunks = (tile_quads + TI_QUADS - 1) / TI_QUADS;  // terrain_cull_indices_k strides over the rest
+        terrain_cull_indices_k<<<dim3(a.ntiles, (unsigned)std::min<uint64_t>(chunks, 65535u)), TI_THREADS, 0, ctx->stream>>>(a, idx_dev);
         MR_LAUNCH_CHECK(ctx, "terrain_cull_indices_k");
     }
     return MR_OK;

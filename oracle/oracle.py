@@ -265,14 +265,25 @@ def scene_node_should_render(xform, p0, p1) -> bool:
     return bool(lib().mr_o_scene_node_should_render(_ptr(m), _ptr(a), _ptr(b)))
 
 
-def terrain_cull(bbox, n, tile_rows, tile_cols, xform, want_idx=True):
+def terrain_cull(bbox, n, tile_rows, tile_cols, xform, want_idx=True, idx_capacity=None):
+    """Oracle cull.  The index buffer is allocated for every quad, 6 (n-1)^2 words, unless idx_capacity is given: then a
+    first pass counts the visible indices, and the buffer holds exactly that many (at most idx_capacity words), so that a
+    cull of a large terrain with few visible tiles fits in host memory."""
     bbox = np.ascontiguousarray(bbox, dtype=np.float32)
     m = np.ascontiguousarray(xform, dtype=np.float32).reshape(16)
     ntiles = bbox.shape[0]
     vis = np.zeros(ntiles, dtype=np.uint32)
     ids = np.zeros(ntiles, dtype=np.uint32)
-    idx = np.zeros(6 * (n - 1) * (n - 1), dtype=np.uint32) if want_idx else None
     counts = np.zeros(2, dtype=np.uint64)
+    words = 6 * (n - 1) * (n - 1)
+    if want_idx and idx_capacity is not None:
+        rc = lib().mr_o_terrain_cull(_ptr(bbox), n, tile_rows, tile_cols, _ptr(m), _ptr(vis), _ptr(ids), None, _ptr(counts))
+        if rc != 0:
+            raise RuntimeError(f"oracle terrain_cull rc={rc}")
+        words = int(counts[1])
+        if words > idx_capacity:
+            raise ValueError(f"oracle terrain_cull: {words} visible indices exceed idx_capacity {idx_capacity}")
+    idx = np.zeros(words, dtype=np.uint32) if want_idx else None
     rc = lib().mr_o_terrain_cull(_ptr(bbox), n, tile_rows, tile_cols, _ptr(m), _ptr(vis), _ptr(ids), _ptr(idx), _ptr(counts))
     if rc != 0:
         raise RuntimeError(f"oracle terrain_cull rc={rc}")
