@@ -254,7 +254,25 @@ int mr_heightmap_normalize(mr_context* ctx, const uint16_t* in, uint64_t count, 
  * the tile count is at most 2^31-1 (only 1 x 1 tiles of an n > 46341 terrain exceed it).  The arguments are checked
  * before any kernel runs, so a rejected call writes no output.
  * Alignment (MR_E_BADARG otherwise): bbox_out of mr_terrain_tile_bounds 16 bytes (a box is two float4),
- * idx_out of mr_terrain_cull 8 bytes. */
+ * idx_out of mr_terrain_cull 8 bytes.
+ *
+ * mr_terrain_cull_frustum is mr_terrain_cull with the standard six-plane frustum test in place of the
+ * reference's: the outputs, argument checks, alignment, device / host pointers, the checks before any kernel
+ * runs and the 2^31-1 tile limit with idx_out are those above.  The reference's test does no perspective divide
+ * and is kept for parity; this one is the cull to draw with under a perspective camera.  Bit for bit:
+ *   view_proj is the memory image of mach's Mat4x4, as xform above: clip[i] = sum_j view_proj[4j+i] * v[j].  The
+ *     clip volume is WebGPU's, -w <= x <= w, -w <= y <= w, 0 <= z <= w (math.zig's perspective maps near..far to
+ *     depth 0..w).
+ *   Row i is R_i = (view_proj[i], view_proj[4+i], view_proj[8+i], view_proj[12+i]).  The six planes are
+ *     R3+R0, R3-R0, R3+R1, R3-R1, R2, R3-R2, each component one rounded f32 add or subtract; not normalised.
+ *   Per plane (a, b, c, d) and box: lo = p0.xyz, hi = p1.xyz (the w components are not read);
+ *     px = (a >= 0) ? hi.x : lo.x, py likewise from b, pz from c (so -0 picks hi and a NaN coefficient picks lo);
+ *     s = ((a*px + b*py) + c*pz) + d, every product and sum rounded on its own (no FMA, no flush to zero).
+ *   A tile is culled iff s < 0 for some plane; a NaN s never culls.  bbox may hold any floats.
+ * Properties that follow: in exact arithmetic a box with any point inside the clip volume is never culled; a box
+ * lying wholly on the outer side of one plane is culled; SceneNode's default box (-inf..+inf) is never culled, since
+ * every p-vertex term is +inf or NaN; and, as usual for this test, a box near the frustum's edges and corners can
+ * survive although it lies outside. */
 int mr_terrain_tile_count(uint32_t n, uint32_t tile_rows, uint32_t tile_cols, uint32_t* tiles_r_out,
                           uint32_t* tiles_c_out);
 int mr_terrain_tile_bounds(mr_context* ctx, const void* height, uint32_t height_fmt, uint32_t n,
@@ -263,6 +281,9 @@ int mr_terrain_tile_bounds(mr_context* ctx, const void* height, uint32_t height_
 int mr_terrain_cull(mr_context* ctx, const float* bbox /* tiles * 8 */, uint32_t n, uint32_t tile_rows,
                     uint32_t tile_cols, const float xform[16], uint32_t* visible_out,
                     uint32_t* visible_ids_out, uint32_t* idx_out, uint64_t* counts_out);
+int mr_terrain_cull_frustum(mr_context* ctx, const float* bbox /* tiles * 8 */, uint32_t n, uint32_t tile_rows,
+                            uint32_t tile_cols, const float view_proj[16], uint32_t* visible_out,
+                            uint32_t* visible_ids_out, uint32_t* idx_out, uint64_t* counts_out);
 
 /* ---- polygons --------------------------------------------------------------
  * Triangulates npoly polygons exactly as Triangulation.create_polygon would,

@@ -161,6 +161,9 @@ SIGNATURES = {
     "mr_terrain_cull": (
         C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p,
                   C.c_void_p, C.c_void_p]),
+    "mr_terrain_cull_frustum": (
+        C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p,
+                  C.c_void_p, C.c_void_p]),
     "mr_build_flags": (C.c_int, []),
     "mr_context_trim": (C.c_int, [C.c_void_p]),
     "mr_context_scratch_bytes": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),

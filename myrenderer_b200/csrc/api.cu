@@ -10,8 +10,8 @@ int mr_heightmap_normalize_impl(mr_context* ctx, const uint16_t* in, uint64_t co
 int mr_terrain_tile_bounds_impl(mr_context* ctx, const void* height_dev, uint32_t height_fmt, uint32_t n, uint32_t tile_rows,
                                 uint32_t tile_cols, const mr_terrain_params* p, float* bbox_dev);
 int mr_terrain_cull_impl(mr_context* ctx, const float* bbox_dev, uint32_t n, uint32_t tile_rows, uint32_t tile_cols,
-                         const float xform[16], uint32_t* visible_dev, uint32_t* ids_dev, unsigned long long* first_index_dev,
-                         uint32_t* idx_dev, unsigned long long* counts_dev);
+                         const float xform[16], bool frustum, uint32_t* visible_dev, uint32_t* ids_dev,
+                         unsigned long long* first_index_dev, uint32_t* idx_dev, unsigned long long* counts_dev);
 int mr_selftest_fastdiv_impl(mr_context* ctx, float b, int force_fast, unsigned long long* mismatches_dev);
 int mr_polygon_offsets_impl(mr_context* ctx, const uint64_t* first_point_dev, uint32_t npoly, uint64_t* first_tri_dev);
 int mr_triangulate_tier_counts_impl(mr_context* ctx, uint32_t out[8]);
@@ -394,8 +394,10 @@ int mr_terrain_tile_bounds(mr_context* ctx, const void* height, uint32_t height_
     return mr_finish_host_io(ctx);
 }
 
-int mr_terrain_cull(mr_context* ctx, const float* bbox, uint32_t n, uint32_t tile_rows, uint32_t tile_cols, const float xform[16],
-                    uint32_t* visible_out, uint32_t* visible_ids_out, uint32_t* idx_out, uint64_t* counts_out) {
+namespace {
+// mr_terrain_cull and mr_terrain_cull_frustum: the same checks, staging and copy-back; only the visibility test differs.
+int terrain_cull_common(mr_context* ctx, const float* bbox, uint32_t n, uint32_t tile_rows, uint32_t tile_cols, const float xform[16],
+                        bool frustum, uint32_t* visible_out, uint32_t* visible_ids_out, uint32_t* idx_out, uint64_t* counts_out) {
     if (!ctx || !bbox || !xform) return MR_E_BADARG;
     uint32_t tr = 0, tc = 0;
     if (n > 65535u || mr_terrain_tile_count(n, tile_rows, tile_cols, &tr, &tc) != MR_OK) return mr_fail(ctx, MR_E_BADARG, "cull: bad n or tile size");
@@ -419,7 +421,7 @@ int mr_terrain_cull(mr_context* ctx, const float* bbox, uint32_t n, uint32_t til
     if (idx_out) { rc = mr_stage_out(ctx, 5, idx_out, max_idx_bytes, &xdev, &sx); if (rc) return rc; }
     if (counts_out) { rc = mr_stage_out(ctx, 3, counts_out, 16, &cdev, &sc); if (rc) return rc; }
     else { rc = mr_scratch(ctx, 3, 16, &cdev); if (rc) return rc; }
-    rc = mr_terrain_cull_impl(ctx, static_cast<const float*>(bdev), n, tile_rows, tile_cols, xform, static_cast<uint32_t*>(vdev),
+    rc = mr_terrain_cull_impl(ctx, static_cast<const float*>(bdev), n, tile_rows, tile_cols, xform, frustum, static_cast<uint32_t*>(vdev),
                               static_cast<uint32_t*>(idev), first_index, static_cast<uint32_t*>(xdev),
                               static_cast<unsigned long long*>(cdev));
     if (rc) return rc;
@@ -433,6 +435,18 @@ int mr_terrain_cull(mr_context* ctx, const float* bbox, uint32_t n, uint32_t til
         if (sx && counts[1]) { rc = mr_copy_back(ctx, idx_out, xdev, (size_t)counts[1] * 4); if (rc) return rc; }
     }
     return mr_finish_host_io(ctx);
+}
+}  // namespace
+
+int mr_terrain_cull(mr_context* ctx, const float* bbox, uint32_t n, uint32_t tile_rows, uint32_t tile_cols, const float xform[16],
+                    uint32_t* visible_out, uint32_t* visible_ids_out, uint32_t* idx_out, uint64_t* counts_out) {
+    return terrain_cull_common(ctx, bbox, n, tile_rows, tile_cols, xform, false, visible_out, visible_ids_out, idx_out, counts_out);
+}
+
+int mr_terrain_cull_frustum(mr_context* ctx, const float* bbox, uint32_t n, uint32_t tile_rows, uint32_t tile_cols,
+                            const float view_proj[16], uint32_t* visible_out, uint32_t* visible_ids_out, uint32_t* idx_out,
+                            uint64_t* counts_out) {
+    return terrain_cull_common(ctx, bbox, n, tile_rows, tile_cols, view_proj, true, visible_out, visible_ids_out, idx_out, counts_out);
 }
 
 int mr_selftest_fastdiv(mr_context* ctx, float divisor, int force_fast, uint64_t* mismatches_out) {

@@ -490,9 +490,33 @@ struct CullArgs {
     unsigned long long* counts;       // [0] visible tiles, [1] indices
 };
 
-// SceneNode.zig:96-110 per tile, then an ordered compaction.  One CTA of 1024 threads walks the tiles in chunks
-// (a terrain has at most a few 10^4 tiles); the order of the visible list is the tile order.
-__global__ void __launch_bounds__(1024) terrain_cull_k(const CullArgs a) {
+// The six clip planes of the frustum test, (a, b, c, d) each, in the order of the header: R3+R0, R3-R0, R3+R1, R3-R1, R2,
+// R3-R2 with R_i row i of the view-projection.  A parameter of its own rather than a tail of CullArgs, so that
+// terrain_cull_indices_k, which takes CullArgs and then idx_out, keeps its parameter layout.
+struct CullPlanes {
+    float p[24];
+};
+
+// The frustum test for one box: culled iff s < 0 for some plane, s = ((a*px + b*py) + c*pz) + d at the p-vertex
+// (hi where the coefficient is >= 0, else lo; -0 picks hi, NaN picks lo); every operation rounded on its own, so a NaN
+// s never culls.  The w components of the box are not read.
+__device__ __forceinline__ bool frustum_visible(const CullPlanes& pl, const float4 lo, const float4 hi) {
+    bool culled = false;
+#pragma unroll
+    for (int k = 0; k < 6; ++k) {
+        const float pa = pl.p[4 * k], pb = pl.p[4 * k + 1], pc = pl.p[4 * k + 2], pd = pl.p[4 * k + 3];
+        const float px = pa >= 0.0f ? hi.x : lo.x, py = pb >= 0.0f ? hi.y : lo.y, pz = pc >= 0.0f ? hi.z : lo.z;
+        const float s = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(pa, px), __fmul_rn(pb, py)), __fmul_rn(pc, pz)), pd);
+        culled |= s < 0.0f;
+    }
+    return !culled;
+}
+
+// Per tile either SceneNode.zig:96-110 (FRUSTUM false) or the six-plane frustum test (FRUSTUM true), then an ordered
+// compaction.  One CTA of 1024 threads walks the tiles in chunks (a terrain has at most a few 10^4 tiles); the order of
+// the visible list is the tile order.
+template <bool FRUSTUM>
+__global__ void __launch_bounds__(1024) terrain_cull_k(const CullArgs a, const CullPlanes pl) {
     __shared__ uint32_t wsum_t[32];
     __shared__ unsigned long long wsum_q[32];
     __shared__ uint32_t base_t;
@@ -511,10 +535,14 @@ __global__ void __launch_bounds__(1024) terrain_cull_k(const CullArgs a) {
         if (t < a.ntiles) {
             float4 p0 = *reinterpret_cast<const float4*>(a.bbox + 8 * (size_t)t);
             float4 p1 = *reinterpret_cast<const float4*>(a.bbox + 8 * (size_t)t + 4);
-            if (fminf(fminf(p0.x, p0.y), fminf(p0.z, p0.w)) != -inf) p0 = mach_mul_vec(a.m, p0);  // :100-101
-            if (fmaxf(fmaxf(p1.x, p1.y), fmaxf(p1.z, p1.w)) != inf) p1 = mach_mul_vec(a.m, p1);   // :103-105
-            vis = (p1.x > 0.0f && p1.y > 0.0f && p1.z > 0.0f && p1.w > 0.0f) ||
-                  (p0.x < 1.0f && p0.y < 1.0f && p0.z < 1.0f && p0.w < 1.0f);  // :111
+            if (FRUSTUM) {
+                vis = frustum_visible(pl, p0, p1);
+            } else {
+                if (fminf(fminf(p0.x, p0.y), fminf(p0.z, p0.w)) != -inf) p0 = mach_mul_vec(a.m, p0);  // :100-101
+                if (fmaxf(fmaxf(p1.x, p1.y), fmaxf(p1.z, p1.w)) != inf) p1 = mach_mul_vec(a.m, p1);   // :103-105
+                vis = (p1.x > 0.0f && p1.y > 0.0f && p1.z > 0.0f && p1.w > 0.0f) ||
+                      (p0.x < 1.0f && p0.y < 1.0f && p0.z < 1.0f && p0.w < 1.0f);  // :111
+            }
             const uint32_t tr = t / a.tiles_c, tc = t - tr * a.tiles_c;
             const uint32_t qr = min(a.tile_rows, a.n - 1u - tr * a.tile_rows), qc = min(a.tile_cols, a.n - 1u - tc * a.tile_cols);
             quads = vis ? qr * qc : 0u;
@@ -767,9 +795,22 @@ int mr_terrain_tile_bounds_impl(mr_context* ctx, const void* height_dev, uint32_
 }
 
 int mr_terrain_cull_impl(mr_context* ctx, const float* bbox_dev, uint32_t n, uint32_t tile_rows, uint32_t tile_cols,
-                         const float xform[16], uint32_t* visible_dev, uint32_t* ids_dev, unsigned long long* first_index_dev,
-                         uint32_t* idx_dev, unsigned long long* counts_dev) {
+                         const float xform[16], bool frustum, uint32_t* visible_dev, uint32_t* ids_dev,
+                         unsigned long long* first_index_dev, uint32_t* idx_dev, unsigned long long* counts_dev) {
     CullArgs a;
+    CullPlanes pl;
+    memset(&pl, 0, sizeof(pl));
+    if (frustum) {  // rows R_i = (xform[i], xform[4+i], xform[8+i], xform[12+i]); one rounded add or subtract per component
+        for (int j = 0; j < 4; ++j) {
+            const float r0 = xform[4 * j], r1 = xform[4 * j + 1], r2 = xform[4 * j + 2], r3 = xform[4 * j + 3];
+            pl.p[0 + j] = r3 + r0;   // left:   w + x >= 0
+            pl.p[4 + j] = r3 - r0;   // right:  w - x >= 0
+            pl.p[8 + j] = r3 + r1;   // bottom: w + y >= 0
+            pl.p[12 + j] = r3 - r1;  // top:    w - y >= 0
+            pl.p[16 + j] = r2;       // near:   z >= 0 (WebGPU depth range)
+            pl.p[20 + j] = r3 - r2;  // far:    w - z >= 0
+        }
+    }
     a.bbox = bbox_dev;
     a.n = n;
     a.tile_rows = tile_rows;
@@ -784,7 +825,10 @@ int mr_terrain_cull_impl(mr_context* ctx, const float* bbox_dev, uint32_t n, uin
     a.counts = counts_dev;
     // one CTA column per tile: checked before anything runs, so that an error leaves every output untouched
     if (idx_dev && a.ntiles > 0x7FFFFFFFu) return mr_fail(ctx, MR_E_BADARG, "cull: more than 2^31-1 tiles with idx_out");
-    terrain_cull_k<<<1, 1024, 0, ctx->stream>>>(a);
+    if (frustum)
+        terrain_cull_k<true><<<1, 1024, 0, ctx->stream>>>(a, pl);
+    else
+        terrain_cull_k<false><<<1, 1024, 0, ctx->stream>>>(a, pl);
     MR_LAUNCH_CHECK(ctx, "terrain_cull_k");
     if (idx_dev) {
         const uint64_t tile_quads = (uint64_t)std::min(tile_rows, n - 1u) * std::min(tile_cols, n - 1u);

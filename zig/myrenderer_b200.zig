@@ -71,6 +71,8 @@ pub extern fn mr_pinned_free(ctx: ?*Context, host: ?*anyopaque) c_int;
 pub extern fn mr_terrain_tile_count(n: u32, tile_rows: u32, tile_cols: u32, tiles_r_out: ?*u32, tiles_c_out: ?*u32) c_int;
 pub extern fn mr_terrain_tile_bounds(ctx: ?*Context, height: *const anyopaque, height_fmt: u32, n: u32, tile_rows: u32, tile_cols: u32, params: ?*const TerrainParams, bbox_out: [*]f32) c_int;
 pub extern fn mr_terrain_cull(ctx: ?*Context, bbox: [*]const f32, n: u32, tile_rows: u32, tile_cols: u32, xform: *const [16]f32, visible_out: ?[*]u32, visible_ids_out: ?[*]u32, idx_out: ?[*]u32, counts_out: ?*[2]u64) c_int;
+// the six-plane frustum test (WebGPU clip volume) in place of SceneNode's; same arguments and outputs
+pub extern fn mr_terrain_cull_frustum(ctx: ?*Context, bbox: [*]const f32, n: u32, tile_rows: u32, tile_cols: u32, view_proj: *const [16]f32, visible_out: ?[*]u32, visible_ids_out: ?[*]u32, idx_out: ?[*]u32, counts_out: ?*[2]u64) c_int;
 
 pub const Error = error{GeometryBackend};
 
