@@ -9,7 +9,7 @@
  *
  *   Terrain.create_terrain            Terrain/Terrain.zig:88-129   -> mr_terrain_build
  *   WGSL vertex formula               Terrain/Terrain.zig:21-50    -> mr_terrain_build (positions)
- *   Polygon.create_polygon            Polygon/Polygon.zig:81-107   -> mr_triangulate_batch
+ *   Polygon.create_polygon            Polygon/Polygon.zig:81-107   -> mr_triangulate_batch (mr_triangulate_earclip)
  *   Triangulation.create_polygon      Polygon/Triangulation.zig:446-589 -> mr_triangulate_batch
  *   render_point (emit sink)          Polygon/Polygon.zig:65-79    -> mr_triangulate_batch (vtx_out, bbox_out)
  *   unirand_seed / Unirand.next       Polygon/unirand.zig:12-50    -> mr_unirand_seed_batch (+ inside the kernel)
@@ -64,6 +64,7 @@ extern "C" {
 #define MR_POLY_TOO_LARGE 32u   /* n above MR_MAX_POLYGON_POINTS; nothing emitted                        */
 #define MR_POLY_ARENA 64u       /* resource cap hit: node id >= MR_NODE_CAP(n) or DFS stack >= MR_STACK_CAP(n); nothing emitted */
 #define MR_POLY_UNDERFILL 128u  /* fewer than n-2 triangles produced; tail of the range is zero (WebGPU zero-init) */
+#define MR_POLY_NO_EAR 256u     /* mr_triangulate_earclip only: a lap of the ring found no ear (never on a simple polygon) */
 
 #define MR_MAX_POLYGON_POINTS 4096u
 /* Resource caps (part of the contract; the oracle applies the same ones).  The reference's
@@ -329,6 +330,40 @@ int mr_triangulate_batch(mr_context* ctx, const mr_polygon_job* job);
  * points handed to the general path (coincident points, not-acute corner, ...); out[7] = polygons
  * of 3073..MR_MAX_POLYGON_POINTS points (always general path).  Synchronises the stream. */
 int mr_triangulate_tier_counts(mr_context* ctx, uint32_t out[8]);
+/* ---- ear clipping ------------------------------------------------------------
+ * mr_triangulate_batch reproduces the reference's triangulator, which fails on many non-convex polygons (DESIGN.md
+ * section 2).  mr_triangulate_earclip triangulates every simple polygon correctly, into the same output format: the
+ * job, its checks, alignment, layouts, host / device pointers, point_base / tri_base and the optional outputs are those
+ * of mr_triangulate_batch; offset_prime, seed and poly_index0 are ignored.  It stages host pointers like a large batch
+ * (no small-batch path), and leaves mr_triangulate_tier_counts and the reference path's launch state as they were.
+ *   n < 3, a NaN / +-inf coordinate on either axis, n > MR_MAX_POLYGON_POINTS: MR_POLY_DEGENERATE / NONFINITE /
+ *     TOO_LARGE written exactly as mr_triangulate_batch writes them (range zeroed, ntri 0, bbox +0).
+ *   Every other polygon emits exactly n-2 triangles, triangle k coloured palette[k % 4], bbox by the rule of
+ *   mr_triangulate_batch over the emitted vertices in order.  A first_tri range of another size keeps the reference
+ *   path's rule: triangles past it are dropped (MR_POLY_OVERFLOW, still counted in the bbox), a shorter polygon leaves a
+ *   zeroed tail (MR_POLY_UNDERFILL); ntri = min(n-2, range).
+ * Bit for bit.  P[i] is point i; a == b is float equality of both coordinates (-0 == +0).
+ *   orient(a, b, c) = sign of the EXACT value of (bx-ax)(cy-ay) - (by-ay)(cx-ax) for the float inputs (nothing rounded
+ *     or flushed; mr_selftest_orient exposes the device's predicate).
+ *   Winding s: m = the first index smallest in (y, x); pm / nm = the nearest ring predecessor / successor of m whose
+ *     point differs from P[m]; s = orient(P[pm], P[m], P[nm]), or +1 if that is 0 or all points coincide.
+ *   Ring: doubly linked over 0..n-1.  Cursor c = 0, stop = c.  While the ring has k > 3 vertices, with p = prev(c),
+ *     q = next(c), c is an ear if
+ *       (a) P[c] == P[p] or P[c] == P[q] (a zero-length edge), or
+ *       (b) s*orient(p, c, q) > 0 and no blocker lies in the closed triangle: a blocker is a ring vertex r not in
+ *           {p, c, q} with s*orient(prev(r), r, next(r)) <= 0, P[r] different from P[p], P[c] and P[q], and
+ *           s*orient(p, c, r) >= 0, s*orient(c, q, r) >= 0, s*orient(q, p, r) >= 0.
+ *     Ear: emit (p, c, q) if s > 0 else (q, c, p), unlink c, c = next(q), stop = c.
+ *     Not an ear: c = next(c); if c == stop, a whole lap found no ear: clip c anyway as above and set MR_POLY_NO_EAR.
+ *   At k = 3: emit (prev(c), c, next(c)), ordered by the same rule.
+ * Properties: a simple polygon (collinear and repeated vertices allowed) never sets MR_POLY_NO_EAR and its triangles
+ * tile it exactly, every one with orientation >= 0 in raw (x, y) (two-ears theorem: a vertex that is not strictly
+ * convex is the only kind that can lie in an ear's triangle).  Any other input still gets n-2 triangles and a defined,
+ * bit-exact result.  Cost: O(n^2) candidate tests per polygon in the worst case, each scanning up to n blockers. */
+int mr_triangulate_earclip(mr_context* ctx, const mr_polygon_job* job);
+/* Self-test used by the test-suite: sign_out[i] = orient of the triple abc[6i..6i+5] = (ax, ay, bx, by, cx, cy), as
+ * mr_triangulate_earclip evaluates it (-1, 0, +1). */
+int mr_selftest_orient(mr_context* ctx, const float* abc /* 6 per triple */, uint64_t count, int8_t* sign_out);
 /* first_tri[0..npoly] from first_point[0..npoly] (device or host pointers). */
 int mr_polygon_offsets(mr_context* ctx, const uint64_t* first_point, uint32_t npoly,
                        uint64_t* first_tri_out);

@@ -138,6 +138,8 @@ SIGNATURES = {
     "mr_heightmap_normalize": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
     "mr_selftest_fastdiv": (C.c_int, [C.c_void_p, C.c_float, C.c_int, C.POINTER(C.c_uint64)]),
     "mr_triangulate_batch": (C.c_int, [C.c_void_p, C.POINTER(MrPolygonJob)]),
+    "mr_triangulate_earclip": (C.c_int, [C.c_void_p, C.POINTER(MrPolygonJob)]),
+    "mr_selftest_orient": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
     "mr_polygon_offsets": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]),
     "mr_triangulate_tier_counts": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint32)]),
     "mr_polygon_draw_range": (

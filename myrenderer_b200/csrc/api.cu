@@ -513,7 +513,10 @@ int mr_polygon_draw_range(uint64_t first_tri_i, uint64_t first_tri_next, uint64_
     return MR_OK;
 }
 
-int mr_triangulate_batch(mr_context* ctx, const mr_polygon_job* job) {
+namespace {
+// mr_triangulate_batch and mr_triangulate_earclip: the same checks, staging and copy-back; ear clipping takes no edge
+// order and has no small-batch path.
+int triangulate_common(mr_context* ctx, const mr_polygon_job* job, bool earclip) {
     if (!ctx || !job) return MR_E_BADARG;
     const mr_polygon_job& j = *job;
     if (j.npoly == 0) return MR_OK;
@@ -522,7 +525,7 @@ int mr_triangulate_batch(mr_context* ctx, const mr_polygon_job* job) {
     if (j.layout.nattr > 1 && j.layout.attr[1].ncomp < 3) return mr_fail(ctx, MR_E_BADARG, "polygons: colour needs 3 components");
     if (reinterpret_cast<uintptr_t>(j.vtx_out) & 3u) return mr_fail(ctx, MR_E_BADARG, "polygons: vtx_out must be 4-byte aligned");
     MR_CUDA(ctx, cudaSetDevice(ctx->device));
-    {   // the reference's own call shape (Polygon.create_polygon: one small polygon, everything in host memory)
+    if (!earclip) {  // the reference's own call shape (Polygon.create_polygon: one small polygon, everything in host memory)
         int rc_small = MR_OK;
         if (mr_triangulate_small(ctx, &j, &rc_small)) return rc_small;
     }
@@ -565,7 +568,8 @@ int mr_triangulate_batch(mr_context* ctx, const mr_polygon_job* job) {
     rc = mr_stage_in(ctx, 2, j.first_tri, (size_t)(j.npoly + 1) * 8, &p);
     if (rc) return rc;
     d.first_tri = static_cast<const uint64_t*>(p);
-    if (j.offset_prime) {
+    d.offset_prime = nullptr;
+    if (j.offset_prime && !earclip) {
         rc = mr_stage_in(ctx, 3, j.offset_prime, (size_t)j.npoly * 8, &p);
         if (rc) return rc;
         d.offset_prime = static_cast<const uint32_t*>(p);
@@ -599,7 +603,7 @@ int mr_triangulate_batch(mr_context* ctx, const mr_polygon_job* job) {
         if (rc) return rc;
         d.ntri_out = static_cast<uint32_t*>(q);
     }
-    rc = mr_triangulate_impl(ctx, &d, fp_dev ? nullptr : j.first_point);
+    rc = earclip ? mr_triangulate_earclip_impl(ctx, &d) : mr_triangulate_impl(ctx, &d, fp_dev ? nullptr : j.first_point);
     if (rc) return rc;
     if (sv) {
         // the polygons of this job own [first_tri[0], first_tri[npoly]) only
@@ -615,6 +619,30 @@ int mr_triangulate_batch(mr_context* ctx, const mr_polygon_job* job) {
     if (sb) { rc = mr_copy_back(ctx, j.bbox_out, d.bbox_out, (size_t)j.npoly * 16); if (rc) return rc; }
     if (ss) { rc = mr_copy_back(ctx, j.status_out, d.status_out, (size_t)j.npoly * 4); if (rc) return rc; }
     if (sn) { rc = mr_copy_back(ctx, j.ntri_out, d.ntri_out, (size_t)j.npoly * 4); if (rc) return rc; }
+    return mr_finish_host_io(ctx);
+}
+}  // namespace
+
+int mr_triangulate_batch(mr_context* ctx, const mr_polygon_job* job) { return triangulate_common(ctx, job, false); }
+
+int mr_triangulate_earclip(mr_context* ctx, const mr_polygon_job* job) { return triangulate_common(ctx, job, true); }
+
+int mr_selftest_orient(mr_context* ctx, const float* abc, uint64_t count, int8_t* sign_out) {
+    if (!ctx || (count && (!abc || !sign_out))) return MR_E_BADARG;
+    MR_CUDA(ctx, cudaSetDevice(ctx->device));
+    const void* din = nullptr;
+    int rc = mr_stage_in(ctx, 0, abc, (size_t)count * 24, &din);
+    if (rc) return rc;
+    void* dout = nullptr;
+    bool st = false;
+    rc = mr_stage_out(ctx, 4, sign_out, (size_t)count, &dout, &st);
+    if (rc) return rc;
+    rc = mr_selftest_orient_impl(ctx, static_cast<const float*>(din), count, static_cast<int8_t*>(dout));
+    if (rc) return rc;
+    if (st) {
+        rc = mr_copy_back(ctx, sign_out, dout, (size_t)count);
+        if (rc) return rc;
+    }
     return mr_finish_host_io(ctx);
 }
 

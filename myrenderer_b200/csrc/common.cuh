@@ -10,7 +10,7 @@
 #include <vector>
 #include "../../include/myrenderer_b200.h"
 
-#define MR_NUM_SCRATCH 13
+#define MR_NUM_SCRATCH 14
 
 constexpr int MR_NUM_AUX = 12;
 
@@ -183,3 +183,13 @@ int mr_triangulate_impl(mr_context* ctx, const mr_polygon_job* job, const uint64
 // all-host-pointer jobs small enough for the one-block path; returns 1 when it handled the job, 0 when it does not apply
 int mr_triangulate_small(mr_context* ctx, const mr_polygon_job* job, int* rc_out);
 void mr_polygon_plan_free(mr_context* ctx);
+// Stable counting sort of polygon ids by size, largest first (triangulate.cu; sizes above MR_MAX_POLYGON_POINTS ride in
+// bin 0).  hist and cursor hold MR_SIZE_BINS words each and must be zero; afterwards order[0..npoly) holds the ids and
+// cursor[b] is the number of polygons of size >= b, so the sizes lo..hi occupy order[cursor[hi + 1] .. cursor[lo]).
+// class_begin / class_end receive the reference path's size-class ranges (NUM_CLASSES words each).
+constexpr uint32_t MR_SIZE_BINS = MR_MAX_POLYGON_POINTS + 1;
+int mr_polygon_size_sort(mr_context* ctx, const uint64_t* first_point, uint32_t npoly, uint32_t* hist, uint32_t* cursor,
+                         uint32_t* class_begin, uint32_t* class_end, uint32_t* order);
+// ear clipping (earclip.cu); pointers as for mr_triangulate_impl
+int mr_triangulate_earclip_impl(mr_context* ctx, const mr_polygon_job* job);
+int mr_selftest_orient_impl(mr_context* ctx, const float* abc, uint64_t count, int8_t* sign_out);

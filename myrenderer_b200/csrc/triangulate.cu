@@ -538,85 +538,7 @@ __device__ __forceinline__ void triangle_order(uint32_t point, uint32_t axis1, u
     }
 }
 
-// Polygon.zig:50-57,66-71: palette[(len/3)%4], channels (hex&0xff, hex>>8&0xff, hex>>16&0xff)/255.0 of
-// 0x5e315b, 0xcfff70, 0x3ca370, 0x4b5bab.  The twelve quotients are constants; their bit patterns
-// (IEEE f32 division) are the ones of SURVEY 8-a12 and are checked against the oracle's computed
-// palette in tests/test_oracle_cpu.py::test_palette_bits and by every vertex-buffer comparison.
-__device__ __forceinline__ float3 palette(uint32_t tri) {
-    switch (tri & 3u) {
-        case 0: return make_float3(__uint_as_float(0x3EB6B6B7u), __uint_as_float(0x3E44C4C5u), __uint_as_float(0x3EBCBCBDu));
-        case 1: return make_float3(__uint_as_float(0x3EE0E0E1u), __uint_as_float(0x3F800000u), __uint_as_float(0x3F4FCFD0u));
-        case 2: return make_float3(__uint_as_float(0x3EE0E0E1u), __uint_as_float(0x3F23A3A4u), __uint_as_float(0x3E70F0F1u));
-        default: return make_float3(__uint_as_float(0x3F2BABACu), __uint_as_float(0x3EB6B6B7u), __uint_as_float(0x3E969697u));
-    }
-}
-
-struct Sink {
-    unsigned char* base;  // polygon's vertex range
-    uint32_t cap_vtx;     // 3*(n-2)
-    uint32_t stride, off_x, off_c;
-    int fast32;
-
-    // vertex `k` of the polygon: position P, colour of triangle k/3
-    __device__ __forceinline__ void write(uint32_t k, float2 P) const {
-        const float3 c = palette(k / 3u);
-        unsigned char* v = base + (size_t)k * stride;
-        if (fast32) {
-            if (off_x == 0)
-                asm volatile("st.global.v8.f32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(v), "f"(P.x), "f"(P.y),
-                             "f"(0.0f), "f"(0.0f), "f"(c.x), "f"(c.y), "f"(c.z), "f"(0.0f)
-                             : "memory");
-            else
-                asm volatile("st.global.v8.f32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(v), "f"(c.x), "f"(c.y),
-                             "f"(c.z), "f"(0.0f), "f"(P.x), "f"(P.y), "f"(0.0f), "f"(0.0f)
-                             : "memory");
-        } else {
-            float* f = reinterpret_cast<float*>(v);
-            for (uint32_t i = 0; i < stride / 4; ++i) f[i] = 0.0f;
-            float* px = reinterpret_cast<float*>(v + off_x);
-            px[0] = P.x;
-            px[1] = P.y;
-            if (off_c != 0xFFFFFFFFu) {
-                float* pc = reinterpret_cast<float*>(v + off_c);
-                pc[0] = c.x;
-                pc[1] = c.y;
-                pc[2] = c.z;
-            }
-        }
-    }
-    // zero vertices [k0, k1) cooperatively
-    // -DMR_OUTLINE_COLD (experiment, off by default; DESIGN.md section 9 item 2): zero() and the exact acute test out of
-    // line -- a sixth of the n <= 64 kernel's code, which runs short of instruction cache: measured -2..-4 % on that
-    // kernel.  Out of line the 256-bit asm store of one repeated operand was compiled as a 32-bit store, hence the
-    // plain stores under the flag.  Not shipped: the bounds-checked build did not finish its fuzz run with it.
-#ifdef MR_OUTLINE_COLD
-    __noinline__
-#endif
-    __device__ void zero(uint32_t k0, uint32_t k1, uint32_t lane, uint32_t nthreads = 32u) const {
-        if (k1 <= k0) return;
-        if (fast32) {
-#ifdef MR_OUTLINE_COLD
-            for (uint32_t k = k0 + lane; k < k1; k += nthreads) {
-                uint4* p = reinterpret_cast<uint4*>(base + (size_t)k * 32);
-                p[0] = make_uint4(0u, 0u, 0u, 0u);
-                p[1] = make_uint4(0u, 0u, 0u, 0u);
-            }
-#else
-            for (uint32_t k = k0 + lane; k < k1; k += nthreads)
-                asm volatile("st.global.v8.f32 [%0], {%1,%1,%1,%1,%1,%1,%1,%1};" ::"l"(base + (size_t)k * 32),
-                             "f"(0.0f)
-                             : "memory");
-#endif
-        } else {
-            uint32_t* w = reinterpret_cast<uint32_t*>(base + (size_t)k0 * stride);
-            const size_t words = (size_t)(k1 - k0) * stride / 4;
-            for (size_t i = lane; i < words; i += nthreads) w[i] = 0u;
-        }
-    }
-};
-
-__device__ __forceinline__ float fmin_acc(float acc, float v) { return v < acc ? v : acc; }
-__device__ __forceinline__ float fmax_acc(float acc, float v) { return v > acc ? v : acc; }
+#include "polygon_sink.cuh"
 
 // Result of one polygon
 struct Result {
@@ -1346,6 +1268,19 @@ static_assert(NUM_CLASSES <= CLASS_SLOTS && 2 * NUM_CLASSES + 2 <= 3 * CLASS_SLO
 enum { SLOT_XY = 0, SLOT_FP = 1, SLOT_FT = 2, SLOT_OP = 3, SLOT_VTX = 4, SLOT_BBOX = 5, SLOT_STATUS = 6, SLOT_NTRI = 7,
        SLOT_WORK = 8, SLOT_TIER1 = 9, SLOT_MISC = 10, SLOT_TIER1B = 11, SLOT_PAR = 12 };
 
+int mr_polygon_size_sort(mr_context* ctx, const uint64_t* first_point, uint32_t npoly, uint32_t* hist, uint32_t* cursor,
+                         uint32_t* class_begin, uint32_t* class_end, uint32_t* order) {
+    static_assert(NBINS == MR_SIZE_BINS, "size bins");
+    const unsigned cblocks = (unsigned)std::min<uint64_t>(((uint64_t)npoly + 255) / 256, (uint64_t)ctx->sm_count * 2);
+    size_hist_k<<<cblocks, 256, 0, ctx->stream>>>(first_point, npoly, hist);
+    MR_LAUNCH_CHECK(ctx, "size_hist_k");
+    size_scan_k<<<1, 1024, 0, ctx->stream>>>(hist, cursor, class_begin, class_end);
+    MR_LAUNCH_CHECK(ctx, "size_scan_k");
+    size_scatter_k<<<cblocks, 256, 0, ctx->stream>>>(first_point, npoly, cursor, order);
+    MR_LAUNCH_CHECK(ctx, "size_scatter_k");
+    return MR_OK;
+}
+
 int mr_polygon_offsets_impl(mr_context* ctx, const uint64_t* first_point_dev, uint32_t npoly,
                             uint64_t* first_tri_dev) {
     // counts are written into first_tri_dev[0..npoly) then scanned in place via a temp
@@ -1586,13 +1521,8 @@ int mr_triangulate_impl(mr_context* ctx, const mr_polygon_job* j, const uint64_t
     ctx->last_header_dev = w;
     MR_CUDA(ctx, cudaMemsetAsync(w, 0, (header_words + 2 * (size_t)NBINS) * 4, ctx->stream));
 
-    const unsigned cblocks = (unsigned)std::min<uint64_t>(((uint64_t)npoly + 255) / 256, (uint64_t)ctx->sm_count * 2);
-    size_hist_k<<<cblocks, 256, 0, ctx->stream>>>(j->first_point, npoly, hist);
-    MR_LAUNCH_CHECK(ctx, "size_hist_k");
-    size_scan_k<<<1, 1024, 0, ctx->stream>>>(hist, cursor, w + HDR_CLASS_BEGIN, w + HDR_CLASS_END);
-    MR_LAUNCH_CHECK(ctx, "size_scan_k");
-    size_scatter_k<<<cblocks, 256, 0, ctx->stream>>>(j->first_point, npoly, cursor, order);
-    MR_LAUNCH_CHECK(ctx, "size_scatter_k");
+    rc = mr_polygon_size_sort(ctx, j->first_point, npoly, hist, cursor, w + HDR_CLASS_BEGIN, w + HDR_CLASS_END, order);
+    if (rc) return rc;
 
     // Polygons per class: known exactly when the caller's first_point lives on the host (then empty classes cost no
     // launch at all); otherwise every class may hold up to npoly polygons and its kernel finds out on the device.

@@ -32,43 +32,6 @@
 //     O(k) scan of :329-337: same winner, because ties go to the lowest stack index in both.
 #pragma once
 
-// ---- checked build -----------------------------------------------------------------------------------
-// compute-sanitizer is not available on the GPU pool this library was developed on, and the workspace below is full of
-// deliberate overlays (five arrays laid over dead space), which is where an out-of-bounds write hides.  Every workspace
-// array of the fast path is therefore declared through MR_SPAN / MR_MAKE_SPAN: in the product build these are raw
-// pointers (no cost); with -DMR_CHECKED (make -C myrenderer_b200/csrc checked) they carry their length and every
-// access traps on an index out of range.  tests/test_gpu_checked.py runs the parity cases against that library.
-#ifdef MR_CHECKED
-template <class T>
-struct mr_span {
-    T* p;
-    uint32_t n;
-    int line;
-    __device__ __forceinline__ T& operator[](size_t i) const {
-        if (i >= n) {
-            printf("MR_CHECKED: index %llu out of range %u (span declared at triangulate_fast.cuh:%d; block %u thread %u)\n",
-                   (unsigned long long)i, n, line, blockIdx.x, threadIdx.x);
-            __trap();
-        }
-        return p[i];
-    }
-    __device__ __forceinline__ bool is_null() const { return p == nullptr; }
-    template <class U>
-    __device__ __forceinline__ operator mr_span<U>() const { return mr_span<U>{p, n, line}; }  // T* -> const T*
-};
-#define MR_SPAN(T) mr_span<T>
-#define MR_MAKE_SPAN(T, ptr, len) (mr_span<T>{(ptr), (uint32_t)(len), __LINE__})
-#define MR_SPAN_NULL(T) (mr_span<T>{nullptr, 0u, __LINE__})
-#define MR_SPAN_IS_NULL(s) ((s).is_null())
-#define MR_SPAN_RAW(s) ((s).p)
-#else
-#define MR_SPAN(T) T*
-#define MR_MAKE_SPAN(T, ptr, len) (ptr)
-#define MR_SPAN_NULL(T) (static_cast<T*>(nullptr))
-#define MR_SPAN_IS_NULL(s) ((s) == nullptr)
-#define MR_SPAN_RAW(s) (s)
-#endif
-
 __device__ __forceinline__ uint32_t mr_lds_u16(uint32_t shared_addr) {
     unsigned short v;
     asm volatile("ld.shared.u16 %0, [%1];" : "=h"(v) : "r"(shared_addr));

@@ -298,6 +298,16 @@ def polygon_offsets_host(first_point: np.ndarray) -> np.ndarray:
     return ft
 
 
+_ALGORITHMS = {"reference": "mr_triangulate_batch", "earclip": "mr_triangulate_earclip"}
+
+
+def _check_algorithm(algorithm, offset_prime):
+    if algorithm not in _ALGORITHMS:
+        raise ValueError(f"algorithm must be one of {sorted(_ALGORITHMS)}, not {algorithm!r}")
+    if algorithm == "earclip" and offset_prime is not None:
+        raise ValueError("ear clipping has no edge order: offset_prime applies to the reference algorithm only")
+
+
 class Polygon:
     """Mirror of the Polygon module (one reusable Triangulation inside: the Context's scratch)."""
 
@@ -315,12 +325,18 @@ class Polygon:
         j.bbox_out, j.status_out, j.ntri_out = _ptr(bbox_out), _ptr(status_out), _ptr(ntri_out)
         return j
 
-    def triangulate(self, job: MrPolygonJob):
-        self.ctx.check(self.ctx.lib.mr_triangulate_batch(self.ctx.handle, C.byref(job)), "mr_triangulate_batch")
+    def triangulate(self, job: MrPolygonJob, algorithm: str = "reference"):
+        """algorithm "reference": mr_triangulate_batch (the reference's triangulator, for parity); "earclip":
+        mr_triangulate_earclip (correct on every simple polygon, same output format)."""
+        _check_algorithm(algorithm, None)
+        name = _ALGORITHMS[algorithm]
+        self.ctx.check(getattr(self.ctx.lib, name)(self.ctx.handle, C.byref(job)), name)
 
     def create_polygons(self, xy, first_point, *, offset_prime=None, seed=0, poly_index0=0,
-                        device="cuda") -> PolygonBatch:
-        """Batched create_polygon.  xy: [npts,2] f32 (numpy or cuda tensor); first_point: npoly+1 offsets."""
+                        device="cuda", algorithm="reference") -> PolygonBatch:
+        """Batched create_polygon.  xy: [npts,2] f32 (numpy or cuda tensor); first_point: npoly+1 offsets.
+        algorithm: "reference" or "earclip" (see triangulate); ear clipping takes no offset_prime."""
+        _check_algorithm(algorithm, offset_prime)
         fp_host = np.ascontiguousarray(
             first_point.cpu().numpy() if _is_cuda(first_point) else first_point, dtype=np.uint64)
         npoly = len(fp_host) - 1
@@ -342,16 +358,17 @@ class Polygon:
         nt = torch.empty(npoly, dtype=torch.int32, device=dev)
         self.triangulate(self.job(xy_d, fp_d, npoly, vtx_out=vtx, first_tri=ft_d, bbox_out=bbox,
                                   status_out=status, ntri_out=nt, offset_prime=op_d, seed=seed,
-                                  poly_index0=poly_index0, point_base=int(fp_host[0])))
+                                  poly_index0=poly_index0, point_base=int(fp_host[0])), algorithm)
         return PolygonBatch(npoly, fp_host, ft_host, vtx[: ntri * 3 * self.layout.stride], bbox, status, nt,
                             self.layout)
 
-    def create_polygon(self, vertices, *, offset_prime=None, seed=0, index=0) -> PolygonObj:
+    def create_polygon(self, vertices, *, offset_prime=None, seed=0, index=0, algorithm="reference") -> PolygonObj:
         """Polygon.create_polygon(vertices): one polygon -> VertexBuffer of n-2 triangles + bbox.
 
         Like the reference (Polygon.zig:82-92: a mapped-at-creation buffer filled by the emit callback) the
         vertex range is HOST memory -- the stand-in for the mapped range -- so the call takes the library's
-        small-batch path: one copy in, one kernel, one copy out."""
+        small-batch path: one copy in, one kernel, one copy out.  algorithm: as for create_polygons."""
+        _check_algorithm(algorithm, offset_prime)
         v = np.ascontiguousarray(vertices, dtype=np.float32).reshape(-1, 2)
         n = len(v)
         if n < 2:  # Polygon.zig:82: vertices.len - 2 underflows
@@ -364,7 +381,7 @@ class Polygon:
         st = np.zeros(1, dtype=np.uint32)
         nt = np.zeros(1, dtype=np.uint32)
         self.triangulate(self.job(v, fp, 1, vtx_out=mapped, first_tri=ft, bbox_out=bb, status_out=st, ntri_out=nt,
-                                  offset_prime=op, seed=seed, poly_index0=index))
+                                  offset_prime=op, seed=seed, poly_index0=index), algorithm)
         buf = torch.from_numpy(mapped) if torch is not None else mapped
         vb = VertexBuffer(buf, (n - 2) * 3, 1, 0, 0)
         return PolygonObj(vb, (float(bb[0]), float(bb[1]), 0.0), (float(bb[2]), float(bb[3]), 0.0),

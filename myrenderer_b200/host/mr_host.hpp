@@ -202,6 +202,32 @@ class Polygon {
         o.bounding_box_p1[1] = bbox[3];
         return o;
     }
+    // The same polygon triangulated by ear clipping (mr_triangulate_earclip): correct on every simple polygon, no edge order.
+    PolygonObj create_polygon_earclip(const std::vector<Point>& vertices) {
+        if (vertices.size() < 2) throw Error(MR_E_BADARG, "create_polygon: vertices.len - 2 underflows (Polygon.zig:82)");
+        PolygonObj o;
+        const uint32_t n = static_cast<uint32_t>(vertices.size());
+        o.vertex_buffer = VertexBuffer::create(0, n - 2, layout_.native.stride);
+        const uint64_t first_point[2] = {0, n};
+        const uint64_t first_tri[2] = {0, n - 2};
+        float bbox[4];
+        mr_polygon_job j{};
+        j.xy = reinterpret_cast<const float*>(vertices.data());
+        j.first_point = first_point;
+        j.npoly = 1;
+        j.layout = layout_.native;
+        j.vtx_out = o.vertex_buffer.mapped.data();
+        j.first_tri = first_tri;
+        j.bbox_out = bbox;
+        j.status_out = &o.status;
+        j.ntri_out = &o.ntri;
+        ctx_.check(mr_triangulate_earclip(ctx_.get(), &j), "mr_triangulate_earclip");
+        o.bounding_box_p0[0] = bbox[0];
+        o.bounding_box_p0[1] = bbox[1];
+        o.bounding_box_p1[0] = bbox[2];
+        o.bounding_box_p1[1] = bbox[3];
+        return o;
+    }
     const VertexLayout& layout() const { return layout_; }
 
    private:

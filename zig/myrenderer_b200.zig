@@ -62,6 +62,7 @@ pub extern fn mr_terrain_build(ctx: ?*Context, job: *const TerrainJob) c_int;
 pub extern fn mr_terrain_build_full(ctx: ?*Context, height: *const anyopaque, height_fmt: u32, n: u32, layout: ?*const Layout, params: ?*const TerrainParams, vtx_out: ?*anyopaque, idx_out: ?[*]u32) c_int;
 pub extern fn mr_terrain_describe(n: u32, params: ?*const TerrainParams, bbox_min: ?*[3]f32, bbox_max: ?*[3]f32, vertex_count: ?*u64, index_count: ?*u64) c_int;
 pub extern fn mr_triangulate_batch(ctx: ?*Context, job: *const PolygonJob) c_int;
+pub extern fn mr_triangulate_earclip(ctx: ?*Context, job: *const PolygonJob) c_int;
 pub extern fn mr_polygon_draw_range(first_tri_i: u64, first_tri_next: u64, tri_base: u64, out: *DrawRange) c_int;
 pub extern fn mr_unirand_seed_host(top: u32, seed: u64, index: u64, offset_out: *u32, prime_out: *u32) c_int;
 pub extern fn mr_context_trim(ctx: ?*Context) c_int;
