@@ -87,28 +87,13 @@ struct Sink {
         }
     }
     // zero vertices [k0, k1) cooperatively
-    // -DMR_OUTLINE_COLD (experiment, off by default; DESIGN.md section 9 item 2): zero() and the exact acute test out of
-    // line -- a sixth of the n <= 64 kernel's code, which runs short of instruction cache: measured -2..-4 % on that
-    // kernel.  Out of line the 256-bit asm store of one repeated operand was compiled as a 32-bit store, hence the
-    // plain stores under the flag.  Not shipped: the bounds-checked build did not finish its fuzz run with it.
-#ifdef MR_OUTLINE_COLD
-    __noinline__
-#endif
     __device__ void zero(uint32_t k0, uint32_t k1, uint32_t lane, uint32_t nthreads = 32u) const {
         if (k1 <= k0) return;
         if (fast32) {
-#ifdef MR_OUTLINE_COLD
-            for (uint32_t k = k0 + lane; k < k1; k += nthreads) {
-                uint4* p = reinterpret_cast<uint4*>(base + (size_t)k * 32);
-                p[0] = make_uint4(0u, 0u, 0u, 0u);
-                p[1] = make_uint4(0u, 0u, 0u, 0u);
-            }
-#else
             for (uint32_t k = k0 + lane; k < k1; k += nthreads)
                 asm volatile("st.global.v8.f32 [%0], {%1,%1,%1,%1,%1,%1,%1,%1};" ::"l"(base + (size_t)k * 32),
                              "f"(0.0f)
                              : "memory");
-#endif
         } else {
             uint32_t* w = reinterpret_cast<uint32_t*>(base + (size_t)k0 * stride);
             const size_t words = (size_t)(k1 - k0) * stride / 4;

@@ -24,13 +24,7 @@
 namespace {
 
 constexpr int TV_THREADS = 256;  // columns per tile
-#ifndef MR_TV_ROWS
-#define MR_TV_ROWS 8  // measured: 8 beats 4, 16 and 32 at n = 4096 and n = 16384
-#endif
-#ifndef MR_TV_STORE
-#define MR_TV_STORE 0  // 0: default policy, 1: evict-first (.cs), 2: L1 no-allocate
-#endif
-constexpr int TV_ROWS = MR_TV_ROWS;  // rows per tile
+constexpr int TV_ROWS = 8;  // rows per tile; measured: 8 beats 4, 16 and 32 at n = 4096 and n = 16384
 
 struct DivConst {
     float b;  // divisor
@@ -79,13 +73,7 @@ __device__ __forceinline__ float load_height(const void* base, size_t idx) {
 __device__ __forceinline__ void store_vertex32(unsigned char* p, float a0, float a1, float a2, float b0,
                                                float b1, float b2) {
     // one 256-bit store: [a0 a1 a2 0 | b0 b1 b2 0]
-#if MR_TV_STORE == 1
-    asm volatile("st.global.cs.v8.f32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(p), "f"(a0), "f"(a1), "f"(a2),
-#elif MR_TV_STORE == 2
-    asm volatile("st.global.L1::no_allocate.v8.f32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(p), "f"(a0), "f"(a1), "f"(a2),
-#else
     asm volatile("st.global.v8.f32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(p), "f"(a0), "f"(a1), "f"(a2),
-#endif
                  "f"(0.0f), "f"(b0), "f"(b1), "f"(b2), "f"(0.0f)
                  : "memory");
 }
@@ -398,11 +386,9 @@ __global__ void __launch_bounds__(256) terrain_tile_bounds_strip_k(const TileArg
 // height 1 - v/65535 (Terrain.zig:120) is monotone non-increasing in the texel v, so the minimum height of a tile is the
 // height of its LARGEST texel and vice versa: the reduction runs on the packed u16 pairs (vmaxu2 / vminu2, exact) and
 // only the two results per tile go through the conversion.  A thread takes eight columns with one 128-bit load; four
-// threads share a column group, each taking every fourth row, TB_DEPTH independent loads in flight per thread (rows
+// threads share a column group, each taking every fourth row, TB_LOADS independent loads in flight per thread (rows
 // past the tile repeat its last row, harmless for min / max).
-#ifndef TB_DEPTH
-#define TB_DEPTH 8
-#endif
+constexpr int TB_LOADS = 8;
 __global__ void __launch_bounds__(256) terrain_tile_bounds_wide_k(const TileArgs a, uint32_t tiles_per_cta) {
     __shared__ __align__(16) uint16_t cmin[4][TB_COLS + 8], cmax[4][TB_COLS + 8];
     const uint32_t tr = blockIdx.y, tc0 = blockIdx.x * tiles_per_cta;
@@ -415,13 +401,13 @@ __global__ void __launch_bounds__(256) terrain_tile_bounds_wide_k(const TileArgs
     for (uint32_t g = tx; g < groups; g += 64u) {
         const uint16_t* col = h16 + c_begin + 8u * g;
         uint4 lo = make_uint4(0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu), hi = make_uint4(0u, 0u, 0u, 0u);
-        for (uint32_t r = r0 + ty; r <= r1; r += 4u * TB_DEPTH) {
-            uint4 q[TB_DEPTH];
+        for (uint32_t r = r0 + ty; r <= r1; r += 4u * TB_LOADS) {
+            uint4 q[TB_LOADS];
 #pragma unroll
-            for (int j = 0; j < TB_DEPTH; ++j)
+            for (int j = 0; j < TB_LOADS; ++j)
                 q[j] = __ldg(reinterpret_cast<const uint4*>(col + (size_t)min(r + 4u * j, r1) * a.n));
 #pragma unroll
-            for (int j = 0; j < TB_DEPTH; ++j) {
+            for (int j = 0; j < TB_LOADS; ++j) {
                 lo.x = __vminu2(lo.x, q[j].x), hi.x = __vmaxu2(hi.x, q[j].x);
                 lo.y = __vminu2(lo.y, q[j].y), hi.y = __vmaxu2(hi.y, q[j].y);
                 lo.z = __vminu2(lo.z, q[j].z), hi.z = __vmaxu2(hi.z, q[j].z);

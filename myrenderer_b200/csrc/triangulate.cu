@@ -494,23 +494,12 @@ __device__ __forceinline__ bool angle_clear_of_pi(float dy, float dx) {
 // Same value as is_acute.  When both angles are certainly in [0, pi - 7e-7], |a - b| <= max(a, b) < (f32)pi without
 // evaluating them -- the case of every triangle of a sorted mountain (SURVEY 8-c) except a centre that sees a neighbour
 // within 1e-6 rad of the negative x axis, which takes the exact evaluation.
-#ifdef MR_OUTLINE_COLD
-__noinline__ __device__ bool is_acute_exact_outlined(float2 P, float2 A1, float2 A2) {
-    const float a = dev_atan2f(__fsub_rn(P.y, A1.y), __fsub_rn(P.x, A1.x));
-    const float b = dev_atan2f(__fsub_rn(P.y, A2.y), __fsub_rn(P.x, A2.x));
-    return fabsf(__fsub_rn(a, b)) < __uint_as_float(0x40490fdbu);
-}
-#endif
 __device__ __forceinline__ bool is_acute_shortcut(const float2* pts, uint32_t point, uint32_t axis1, uint32_t axis2) {
     const float2 P = pts[point], A1 = pts[axis1], A2 = pts[axis2];
     if (angle_clear_of_pi(__fsub_rn(P.y, A1.y), __fsub_rn(P.x, A1.x)) &&
         angle_clear_of_pi(__fsub_rn(P.y, A2.y), __fsub_rn(P.x, A2.x)))
         return true;
-#ifdef MR_OUTLINE_COLD
-    return is_acute_exact_outlined(P, A1, A2);
-#else
     return is_acute(pts, point, axis1, axis2);
-#endif
 }
 
 // emit order of Triangulation.zig:405-422; returns ids packed, count in *cnt (3, or 1 when an

@@ -411,7 +411,7 @@ struct FPoly {
     __device__ bool pass2(uint32_t p1, uint32_t up, uint32_t lo, uint32_t lane, uint32_t serial_below) {
         return !MR_SPAN_IS_NULL(gstack) ? pass2_on<true>(p1, up, lo, lane, serial_below) : pass2_on<false>(p1, up, lo, lane, serial_below);
     }
-    // Pass 2 for a stack of K <= 4 entries, written out straight (every lane runs the same code; no loop, no
+    // Pass 2 for a stack of K <= 2 entries, written out straight (every lane runs the same code; no loop, no
     // selection scan).  The loop :325-395 takes the crossed trapezoids in the order of their lower points (highest
     // first) and ends with the one that holds the segment's lower point; each step converts its trapezoid into a
     // segment node and closes the open trapezoid on the side its lower point lies on (:375), opening a new one there.
@@ -423,6 +423,7 @@ struct FPoly {
     // loop as written.
     template <int K>
     __device__ __forceinline__ int pass2_small(uint32_t p1, uint32_t up, uint32_t lo) {
+        static_assert(K <= 2, "three and four entries written out straight measured slower (DESIGN 5.3)");
         const uint32_t A = nnodes;
         const uint32_t cap = min(tier_node_cap, spec_node_cap);
         uint32_t e[K], x[K], np[K];
@@ -450,27 +451,18 @@ struct FPoly {
         }
         nnodes = A + (uint32_t)K + 1u;
         // ascending lower point: the steps in the loop's order, then the entry that holds `lo`
-#define MR_CSWAP(a, b)                                  \
-    {                                                   \
-        const bool sw_ = np[a] > np[b];                 \
-        const uint32_t n_ = sw_ ? np[b] : np[a];        \
-        const uint32_t e_ = sw_ ? e[b] : e[a];          \
-        const uint32_t x_ = sw_ ? x[b] : x[a];          \
-        np[b] = sw_ ? np[a] : np[b];                    \
-        e[b] = sw_ ? e[a] : e[b];                       \
-        x[b] = sw_ ? x[a] : x[b];                       \
-        np[a] = n_;                                     \
-        e[a] = e_;                                      \
-        x[a] = x_;                                      \
-    }
-        if (K == 2) {
-            MR_CSWAP(0, 1)
-        } else if (K == 3) {
-            MR_CSWAP(0, 1) MR_CSWAP(1, 2) MR_CSWAP(0, 1)
-        } else if (K == 4) {
-            MR_CSWAP(0, 1) MR_CSWAP(2, 3) MR_CSWAP(0, 2) MR_CSWAP(1, 3) MR_CSWAP(1, 2)
+        if constexpr (K == 2) {
+            const bool sw = np[0] > np[1];
+            const uint32_t n0 = sw ? np[1] : np[0];
+            const uint32_t e0 = sw ? e[1] : e[0];
+            const uint32_t x0 = sw ? x[1] : x[0];
+            np[1] = sw ? np[0] : np[1];
+            e[1] = sw ? e[0] : e[1];
+            x[1] = sw ? x[0] : x[1];
+            np[0] = n0;
+            e[0] = e0;
+            x[0] = x0;
         }
-#undef MR_CSWAP
         bool is_left[K];  // :375, one independent test per step
 #pragma unroll
         for (int i = 0; i + 1 < K; ++i) is_left[i] = left_of(sxy[np[i]], up, lo);
@@ -497,146 +489,19 @@ struct FPoly {
         return 1;
     }
 
-    // Pass 2 with one lane per stack entry (at most 32).  The loop :325-395 processes the crossed trapezoids in the
-    // order of their lower points (highest first) and ends with the one that holds the segment's lower point; every
-    // step converts its trapezoid into a segment node and closes the open trapezoid on the side its lower point lies
-    // on.  When the lower points above `lo` are pairwise distinct and exactly one entry has a lower point that is not
-    // above `lo` (the case of every consistent trapezoidation), the order is a sort, the node ids are a prefix count
-    // (left = A, right = A + 1, step s allocates A + 2 + s) and every write of the loop is a function of (own entry,
-    // the previous step that closed the same side): all steps can run at once.  Returns 1 done, 0 failed (status /
-    // requeue set as the loop would), -1 when the conditions do not hold (duplicates, null lower points, ...): the
-    // caller then runs the loop as written.
-    // MEASURED (round 2, B200): bit-exact (the whole parity suite passes with MR_PASS2_PAR_MAX = 32) but 4-8 % SLOWER than
-    // the loop on the 8..1024-point batches -- with the 2-3 entries of sound input the ballots, MATCH and shuffle loops
-    // cost more than they save.  Stacks of one and two entries take pass2_small instead; this form is kept behind
-    // MR_PASS2_PAR_MAX (default 0: off) for inputs with long stacks.
-    __device__ __forceinline__ int pass2_parallel(uint32_t p1, uint32_t up, uint32_t lo, uint32_t lane) {
-        const uint32_t k = nstack;
-        const uint32_t A = nnodes;
-        const uint32_t cap = min(tier_node_cap, spec_node_cap);
-        const uint32_t seg_y = up | ((p1 == up) ? 0u : CRUMB_RIGHT) | (T_SEGMENT << 14) | (lo << 16);  // :351-360
-        if (k == 1u) {  // the segment stays inside one trapezoid: it becomes the segment node, both new trapezoids close
-            const uint32_t e = stack[0];
-            const uint2 w = nd[e];
-            const uint32_t np = w.y >> 16;
-            if (np == FNIL || np < lo) return -1;
-            if (A + 2u > cap) {
-                if (cap >= spec_node_cap) status |= MR_POLY_ARENA; else requeue = true;
-                return 0;
-            }
-            nnodes = A + 2u;
-            __syncwarp();
-            nd[e] = make_uint2(A | ((A + 1u) << 16), seg_y);
-            const uint32_t ty = up | (T_TRAPEZOID << 14) | (lo << 16);
-            nd[A] = make_uint2((w.x & 0xFFFFu) | (e << 16), ty);
-            nd[A + 1u] = make_uint2(e | (w.x & 0xFFFF0000u), ty);
-            return 1;
-        }
-#ifndef MR_PASS2_NO_K2
-        if (k == 2u) {  // one trapezoid above the one that holds `lo`: one step plus the final one, written out straight
-            const uint32_t e0 = stack[0], e1 = stack[1];
-            const uint2 w0 = nd[e0], w1 = nd[e1];
-            const uint32_t n0 = w0.y >> 16, n1 = w1.y >> 16;
-            if (n0 == FNIL || n1 == FNIL || ((n0 < lo) == (n1 < lo))) return -1;
-            if (A + 3u > cap) {
-                if (cap >= spec_node_cap) status |= MR_POLY_ARENA; else requeue = true;
-                return 0;
-            }
-            nnodes = A + 3u;
-            const bool first0 = n0 < lo;  // which entry is the step
-            const uint32_t es = first0 ? e0 : e1, ef = first0 ? e1 : e0;
-            const uint32_t xs = first0 ? w0.x : w1.x, xf = first0 ? w1.x : w0.x;
-            const uint32_t nps = first0 ? n0 : n1;
-            const bool is_left = left_of(sxy[nps], up, lo);  // :375
-            const uint32_t t_up = up | (T_TRAPEZOID << 14), t_mid = nps | (T_TRAPEZOID << 14);
-            __syncwarp();
-            nd[es] = make_uint2(A | ((A + 1u) << 16), seg_y);
-            if (is_left) {  // the left trapezoid closes at the step; a new one (A + 2) runs down to `lo`
-                nd[A] = make_uint2((xs & 0xFFFFu) | (es << 16), t_up | (nps << 16));
-                nd[A + 2u] = make_uint2((xf & 0xFFFFu) | (ef << 16), t_mid | (lo << 16));
-                nd[A + 1u] = make_uint2(ef | (xf & 0xFFFF0000u), t_up | (lo << 16));
-                nd[ef] = make_uint2((A + 2u) | ((A + 1u) << 16), seg_y);
-            } else {
-                nd[A + 1u] = make_uint2(es | (xs & 0xFFFF0000u), t_up | (nps << 16));
-                nd[A + 2u] = make_uint2(ef | (xf & 0xFFFF0000u), t_mid | (lo << 16));
-                nd[A] = make_uint2((xf & 0xFFFFu) | (ef << 16), t_up | (lo << 16));
-                nd[ef] = make_uint2(A | ((A + 2u) << 16), seg_y);
-            }
-            return 1;
-        }
-#endif
-        const bool act = lane < k;
-        const uint32_t e = act ? stack[lane] : 0u;
-        const uint2 w = nd[e];
-        const uint32_t np = w.y >> 16;
-        const bool in_s = act && np < lo;  // lower point strictly above `lo`: a step of its own
-        const uint32_t ms = __ballot_sync(0xFFFFFFFFu, in_s);
-        const uint32_t mr = __ballot_sync(0xFFFFFFFFu, act && !in_s);
-        const uint32_t same = __match_any_sync(0xFFFFFFFFu, in_s ? np : (0x10000u + lane));
-        const bool odd = (act && np == FNIL) || (same & (same - 1u)) != 0u;
-        if (__any_sync(0xFFFFFFFFu, odd) || __popc(mr) != 1) return -1;
-        const uint32_t m = __popc(ms);
-        if (A + 2u + m > cap) {  // the loop's failing add_node sees nnodes == cap
-            if (cap >= spec_node_cap) status |= MR_POLY_ARENA; else requeue = true;
-            return 0;
-        }
-        nnodes = A + 2u + m;
-        // step index: rank of the lower point among the steps; the entry holding `lo` comes last
-        uint32_t s = 0;
-        for (uint32_t j = 0; j < k; ++j) {
-            const uint32_t vj = __shfl_sync(0xFFFFFFFFu, np, j);
-            s += (((ms >> j) & 1u) && vj < np) ? 1u : 0u;
-        }
-        if (!in_s) s = m;
-        // :375 the side the step's lower point lies on
-        const bool is_left = in_s && left_of(sxy[np], up, lo);
-        const uint32_t ml = __ballot_sync(0xFFFFFFFFu, is_left);
-        // the previous step that closed (and re-opened) each side: largest step index below mine
-        uint32_t pl = 0, pr = 0;  // (step + 1) << 16 | lower point; 0 = none: the trapezoids allocated up front
-        for (uint32_t j = 0; j < k; ++j) {
-            const uint32_t sj = __shfl_sync(0xFFFFFFFFu, s, j);
-            const uint32_t vj = __shfl_sync(0xFFFFFFFFu, np, j);
-            if (((ms >> j) & 1u) && sj < s) {
-                const uint32_t key = ((sj + 1u) << 16) | vj;
-                if ((ml >> j) & 1u) pl = max(pl, key); else pr = max(pr, key);
-            }
-        }
-        const uint32_t left_id = pl ? A + 1u + (pl >> 16) : A;            // A + 2 + step
-        const uint32_t right_id = pr ? A + 1u + (pr >> 16) : A + 1u;
-        const uint32_t left_p1 = pl ? (pl & 0xFFFFu) : up;
-        const uint32_t right_p1 = pr ? (pr & 0xFFFFu) : up;
-        __syncwarp();
-        if (act) {
-            nd[e] = make_uint2(left_id | (right_id << 16), seg_y);                 // :347-360
-            const uint32_t low = in_s ? np : lo;
-            if (!in_s || is_left)                                                   // :366-369, :375-378
-                nd[left_id] = make_uint2((w.x & 0xFFFFu) | (e << 16), left_p1 | (T_TRAPEZOID << 14) | (low << 16));
-            if (!in_s || !is_left)                                                  // :370-372, :383-386
-                nd[right_id] = make_uint2(e | (w.x & 0xFFFF0000u), right_p1 | (T_TRAPEZOID << 14) | (low << 16));
-        }
-        return 1;
-    }
-
-#ifndef MR_PASS2_SMALL_MAX
-#define MR_PASS2_SMALL_MAX 2u  // straight-line pass 2 for stacks of up to this many entries (<= 4; measured: 2 best overall, see DESIGN 5.3)
-#endif
-#ifndef MR_PASS2_PAR_MAX
-#define MR_PASS2_PAR_MAX 0u  // lane-parallel pass 2 up to this many entries: measured slower than the loop (see its note)
-#endif
     template <bool GLOBAL>
     __device__ bool pass2_on(uint32_t p1, uint32_t up, uint32_t lo, uint32_t lane, uint32_t serial_below) {
-        if (!GLOBAL && nstack <= MR_PASS2_SMALL_MAX && nstack > 0u) {
-            int r;
-            switch (nstack) {
-                case 1: r = pass2_small<1>(p1, up, lo); break;
-                case 2: r = pass2_small<2>(p1, up, lo); break;
-                case 3: r = pass2_small<3>(p1, up, lo); break;
-                default: r = pass2_small<4>(p1, up, lo); break;
+        // Stacks of one and two entries written out straight (measured: up to two beats up to three and four, DESIGN
+        // 5.3).  Each size returns on its own: one `r` for both sizes costs the team kernels 16 bytes of spill at their
+        // 80-register cap.
+        if (!GLOBAL && nstack <= 2u && nstack > 0u) {
+            if (nstack == 1u) {
+                const int r = pass2_small<1>(p1, up, lo);
+                if (r >= 0) return r != 0;
+            } else {
+                const int r = pass2_small<2>(p1, up, lo);
+                if (r >= 0) return r != 0;
             }
-            if (r >= 0) return r != 0;
-        } else if (!GLOBAL && nstack <= MR_PASS2_PAR_MAX && nstack > 0u) {
-            const int r = pass2_parallel(p1, up, lo, lane);
-            if (r >= 0) return r != 0;
         }
         MR_SPAN(uint16_t) stk = GLOBAL ? gstack : stack;
         // The two open trapezoids live in registers until they are closed.
@@ -1260,17 +1125,12 @@ __device__ int process_polygon_fast(const BatchArgs& a, uint32_t pi, unsigned ch
 
     // ---- conflict lists of the pending edges (items tier) ---------------------------------------------
     constexpr bool use_items = ITEMS;
-#ifndef MR_TEAM_LOC_DIV
-#define MR_TEAM_LOC_DIV 64u
-#endif
-#ifndef MR_TEAM_ITEM_MULT
-#define MR_TEAM_ITEM_MULT 3u
-#endif
     // the caches are refreshed every refresh_every edges, the conflict lists every item_mult-th refresh (single warp:
     // measured best of 1/2/4/8 on n <= 1024); countdowns instead of `at % period` (a run-time modulo per edge)
     // (without conflict lists -- n <= 64 and the retry tiers -- every 4th edge measured best of 1/2/3/4/6/8/16)
-    const uint32_t refresh_every = W > 1 ? (n + MR_TEAM_LOC_DIV - 1u) / MR_TEAM_LOC_DIV : (!ITEMS ? 4u * ((n + 63u) / 64u) : (n + 63u) / 64u);
-    const uint32_t item_mult = W > 1 ? MR_TEAM_ITEM_MULT : 4u;
+    // (teams: caches every n/64 edges measured best of n/32..n/128, lists every 3rd refresh best of 2/3/4/8, DESIGN 5.3)
+    const uint32_t refresh_every = W > 1 ? (n + 63u) / 64u : (!ITEMS ? 4u * ((n + 63u) / 64u) : (n + 63u) / 64u);
+    const uint32_t item_mult = W > 1 ? 3u : 4u;
     uint32_t refresh_wait = 0, item_wait = 0;
     const FItems I = fast_items(ws, L, caps);
     MR_SPAN(uint16_t) it_node = I.it_node;
@@ -1319,13 +1179,7 @@ __device__ int process_polygon_fast(const BatchArgs& a, uint32_t pi, unsigned ch
     const bool ur_simple = ur_offset < n && ur_prime < n;
     uint32_t ur_edge = ur_offset;
     bool ok = true;
-#ifdef MR_DEBUG_ITEMS
-    uint32_t dbg_freed = 0, dbg_maxlive = 0;
-#endif
     for (uint32_t at = 0; at < n && ok; ++at) {  // :484-494
-#ifdef MR_DEBUG_ITEMS
-        if (use_items) dbg_maxlive = max(dbg_maxlive, ctr[0] - dbg_freed);
-#endif
         const bool refresh_now = refresh_wait == 0u;
         refresh_wait = refresh_now ? refresh_every - 1u : refresh_wait - 1u;
         const bool items_now = use_items && refresh_now && item_wait == 0u;
@@ -1452,9 +1306,6 @@ __device__ int process_polygon_fast(const BatchArgs& a, uint32_t pi, unsigned ch
             P.nstack = 0;
             bool first_item = true;
             while (it != FNIL && ok) {
-#ifdef MR_DEBUG_ITEMS
-                ++dbg_freed;
-#endif
                 uint32_t node = first_item ? it_node0 : it_node[it];
                 uint32_t nxt = first_item ? it_next0 : it_next[it];
                 first_item = false;
@@ -1514,10 +1365,6 @@ __device__ int process_polygon_fast(const BatchArgs& a, uint32_t pi, unsigned ch
         ok = P.pass2(p1, up, lo, lane, 16u);  // pass 2: scan as written below 16 entries, REDUX arg-min above
         __syncwarp();
     }
-#ifdef MR_DEBUG_ITEMS
-    if (use_items && lane == 0 && (pi % 97u) == 0u)
-        printf("DBG n %u created %u maxlive %u nodes %u requeue %d\n", n, ctr[0], dbg_maxlive, P.nnodes, (int)P.requeue);
-#endif
     if (P.requeue) return F_REQUEUE_SPEC;
     if (!ok) {
         res->status = P.status | (sink.cap_vtx ? MR_POLY_UNDERFILL : 0u);
