@@ -364,6 +364,67 @@ int mr_triangulate_earclip(mr_context* ctx, const mr_polygon_job* job);
 /* Self-test used by the test-suite: sign_out[i] = orient of the triple abc[6i..6i+5] = (ax, ay, bx, by, cx, cy), as
  * mr_triangulate_earclip evaluates it (-1, 0, +1). */
 int mr_selftest_orient(mr_context* ctx, const float* abc /* 6 per triple */, uint64_t count, int8_t* sign_out);
+/* ---- ear clipping of polygons with holes ---------------------------------------------------------------------
+ * mr_triangulate_earclip_holes triangulates polygons whose point range holds several rings: an outer boundary and holes.
+ * The job, its checks, alignment, layouts, host / device pointers, sub-ranges, optional outputs, palette, bbox rule and
+ * OVERFLOW / UNDERFILL rule are those of mr_triangulate_earclip, with the triangle count T = N + 2H - 2 in place of
+ * n - 2 (N points, H holes; see mr_polygon_offsets_rings).  The rings of polygon i are first_ring[i] ..
+ * first_ring[i+1]-1; ring r starts at point ring_start[r - ring_base] and ends where the next ring starts (the last one
+ * at first_point[i+1]).  first_ring and ring_start may be device or host pointers (host ones are staged like
+ * first_point).  The ring arrays are read per polygon inside the kernel, so bad ring data is a polygon status, not an
+ * MR_E_BADARG.  Checks, in this order, each written as mr_triangulate_earclip writes a reject (range zeroed, ntri 0,
+ * bbox +0):
+ *   R = first_ring[i+1] - first_ring[i] (as uint64) is 0 or larger than N:                     MR_POLY_DEGENERATE
+ *   N + 2(R-1) > MR_MAX_POLYGON_POINTS:                                                          MR_POLY_TOO_LARGE
+ *   the first ring start differs from first_point[i], ring starts do not increase, or a ring has fewer than 3 points:
+ *                                                                                                MR_POLY_DEGENERATE
+ *   a NaN / +-inf coordinate on either axis of any point:                                        MR_POLY_NONFINITE
+ * Bit for bit (orient, a == b and the winding rule as for mr_triangulate_earclip):
+ *   s = the winding of the outer ring; each hole has its own winding by the same rule.  M(h) = the first point of hole
+ *   h largest in (x, y).  Holes are merged one at a time in decreasing (x, y) of M(h), equal M in hole order, into the
+ *   current ring C (initially the outer ring, positions 0..L-1 in ring order).  For hole h with M = M(h), y = My:
+ *   1. Crossing edges: ring edges (C[k], C[k+1]) = (a, b) with s*(b.y - a.y) > 0, min(a.y, b.y) <= My <= max(a.y, b.y)
+ *      and s*orient(a, b, M) >= 0.  Edge 2 crosses nearer than edge 1 when
+ *        cross(a1, b1, a2, b2, My) = sign of the EXACT (b2.y - My)*O(a1,b1,a2) + (My - a2.y)*O(a1,b1,b2) > 0
+ *      (O the exact orient value; mr_selftest_crossing exposes the device's predicate).  The nearest edge k is the one
+ *      with the smallest crossing x (the order cross() decides), the first in position order among equal crossings.
+ *      No crossing edge: the hole is bridged to position 0 and MR_POLY_BAD_HOLE is set.
+ *   2. Target t: if a.y == My then t = k; else if b.y == My then t = k+1; else t = k if a.x >= b.x else k+1, and with
+ *      u = sign(P[t].y - My), every position r whose point differs from M, whose vertex is not strictly convex
+ *      (s*orient(C[r-1], C[r], C[r+1]) <= 0) and which lies in the closed triangle (M, crossing point, P[t]) -- u*sign(P[r].y - My) >= 0, s*orient(a, b, r) >= 0,
+ *      u*orient(M, P[t], r) <= 0 -- replaces t, in position order, if u*orient(M, r, t) > 0, or it is 0 and
+ *      P[r].x < P[t].x (smallest angle to the ray, then nearest).
+ *   3. Copy: the first position k' (in position order) whose point equals P[t] and whose wedge contains M:
+ *      s*orient(C[k'-1], P[t], C[k'+1]) > 0 ? (s*orient(C[k'-1], P[t], M) > 0 and s*orient(P[t], C[k'+1], M) > 0)
+ *                                           : (s*orient(C[k'-1], P[t], M) > 0 or  s*orient(P[t], C[k'+1], M) > 0);
+ *      t itself when there is none.
+ *   4. Splice after position k': C[0..k'], M and the rest of the hole from M on (in reverse ring order if the hole's
+ *      winding equals s), M again, C[k'] again, C[k'+1..L-1].
+ *   The merged ring of N + 2H points is then clipped exactly as mr_triangulate_earclip clips a ring of that many points:
+ *   its own winding, ring walk, rules (a) and (b), emit order and NO_EAR fallback, unchanged.  (Rule (b)'s point-equality
+ *   exclusion keeps the two copies of a bridge endpoint from blocking each other's ears.)  With H = 0 the result is
+ *   mr_triangulate_earclip's, byte for byte.
+ * Properties: for valid input -- outer ring and holes simple, holes strictly inside the outer ring and pairwise
+ * disjoint -- neither MR_POLY_NO_EAR nor MR_POLY_BAD_HOLE is set and the N + 2H - 2 triangles tile the polygon with its
+ * holes removed, every one with orientation >= 0 in raw (x, y).  Any other input still gets T triangles and a defined,
+ * bit-exact result.  Cost: the merge is O(H * (N + 2H)) predicate evaluations per polygon, the clip that of a ring of
+ * N + 2H points. */
+#define MR_POLY_BAD_HOLE 512u /* mr_triangulate_earclip_holes only: no ring edge crossed a hole's ray (a hole outside the ring) */
+typedef struct mr_polygon_rings {
+    const uint64_t* first_ring; /* npoly+1 entries: polygon i owns rings first_ring[i] .. first_ring[i+1]-1 */
+    uint64_t ring_base;         /* ring_start is indexed by (ring - ring_base), like point_base / tri_base */
+    const uint64_t* ring_start; /* absolute point index of each ring's first point; a polygon's first ring starts at
+                                   first_point[i] and is its outer boundary, the others are holes */
+} mr_polygon_rings;
+int mr_triangulate_earclip_holes(mr_context* ctx, const mr_polygon_job* job, const mr_polygon_rings* rings);
+/* Self-test used by the test-suite: sign_out[i] = cross(a1, b1, a2, b2, My) above for q[9i..9i+8] =
+ * (a1x, a1y, b1x, b1y, a2x, a2y, b2x, b2y, My), as mr_triangulate_earclip_holes evaluates it (-1, 0, +1). */
+int mr_selftest_crossing(mr_context* ctx, const float* q /* 9 per case */, uint64_t count, int8_t* sign_out);
+/* first_tri[0..npoly] for mr_triangulate_earclip_holes: the exclusive prefix sum of max(N + 2H - 2, 0) with
+ * H = first_ring[i+1] - first_ring[i] - 1 when 1 <= first_ring[i+1] - first_ring[i] <= N, else H = 0 (device or host
+ * pointers, like mr_polygon_offsets). */
+int mr_polygon_offsets_rings(mr_context* ctx, const uint64_t* first_point, const uint64_t* first_ring, uint32_t npoly,
+                             uint64_t* first_tri_out);
 /* first_tri[0..npoly] from first_point[0..npoly] (device or host pointers). */
 int mr_polygon_offsets(mr_context* ctx, const uint64_t* first_point, uint32_t npoly,
                        uint64_t* first_tri_out);

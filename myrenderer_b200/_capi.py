@@ -30,6 +30,8 @@ MR_POLY_STUCK = 16
 MR_POLY_TOO_LARGE = 32
 MR_POLY_ARENA = 64
 MR_POLY_UNDERFILL = 128
+MR_POLY_NO_EAR = 256
+MR_POLY_BAD_HOLE = 512
 
 ERROR_NAMES = {-1: "MR_E_BADARG", -2: "MR_E_CUDA", -3: "MR_E_NOMEM", -4: "MR_E_ARENA"}
 
@@ -94,6 +96,10 @@ class MrPolygonJob(C.Structure):
     ]
 
 
+class MrPolygonRings(C.Structure):
+    _fields_ = [("first_ring", C.c_void_p), ("ring_base", C.c_uint64), ("ring_start", C.c_void_p)]
+
+
 class MrError(RuntimeError):
     def __init__(self, code: int, where: str, detail: str = ""):
         self.code = code
@@ -140,6 +146,9 @@ SIGNATURES = {
     "mr_triangulate_batch": (C.c_int, [C.c_void_p, C.POINTER(MrPolygonJob)]),
     "mr_triangulate_earclip": (C.c_int, [C.c_void_p, C.POINTER(MrPolygonJob)]),
     "mr_selftest_orient": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
+    "mr_triangulate_earclip_holes": (C.c_int, [C.c_void_p, C.POINTER(MrPolygonJob), C.POINTER(MrPolygonRings)]),
+    "mr_selftest_crossing": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
+    "mr_polygon_offsets_rings": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]),
     "mr_polygon_offsets": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]),
     "mr_triangulate_tier_counts": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint32)]),
     "mr_polygon_draw_range": (

@@ -502,6 +502,30 @@ int mr_polygon_offsets(mr_context* ctx, const uint64_t* first_point, uint32_t np
     return mr_finish_host_io(ctx);
 }
 
+int mr_polygon_offsets_rings(mr_context* ctx, const uint64_t* first_point, const uint64_t* first_ring, uint32_t npoly,
+                             uint64_t* first_tri_out) {
+    if (!ctx || !first_point || !first_ring || !first_tri_out) return MR_E_BADARG;
+    MR_CUDA(ctx, cudaSetDevice(ctx->device));
+    const void* dfp = nullptr;
+    int rc = mr_stage_in(ctx, 1, first_point, (size_t)(npoly + 1) * 8, &dfp);
+    if (rc) return rc;
+    const void* dfr = nullptr;
+    rc = mr_stage_in(ctx, 14, first_ring, (size_t)(npoly + 1) * 8, &dfr);
+    if (rc) return rc;
+    void* dft = nullptr;
+    bool st = false;
+    rc = mr_stage_out(ctx, 2, first_tri_out, (size_t)(npoly + 1) * 8, &dft, &st);
+    if (rc) return rc;
+    rc = mr_polygon_ring_counts(ctx, static_cast<const uint64_t*>(dfp), static_cast<const uint64_t*>(dfr), npoly, 2,
+                                static_cast<uint64_t*>(dft));
+    if (rc) return rc;
+    if (st) {
+        rc = mr_copy_back(ctx, first_tri_out, dft, (size_t)(npoly + 1) * 8);
+        if (rc) return rc;
+    }
+    return mr_finish_host_io(ctx);
+}
+
 int mr_polygon_draw_range(uint64_t first_tri_i, uint64_t first_tri_next, uint64_t tri_base, mr_draw_range* out) {
     if (!out || first_tri_next < first_tri_i || first_tri_i < tri_base) return MR_E_BADARG;
     const uint64_t prims = first_tri_next - first_tri_i, off = first_tri_i - tri_base;
@@ -514,10 +538,11 @@ int mr_polygon_draw_range(uint64_t first_tri_i, uint64_t first_tri_next, uint64_
 }
 
 namespace {
-// mr_triangulate_batch and mr_triangulate_earclip: the same checks, staging and copy-back; ear clipping takes no edge
-// order and has no small-batch path.
-int triangulate_common(mr_context* ctx, const mr_polygon_job* job, bool earclip) {
+// mr_triangulate_batch, mr_triangulate_earclip and mr_triangulate_earclip_holes (rings != nullptr): the same checks,
+// staging and copy-back; ear clipping takes no edge order and has no small-batch path.
+int triangulate_common(mr_context* ctx, const mr_polygon_job* job, bool earclip, const mr_polygon_rings* rings = nullptr) {
     if (!ctx || !job) return MR_E_BADARG;
+    if (rings && (!rings->first_ring || !rings->ring_start) && job->npoly) return mr_fail(ctx, MR_E_BADARG, "polygons: null ring pointer");
     const mr_polygon_job& j = *job;
     if (j.npoly == 0) return MR_OK;
     if (!j.xy || !j.first_point || !j.first_tri || !j.vtx_out) return mr_fail(ctx, MR_E_BADARG, "polygons: null pointer");
@@ -574,6 +599,29 @@ int triangulate_common(mr_context* ctx, const mr_polygon_job* job, bool earclip)
         if (rc) return rc;
         d.offset_prime = static_cast<const uint32_t*>(p);
     }
+    mr_polygon_rings dr{};
+    if (rings) {
+        // ring_start covers [ring_base, first_ring[npoly]): its size is needed only when it lives on the host
+        uint64_t nrings = 0;
+        if (!mr_is_device_ptr(rings->ring_start)) {
+            uint64_t fr_end = 0;
+            if (mr_is_device_ptr(rings->first_ring)) {
+                MR_CUDA(ctx, cudaMemcpyAsync(&fr_end, rings->first_ring + j.npoly, 8, cudaMemcpyDeviceToHost, ctx->stream));
+                MR_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+            } else {
+                fr_end = rings->first_ring[j.npoly];
+            }
+            if (fr_end < rings->ring_base) return mr_fail(ctx, MR_E_BADARG, "polygons: ring_base beyond the last ring");
+            nrings = fr_end - rings->ring_base;
+        }
+        dr.ring_base = rings->ring_base;
+        rc = mr_stage_in(ctx, 14, rings->first_ring, (size_t)(j.npoly + 1) * 8, &p);
+        if (rc) return rc;
+        dr.first_ring = static_cast<const uint64_t*>(p);
+        rc = mr_stage_in(ctx, 15, rings->ring_start, (size_t)nrings * 8, &p);
+        if (rc) return rc;
+        dr.ring_start = static_cast<const uint64_t*>(p);
+    }
     bool sv = false, sb = false, ss = false, sn = false;
     void* q = nullptr;
     const size_t vbytes = (size_t)ntri * 3u * j.layout.stride;
@@ -603,7 +651,9 @@ int triangulate_common(mr_context* ctx, const mr_polygon_job* job, bool earclip)
         if (rc) return rc;
         d.ntri_out = static_cast<uint32_t*>(q);
     }
-    rc = earclip ? mr_triangulate_earclip_impl(ctx, &d) : mr_triangulate_impl(ctx, &d, fp_dev ? nullptr : j.first_point);
+    rc = rings     ? mr_triangulate_earclip_holes_impl(ctx, &d, &dr)
+         : earclip ? mr_triangulate_earclip_impl(ctx, &d)
+                   : mr_triangulate_impl(ctx, &d, fp_dev ? nullptr : j.first_point);
     if (rc) return rc;
     if (sv) {
         // the polygons of this job own [first_tri[0], first_tri[npoly]) only
@@ -626,6 +676,30 @@ int triangulate_common(mr_context* ctx, const mr_polygon_job* job, bool earclip)
 int mr_triangulate_batch(mr_context* ctx, const mr_polygon_job* job) { return triangulate_common(ctx, job, false); }
 
 int mr_triangulate_earclip(mr_context* ctx, const mr_polygon_job* job) { return triangulate_common(ctx, job, true); }
+
+int mr_triangulate_earclip_holes(mr_context* ctx, const mr_polygon_job* job, const mr_polygon_rings* rings) {
+    if (!rings) return MR_E_BADARG;
+    return triangulate_common(ctx, job, true, rings);
+}
+
+int mr_selftest_crossing(mr_context* ctx, const float* q, uint64_t count, int8_t* sign_out) {
+    if (!ctx || (count && (!q || !sign_out))) return MR_E_BADARG;
+    MR_CUDA(ctx, cudaSetDevice(ctx->device));
+    const void* din = nullptr;
+    int rc = mr_stage_in(ctx, 0, q, (size_t)count * 36, &din);
+    if (rc) return rc;
+    void* dout = nullptr;
+    bool st = false;
+    rc = mr_stage_out(ctx, 4, sign_out, (size_t)count, &dout, &st);
+    if (rc) return rc;
+    rc = mr_selftest_crossing_impl(ctx, static_cast<const float*>(din), count, static_cast<int8_t*>(dout));
+    if (rc) return rc;
+    if (st) {
+        rc = mr_copy_back(ctx, sign_out, dout, (size_t)count);
+        if (rc) return rc;
+    }
+    return mr_finish_host_io(ctx);
+}
 
 int mr_selftest_orient(mr_context* ctx, const float* abc, uint64_t count, int8_t* sign_out) {
     if (!ctx || (count && (!abc || !sign_out))) return MR_E_BADARG;

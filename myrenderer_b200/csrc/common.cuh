@@ -10,7 +10,7 @@
 #include <vector>
 #include "../../include/myrenderer_b200.h"
 
-#define MR_NUM_SCRATCH 14
+#define MR_NUM_SCRATCH 16
 
 constexpr int MR_NUM_AUX = 12;
 
@@ -193,3 +193,9 @@ int mr_polygon_size_sort(mr_context* ctx, const uint64_t* first_point, uint32_t 
 // ear clipping (earclip.cu); pointers as for mr_triangulate_impl
 int mr_triangulate_earclip_impl(mr_context* ctx, const mr_polygon_job* job);
 int mr_selftest_orient_impl(mr_context* ctx, const float* abc, uint64_t count, int8_t* sign_out);
+int mr_triangulate_earclip_holes_impl(mr_context* ctx, const mr_polygon_job* job, const mr_polygon_rings* rings);
+int mr_selftest_crossing_impl(mr_context* ctx, const float* q, uint64_t count, int8_t* sign_out);
+// out[0..npoly]: exclusive prefix sum of max(N + 2H - sub, 0) with H as for mr_polygon_offsets_rings (triangulate.cu;
+// sub 2: first_tri, sub 0: the merged ring sizes the ear-clip size classes key on); device pointers
+int mr_polygon_ring_counts(mr_context* ctx, const uint64_t* first_point, const uint64_t* first_ring, uint32_t npoly,
+                           uint32_t sub, uint64_t* out);

@@ -4,7 +4,8 @@
 // polygon; the ring (points, prev/next links, a flag byte per point) and the list of vertices that can block an ear
 // live in shared memory, 15 bytes per point.  Polygons are pulled largest first from four size classes.  The ring walk
 // is warp-uniform (every lane holds the same cursor); the blocker scan of a candidate runs lane-parallel over the list
-// of non-convex vertices, behind an exact bounding-box reject.
+// of non-convex vertices, behind an exact bounding-box reject.  mr_triangulate_earclip_holes first bridges a polygon's
+// holes into its outer ring in the same workspace (merge_holes) and then runs the same ring walk on the merged ring.
 #include "common.cuh"
 
 namespace {
@@ -36,6 +37,13 @@ struct EcArgs {
     const uint32_t* order;          // polygon ids, largest first
     const uint32_t* cursor;         // cursor[b] = polygons of size >= b (mr_polygon_size_sort)
     uint32_t* queue_head;           // EC_CLASSES
+};
+
+// ring description of mr_triangulate_earclip_holes (device pointers)
+struct RingArgs {
+    const uint64_t* first_ring;
+    uint64_t ring_base;
+    const uint64_t* ring_start;
 };
 
 // ---- exact orientation ---------------------------------------------------------------------------------------
@@ -229,7 +237,267 @@ __device__ uint32_t clip_ring(const Ring& R, uint32_t n, Emit& em, uint32_t lane
     return status;
 }
 
-__device__ void earclip_polygon(const EcArgs& a, uint32_t pi, const Ring& R, uint32_t lane) {
+// ---- holes: the crossing predicate and the bridge merge (mr_triangulate_earclip_holes) ------------------------------
+__device__ __forceinline__ void two_prod(double a, double b, double& p, double& e) {
+    p = __dmul_rn(a, b);
+    e = __fma_rn(a, b, -p);
+}
+
+// Sign of (b2y - my)*O(a1,b1,a2) + (my - a2y)*O(a1,b1,b2) expanded into 24 products of three floats: the first two
+// multiply exactly in double, the third by two_prod; the 48 terms are summed by grow-expansion.
+__device__ __noinline__ int cross_exact(float2 a1, float2 b1, float2 a2, float2 b2, float my) {
+    const double o1[6] = {__dmul_rn(a1.x, b1.y), -__dmul_rn(a1.x, a2.y), __dmul_rn(b1.x, a2.y),
+                          -__dmul_rn(b1.x, a1.y), __dmul_rn(a2.x, a1.y), -__dmul_rn(a2.x, b1.y)};
+    const double o2[6] = {__dmul_rn(a1.x, b1.y), -__dmul_rn(a1.x, b2.y), __dmul_rn(b1.x, b2.y),
+                          -__dmul_rn(b1.x, a1.y), __dmul_rn(b2.x, a1.y), -__dmul_rn(b2.x, b1.y)};
+    const double f1[2] = {b2.y, -(double)my}, f2[2] = {my, -(double)a2.y};
+    double e[48];
+    int n = 0;
+    for (int k = 0; k < 6; ++k)
+        for (int i = 0; i < 2; ++i) {
+            double t[4];
+            two_prod(o1[k], f1[i], t[0], t[1]);
+            two_prod(o2[k], f2[i], t[2], t[3]);
+            for (int u = 0; u < 4; ++u) {
+                double q = t[u];
+                for (int m = 0; m < n; ++m) two_sum(q, e[m], q, e[m]);
+                e[n++] = q;
+            }
+        }
+    for (int i = 47; i >= 0; --i)
+        if (e[i] != 0.0) return e[i] > 0.0 ? 1 : -1;
+    return 0;
+}
+
+// Exact sign of the crossing comparison of the header.  Filter: the value in double, with the differences of floats
+// and the two orient determinants rounded once each; its error is below 8 * 2^-53 * S (S the sum of the magnitudes of
+// the two products), nothing underflows (every nonzero term is at least 2^-447) and S == 0 means the value is 0.
+__device__ __forceinline__ int cross_sign(float2 a1, float2 b1, float2 a2, float2 b2, float my) {
+    const double l1 = __dmul_rn(__dsub_rn(a1.x, a2.x), __dsub_rn(b1.y, a2.y)), r1 = __dmul_rn(__dsub_rn(a1.y, a2.y), __dsub_rn(b1.x, a2.x));
+    const double l2 = __dmul_rn(__dsub_rn(a1.x, b2.x), __dsub_rn(b1.y, b2.y)), r2 = __dmul_rn(__dsub_rn(a1.y, b2.y), __dsub_rn(b1.x, b2.x));
+    const double f1 = __dsub_rn(b2.y, my), f2 = __dsub_rn(my, a2.y);
+    const double d = __dadd_rn(__dmul_rn(f1, __dsub_rn(l1, r1)), __dmul_rn(f2, __dsub_rn(l2, r2)));
+    const double S = __dadd_rn(__dmul_rn(fabs(f1), __dadd_rn(fabs(l1), fabs(r1))), __dmul_rn(fabs(f2), __dadd_rn(fabs(l2), fabs(r2))));
+    const double bound = 16.0 * 0x1p-53 * S;
+    if (d > bound) return 1;
+    if (-d > bound) return -1;
+    if (S == 0.0) return 0;
+    return cross_exact(a1, b1, a2, b2, my);
+}
+
+__device__ __forceinline__ int cmpf(float a, float b) { return (a > b) - (a < b); }
+__device__ __forceinline__ bool above_xy(float2 a, float2 b) { return a.x > b.x || (a.x == b.x && a.y > b.y); }
+__device__ __forceinline__ uint32_t wrap(uint32_t k, uint32_t L) { return k >= L ? k - L : k; }
+
+// winding of the ring R.P[a .. a+n) by the lowest-vertex rule (warp-uniform)
+__device__ int ring_winding(const Ring& R, uint32_t a, uint32_t n, uint32_t lane) {
+    uint32_t m = 0;
+    for (uint32_t i = lane; i < n; i += 32)
+        if (i == lane || below_yx(R.P[a + i], R.P[a + m])) m = i;
+    if (lane >= n) m = 0;
+#pragma unroll
+    for (int d = 16; d >= 1; d >>= 1) {
+        const uint32_t o = __shfl_xor_sync(0xFFFFFFFFu, m, d);
+        const float2 po = R.P[a + o], pm = R.P[a + m];
+        if (below_yx(po, pm) || (!below_yx(pm, po) && o < m)) m = o;
+    }
+    const float2 pmv = R.P[a + m];
+    uint32_t nb[2] = {n, n};
+    for (int dir = 0; dir < 2; ++dir)
+        for (uint32_t base = 1; base < n; base += 32) {
+            const uint32_t dd = base + lane;
+            const uint32_t i = dir == 0 ? (m + n - dd % n) % n : (m + dd) % n;
+            const uint32_t hit = __ballot_sync(0xFFFFFFFFu, dd < n && !same_pt(R.P[a + i], pmv));
+            if (hit) {
+                const uint32_t k = base + __ffs(hit) - 1u;
+                nb[dir] = dir == 0 ? (m + n - k) % n : (m + k) % n;
+                break;
+            }
+        }
+    if (nb[0] == n) return 1;
+    const int o = orient(R.P[a + nb[0]], pmv, R.P[a + nb[1]]);
+    return o ? o : 1;
+}
+
+// Position of the current ring (point ids R.lst[0..L), points R.P) that the hole vertex M is bridged to (steps 1-3 of the
+// header); bad = no edge crosses the ray.  Warp-uniform.
+__device__ uint32_t bridge_pos(const Ring& R, uint32_t L, float2 M, int s, uint32_t lane, bool& bad) {
+    constexpr uint32_t NONE = 0xFFFFFFFFu;
+    const float my = M.y;
+    // 1. nearest crossing edge: lane-local scan in position order, then a butterfly under (crossing x, position)
+    uint32_t e = NONE;
+    float2 ea = M, eb = M;
+    for (uint32_t k = lane; k < L; k += 32) {
+        const float2 a = R.P[R.lst[k]], b = R.P[R.lst[wrap(k + 1u, L)]];
+        if (s * cmpf(b.y, a.y) <= 0 || !(fminf(a.y, b.y) <= my && my <= fmaxf(a.y, b.y)) || s * orient(a, b, M) < 0) continue;
+        if (e == NONE || cross_sign(ea, eb, a, b, my) > 0) {
+            e = k;
+            ea = a;
+            eb = b;
+        }
+    }
+#pragma unroll
+    for (int d = 16; d >= 1; d >>= 1) {
+        const uint32_t o = __shfl_xor_sync(0xFFFFFFFFu, e, d);
+        const float2 oa = make_float2(__shfl_xor_sync(0xFFFFFFFFu, ea.x, d), __shfl_xor_sync(0xFFFFFFFFu, ea.y, d));
+        const float2 ob = make_float2(__shfl_xor_sync(0xFFFFFFFFu, eb.x, d), __shfl_xor_sync(0xFFFFFFFFu, eb.y, d));
+        if (o == NONE) continue;
+        int w = 1;
+        if (e != NONE) {
+            w = cross_sign(ea, eb, oa, ob, my);
+            if (w == 0) w = o < e ? 1 : -1;
+        }
+        if (w > 0) {
+            e = o;
+            ea = oa;
+            eb = ob;
+        }
+    }
+    bad = e == NONE;
+    if (bad) return 0;
+    // 2. target
+    uint32_t t;
+    if (ea.y == my) {
+        t = e;
+    } else if (eb.y == my) {
+        t = wrap(e + 1u, L);
+    } else {
+        t = ea.x >= eb.x ? e : wrap(e + 1u, L);
+        const float2 Pt = R.P[R.lst[t]];
+        const int u = Pt.y > my ? 1 : -1;
+        uint32_t c = NONE;
+        float2 pc = M;
+        for (uint32_t k = lane; k < L; k += 32) {
+            const float2 pr = R.P[R.lst[k]];
+            if (same_pt(pr, M) || s * orient(R.P[R.lst[k ? k - 1u : L - 1u]], pr, R.P[R.lst[wrap(k + 1u, L)]]) > 0) continue;
+            if (u * cmpf(pr.y, my) < 0 || s * orient(ea, eb, pr) < 0 || u * orient(M, Pt, pr) > 0) continue;
+            int w = 1;
+            if (c != NONE) {
+                w = u * orient(M, pr, pc);
+                if (w == 0) w = cmpf(pc.x, pr.x);
+            }
+            if (w > 0) {
+                c = k;
+                pc = pr;
+            }
+        }
+#pragma unroll
+        for (int d = 16; d >= 1; d >>= 1) {
+            const uint32_t o = __shfl_xor_sync(0xFFFFFFFFu, c, d);
+            const float2 po = make_float2(__shfl_xor_sync(0xFFFFFFFFu, pc.x, d), __shfl_xor_sync(0xFFFFFFFFu, pc.y, d));
+            if (o == NONE) continue;
+            int w = 1;
+            if (c != NONE) {
+                w = u * orient(M, po, pc);
+                if (w == 0) w = cmpf(pc.x, po.x);
+                if (w == 0) w = o < c ? 1 : -1;
+            }
+            if (w > 0) {
+                c = o;
+                pc = po;
+            }
+        }
+        if (c != NONE) {
+            const int w = u * orient(M, pc, Pt);
+            if (w > 0 || (w == 0 && pc.x < Pt.x)) t = c;
+        }
+    }
+    // 3. the first copy of the target point whose wedge contains M
+    const float2 T = R.P[R.lst[t]];
+    for (uint32_t base = 0; base < L; base += 32) {
+        const uint32_t k = base + lane;
+        bool ok = false;
+        if (k < L && same_pt(R.P[R.lst[k]], T)) {
+            const float2 pp = R.P[R.lst[k ? k - 1u : L - 1u]], pn = R.P[R.lst[wrap(k + 1u, L)]];
+            const int o1 = s * orient(pp, T, M), o2 = s * orient(T, pn, M);
+            ok = s * orient(pp, T, pn) > 0 ? (o1 > 0 && o2 > 0) : (o1 > 0 || o2 > 0);
+        }
+        const uint32_t hit = __ballot_sync(0xFFFFFFFFu, ok);
+        if (hit) return base + __ffs(hit) - 1u;
+    }
+    return t;
+}
+
+// Merges the H holes of a polygon into its outer ring (step 4 of the header).  On entry R.P[0..N) holds the polygon's
+// points and hs(h) gives the start of ring h relative to the polygon (hs(H + 1) = N); on exit R.P[0..N+2H) holds the
+// merged ring.  Meanwhile R.lst holds the merged ring as point ids and R.prv / R.nxt each hole's M and the merge order.
+// Returns MR_POLY_BAD_HOLE or 0.
+template <class HS>
+__device__ uint32_t merge_holes(const Ring& R, const float2* src, uint32_t N, uint32_t H, const HS& hs, uint32_t lane) {
+    const uint32_t N0 = hs(1u);
+    const int s = ring_winding(R, 0, N0, lane);
+    for (uint32_t h = lane; h < H; h += 32) {
+        const uint32_t a = hs(h + 1u), b = hs(h + 2u);
+        uint32_t m = a;
+        for (uint32_t k = a + 1u; k < b; ++k)
+            if (above_xy(R.P[k], R.P[m])) m = k;
+        R.prv[h] = (uint16_t)m;
+    }
+    __syncwarp();
+    // merge order: decreasing (x, y) of M, equal M in hole order
+    for (uint32_t h = lane; h < H; h += 32) {
+        const float2 pm = R.P[R.prv[h]];
+        uint32_t rank = 0;
+        for (uint32_t g = 0; g < H; ++g) {
+            const float2 pg = R.P[R.prv[g]];
+            rank += above_xy(pg, pm) || (same_pt(pg, pm) && g < h);
+        }
+        R.nxt[rank] = (uint16_t)h;
+    }
+    for (uint32_t k = lane; k < N0; k += 32) R.lst[k] = (uint16_t)k;
+    __syncwarp();
+    uint32_t L = N0, status = 0;
+    for (uint32_t z = 0; z < H; ++z) {
+        const uint32_t h = R.nxt[z], M = R.prv[h], a = hs(h + 1u), n = hs(h + 2u) - a;
+        bool bad;
+        const uint32_t k = bridge_pos(R, L, R.P[M], s, lane, bad);
+        if (bad) status = MR_POLY_BAD_HOLE;
+        const bool rev = ring_winding(R, a, n, lane) == s;
+        // open a gap of n + 2 after position k (from the end, a chunk of 32 read before it is written)
+        const uint32_t d = n + 2u;
+        for (uint32_t end = L; end > k + 1u;) {
+            const uint32_t start = end - (k + 1u) > 32u ? end - 32u : k + 1u;
+            const uint32_t i = start + lane;
+            const uint16_t v = i < end ? R.lst[i] : (uint16_t)0;
+            __syncwarp();
+            if (i < end) R.lst[i + d] = v;
+            __syncwarp();
+            end = start;
+        }
+        const uint32_t jm = M - a;
+        for (uint32_t dd = lane; dd < n; dd += 32) R.lst[k + 1u + dd] = (uint16_t)(a + (rev ? (jm + n - dd) % n : (jm + dd) % n));
+        if (lane == 0) {
+            R.lst[k + 1u + n] = (uint16_t)M;
+            R.lst[k + 2u + n] = R.lst[k];
+        }
+        __syncwarp();
+        L += d;
+    }
+    // the merged ring's points, from the caller's array (R.P still holds the input order until here)
+    for (uint32_t k = lane; k < L; k += 32) R.P[k] = __ldg(src + R.lst[k]);
+    __syncwarp();
+    return status;
+}
+
+// The ring checks of mr_triangulate_earclip_holes, in the header's order; H = the number of holes when they pass.
+__device__ uint32_t ring_status(const EcArgs& a, const RingArgs& rg, uint32_t pi, uint64_t r0, uint64_t np64, uint32_t& H,
+                                uint32_t lane) {
+    const uint64_t nr = rg.first_ring[pi + 1] - r0;
+    if (nr == 0 || nr > np64) return MR_POLY_DEGENERATE;
+    if (np64 + 2u * (nr - 1u) > MR_MAX_POLYGON_POINTS) return MR_POLY_TOO_LARGE;
+    H = (uint32_t)(nr - 1u);
+    bool ok = true;
+    for (uint32_t h = lane; h <= H; h += 32) {
+        const uint64_t s0 = rg.ring_start[r0 + h - rg.ring_base] - a.first_point[pi];
+        const uint64_t s1 = h < H ? rg.ring_start[r0 + h + 1u - rg.ring_base] - a.first_point[pi] : np64;
+        ok = ok && (h || s0 == 0) && s0 < s1 && s1 - s0 >= 3u && s1 <= np64;
+    }
+    return __all_sync(0xFFFFFFFFu, ok) ? MR_POLY_OK : MR_POLY_DEGENERATE;
+}
+
+// One polygon of mr_triangulate_earclip (HOLES false; rg unused) or mr_triangulate_earclip_holes.
+template <bool HOLES>
+__device__ void earclip_polygon(const EcArgs& a, const RingArgs& rg, uint32_t pi, const Ring& R, uint32_t lane) {
     const uint64_t p0 = a.first_point[pi] - a.point_base;
     const uint64_t np64 = a.first_point[pi + 1] - a.first_point[pi];
     const uint64_t t0 = a.first_tri[pi] - a.tri_base;
@@ -249,10 +517,14 @@ __device__ void earclip_polygon(const EcArgs& a, uint32_t pi, const Ring& R, uin
 
     uint32_t status = MR_POLY_OK, ntri = 0;
     float b1y = 0.0f, b2y = 0.0f;
-    if (n < 3u) {
+    uint32_t H = 0;
+    const uint64_t r0 = HOLES ? rg.first_ring[pi] : 0;
+    if (!HOLES && n < 3u) {
         status = MR_POLY_DEGENERATE;
-    } else if (n > MR_MAX_POLYGON_POINTS) {
+    } else if (!HOLES && n > MR_MAX_POLYGON_POINTS) {
         status = MR_POLY_TOO_LARGE;
+    } else if (HOLES && (status = ring_status(a, rg, pi, r0, np64, H, lane)) != MR_POLY_OK) {
+        // rejected by the ring checks
     } else {
         bool finite = true;
         const float2* src = reinterpret_cast<const float2*>(a.xy) + p0;
@@ -265,8 +537,19 @@ __device__ void earclip_polygon(const EcArgs& a, uint32_t pi, const Ring& R, uin
         if (!__all_sync(0xFFFFFFFFu, finite)) {
             status = MR_POLY_NONFINITE;
         } else {
-            status = clip_ring(R, n, em, lane);
-            const uint32_t T = n - 2u;
+            uint32_t L = n;
+            if constexpr (HOLES) {
+                if (H) {
+                    const uint64_t fp = a.first_point[pi];
+                    auto hs = [&](uint32_t h) -> uint32_t {
+                        return h > H ? n : h ? (uint32_t)(rg.ring_start[r0 + h - rg.ring_base] - fp) : 0u;
+                    };
+                    status = merge_holes(R, src, n, H, hs, lane);
+                    L = n + 2u * H;
+                }
+            }
+            status |= clip_ring(R, L, em, lane);
+            const uint32_t T = L - 2u;
             ntri = T < cap_tri ? T : cap_tri;
             if (T > cap_tri) status |= MR_POLY_OVERFLOW;
             if (T < cap_tri) {
@@ -285,9 +568,10 @@ __device__ void earclip_polygon(const EcArgs& a, uint32_t pi, const Ring& R, uin
     }
 }
 
-// size class C: polygons of ec_nmax(C-1)+1 .. ec_nmax(C) points (class 0 also takes every invalid size)
-template <int C>
-__global__ void __launch_bounds__(ec_wpb(C) * 32) earclip_k(const EcArgs a) {
+// size class C: polygons of ec_nmax(C-1)+1 .. ec_nmax(C) points (class 0 also takes every invalid size); with holes the
+// size is that of the merged ring, N + 2H
+template <bool HOLES, int C>
+__device__ __forceinline__ void earclip_class(const EcArgs& a, const RingArgs& rg) {
     extern __shared__ __align__(16) unsigned char smem[];
     constexpr uint32_t NMAX = ec_nmax(C);
     const uint32_t lane = threadIdx.x & 31u;
@@ -305,9 +589,17 @@ __global__ void __launch_bounds__(ec_wpb(C) * 32) earclip_k(const EcArgs a) {
         if (lane == 0) idx = atomicAdd(&a.queue_head[C], 1u);
         idx = __shfl_sync(0xFFFFFFFFu, idx, 0);
         if (idx >= end - begin) break;
-        earclip_polygon(a, a.order[begin + idx], R, lane);
+        earclip_polygon<HOLES>(a, rg, a.order[begin + idx], R, lane);
         __syncwarp();
     }
+}
+
+template <int C>
+__global__ void __launch_bounds__(ec_wpb(C) * 32) earclip_k(const EcArgs a) { earclip_class<false, C>(a, RingArgs{}); }
+
+template <int C>
+__global__ void __launch_bounds__(ec_wpb(C) * 32) earclip_holes_k(const EcArgs a, const RingArgs rg) {
+    earclip_class<true, C>(a, rg);
 }
 
 __global__ void __launch_bounds__(256) selftest_orient_k(const float* __restrict__ abc, uint64_t count, int8_t* __restrict__ out) {
@@ -317,31 +609,48 @@ __global__ void __launch_bounds__(256) selftest_orient_k(const float* __restrict
     }
 }
 
+__global__ void __launch_bounds__(256) selftest_crossing_k(const float* __restrict__ q, uint64_t count, int8_t* __restrict__ out) {
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < count; i += (uint64_t)gridDim.x * blockDim.x) {
+        const float* t = q + 9 * i;
+        out[i] = (int8_t)cross_sign(make_float2(t[0], t[1]), make_float2(t[2], t[3]), make_float2(t[4], t[5]),
+                                    make_float2(t[6], t[7]), t[8]);
+    }
+}
+
+// rg == nullptr: mr_triangulate_earclip
 template <int C>
-int launch_class(mr_context* ctx, const EcArgs& a, uint32_t npoly) {
+int launch_class(mr_context* ctx, const EcArgs& a, const RingArgs* rg, uint32_t npoly) {
     const int wpb = ec_wpb(C);
     const size_t smem = (size_t)wpb * ec_ws_bytes(ec_nmax(C));
-    MR_CUDA(ctx, cudaFuncSetAttribute(earclip_k<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const void* fn = rg ? reinterpret_cast<const void*>(earclip_holes_k<C>) : reinterpret_cast<const void*>(earclip_k<C>);
+    MR_CUDA(ctx, cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 0;
-    MR_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, earclip_k<C>, wpb * 32, smem));
+    MR_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, wpb * 32, smem));
     uint64_t grid = (uint64_t)ctx->sm_count * (per_sm < 1 ? 1 : per_sm);
     const uint64_t need = ((uint64_t)npoly + wpb - 1) / wpb;
     if (need < grid) grid = need;
-    earclip_k<C><<<(unsigned)grid, wpb * 32, smem, ctx->stream>>>(a);
-    MR_LAUNCH_CHECK(ctx, "earclip_k");
+    if (rg) {
+        earclip_holes_k<C><<<(unsigned)grid, wpb * 32, smem, ctx->stream>>>(a, *rg);
+        MR_LAUNCH_CHECK(ctx, "earclip_holes_k");
+    } else {
+        earclip_k<C><<<(unsigned)grid, wpb * 32, smem, ctx->stream>>>(a);
+        MR_LAUNCH_CHECK(ctx, "earclip_k");
+    }
     return MR_OK;
 }
 }  // namespace
 
-int mr_triangulate_earclip_impl(mr_context* ctx, const mr_polygon_job* j) {
-    // all pointers in *j are device pointers here (staging happened in api.cu)
+namespace {
+int earclip_run(mr_context* ctx, const mr_polygon_job* j, const mr_polygon_rings* rings) {
+    // all pointers in *j and *rings are device pointers here (staging happened in api.cu)
     const uint32_t npoly = j->npoly;
     if (npoly == 0) return MR_OK;
-    // work list: hist | cursor | class ranges of the reference path (unused) | queue heads | order.  A scratch slot of
-    // its own, so that the reference path's work-list header (mr_triangulate_tier_counts) stays as it was.
+    // work list: hist | cursor | class ranges of the reference path (unused) | queue heads | order [| merged sizes].  A
+    // scratch slot of its own, so that the reference path's work-list header (mr_triangulate_tier_counts) stays as it was.
     constexpr size_t ZERO_WORDS = 2 * (size_t)MR_SIZE_BINS + 64 + EC_CLASSES;
+    const size_t order_bytes = ((ZERO_WORDS + npoly) * 4 + 7) / 8 * 8;
     void* work = nullptr;
-    int rc = mr_scratch(ctx, 13, (ZERO_WORDS + npoly) * 4, &work);
+    int rc = mr_scratch(ctx, 13, order_bytes + (rings ? ((size_t)npoly + 1) * 8 : 0), &work);
     if (rc) return rc;
     uint32_t* w = static_cast<uint32_t*>(work);
     uint32_t* hist = w;
@@ -350,7 +659,15 @@ int mr_triangulate_earclip_impl(mr_context* ctx, const mr_polygon_job* j) {
     uint32_t* heads = classes + 64;
     uint32_t* order = heads + EC_CLASSES;
     MR_CUDA(ctx, cudaMemsetAsync(w, 0, ZERO_WORDS * 4, ctx->stream));
-    rc = mr_polygon_size_sort(ctx, j->first_point, npoly, hist, cursor, classes, classes + 32, order);
+    // with holes the classes key on the merged size N + 2H: a prefix sum of it stands in for first_point
+    const uint64_t* sizes = j->first_point;
+    if (rings) {
+        uint64_t* msz = reinterpret_cast<uint64_t*>(static_cast<unsigned char*>(work) + order_bytes);
+        rc = mr_polygon_ring_counts(ctx, j->first_point, rings->first_ring, npoly, 0, msz);
+        if (rc) return rc;
+        sizes = msz;
+    }
+    rc = mr_polygon_size_sort(ctx, sizes, npoly, hist, cursor, classes, classes + 32, order);
     if (rc) return rc;
 
     EcArgs a;
@@ -373,11 +690,29 @@ int mr_triangulate_earclip_impl(mr_context* ctx, const mr_polygon_job* j) {
     a.order = order;
     a.cursor = cursor;
     a.queue_head = heads;
+    RingArgs rg{};
+    if (rings) rg = RingArgs{rings->first_ring, rings->ring_base, rings->ring_start};
+    const RingArgs* rp = rings ? &rg : nullptr;
     // largest class first
-    if ((rc = launch_class<3>(ctx, a, npoly))) return rc;
-    if ((rc = launch_class<2>(ctx, a, npoly))) return rc;
-    if ((rc = launch_class<1>(ctx, a, npoly))) return rc;
-    return launch_class<0>(ctx, a, npoly);
+    if ((rc = launch_class<3>(ctx, a, rp, npoly))) return rc;
+    if ((rc = launch_class<2>(ctx, a, rp, npoly))) return rc;
+    if ((rc = launch_class<1>(ctx, a, rp, npoly))) return rc;
+    return launch_class<0>(ctx, a, rp, npoly);
+}
+}  // namespace
+
+int mr_triangulate_earclip_impl(mr_context* ctx, const mr_polygon_job* j) { return earclip_run(ctx, j, nullptr); }
+
+int mr_triangulate_earclip_holes_impl(mr_context* ctx, const mr_polygon_job* j, const mr_polygon_rings* rings) {
+    return earclip_run(ctx, j, rings);
+}
+
+int mr_selftest_crossing_impl(mr_context* ctx, const float* q, uint64_t count, int8_t* sign_out) {
+    if (count == 0) return MR_OK;
+    const unsigned blocks = (unsigned)std::min<uint64_t>((count + 255) / 256, (uint64_t)ctx->sm_count * 16);
+    selftest_crossing_k<<<blocks, 256, 0, ctx->stream>>>(q, count, sign_out);
+    MR_LAUNCH_CHECK(ctx, "selftest_crossing_k");
+    return MR_OK;
 }
 
 int mr_selftest_orient_impl(mr_context* ctx, const float* abc, uint64_t count, int8_t* sign_out) {

@@ -1191,6 +1191,16 @@ __global__ void polygon_offsets_k(const uint64_t* __restrict__ first_point, uint
     }
 }
 
+// with holes: N + 2H - sub, H = rings - 1 when 1 <= rings <= N (else 0), clamped at 0
+__global__ void polygon_ring_counts_k(const uint64_t* __restrict__ first_point, const uint64_t* __restrict__ first_ring,
+                                      uint32_t npoly, uint32_t sub, uint64_t* __restrict__ count) {
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < npoly; i += gridDim.x * blockDim.x) {
+        const uint64_t n = first_point[i + 1] - first_point[i], r = first_ring[i + 1] - first_ring[i];
+        const uint64_t t = n + (r >= 1 && r <= n ? 2 * (r - 1) : 0);
+        count[i] = t >= sub ? t - sub : 0;
+    }
+}
+
 // single-block exclusive scan of u64 counts (npoly up to a few million: chunked loop)
 __global__ void __launch_bounds__(1024) exclusive_scan_u64_k(const uint64_t* __restrict__ in, uint32_t count,
                                                             uint64_t* __restrict__ out) {
@@ -1280,6 +1290,19 @@ int mr_polygon_offsets_impl(mr_context* ctx, const uint64_t* first_point_dev, ui
     polygon_offsets_k<<<blocks, 256, 0, ctx->stream>>>(first_point_dev, npoly, static_cast<uint64_t*>(tmp));
     MR_LAUNCH_CHECK(ctx, "polygon_offsets_k");
     exclusive_scan_u64_k<<<1, 1024, 0, ctx->stream>>>(static_cast<uint64_t*>(tmp), npoly, first_tri_dev);
+    MR_LAUNCH_CHECK(ctx, "exclusive_scan_u64_k");
+    return MR_OK;
+}
+
+int mr_polygon_ring_counts(mr_context* ctx, const uint64_t* first_point, const uint64_t* first_ring, uint32_t npoly,
+                           uint32_t sub, uint64_t* out) {
+    void* tmp = nullptr;
+    int rc = mr_scratch(ctx, SLOT_MISC, (size_t)(npoly + 1) * 8, &tmp);
+    if (rc) return rc;
+    const unsigned blocks = (unsigned)std::min<uint64_t>(((uint64_t)npoly + 255) / 256 + 1, 1024);
+    polygon_ring_counts_k<<<blocks, 256, 0, ctx->stream>>>(first_point, first_ring, npoly, sub, static_cast<uint64_t*>(tmp));
+    MR_LAUNCH_CHECK(ctx, "polygon_ring_counts_k");
+    exclusive_scan_u64_k<<<1, 1024, 0, ctx->stream>>>(static_cast<uint64_t*>(tmp), npoly, out);
     MR_LAUNCH_CHECK(ctx, "exclusive_scan_u64_k");
     return MR_OK;
 }

@@ -23,7 +23,7 @@ from typing import Callable, Optional, Sequence
 import numpy as np
 
 from . import _capi as capi
-from ._capi import MrError, MrLayout, MrPolygonJob, MrTerrainJob, MrTerrainParams
+from ._capi import MrError, MrLayout, MrPolygonJob, MrPolygonRings, MrTerrainJob, MrTerrainParams
 
 try:  # torch is plumbing (device memory, streams); numpy host arrays work without it
     import torch
@@ -298,6 +298,16 @@ def polygon_offsets_host(first_point: np.ndarray) -> np.ndarray:
     return ft
 
 
+def polygon_offsets_rings_host(first_point: np.ndarray, first_ring: np.ndarray) -> np.ndarray:
+    """first_tri of mr_polygon_offsets_rings: N + 2H - 2 triangles per polygon."""
+    n = np.diff(first_point.astype(np.int64))
+    r = np.diff(first_ring.astype(np.int64))
+    h = np.where((r >= 1) & (r <= n), r - 1, 0)
+    ft = np.zeros(len(first_point), dtype=np.uint64)
+    ft[1:] = np.cumsum(np.maximum(n + 2 * h - 2, 0))
+    return ft
+
+
 _ALGORITHMS = {"reference": "mr_triangulate_batch", "earclip": "mr_triangulate_earclip"}
 
 
@@ -325,22 +335,45 @@ class Polygon:
         j.bbox_out, j.status_out, j.ntri_out = _ptr(bbox_out), _ptr(status_out), _ptr(ntri_out)
         return j
 
-    def triangulate(self, job: MrPolygonJob, algorithm: str = "reference"):
+    def triangulate(self, job: MrPolygonJob, algorithm: str = "reference", rings: Optional[MrPolygonRings] = None):
         """algorithm "reference": mr_triangulate_batch (the reference's triangulator, for parity); "earclip":
-        mr_triangulate_earclip (correct on every simple polygon, same output format)."""
+        mr_triangulate_earclip (correct on every simple polygon, same output format), or with `rings`
+        mr_triangulate_earclip_holes (polygons with holes)."""
         _check_algorithm(algorithm, None)
+        if rings is not None:
+            if algorithm != "earclip":
+                raise ValueError("holes are triangulated by the earclip algorithm only")
+            self.ctx.check(self.ctx.lib.mr_triangulate_earclip_holes(self.ctx.handle, C.byref(job), C.byref(rings)),
+                           "mr_triangulate_earclip_holes")
+            return
         name = _ALGORITHMS[algorithm]
         self.ctx.check(getattr(self.ctx.lib, name)(self.ctx.handle, C.byref(job)), name)
 
     def create_polygons(self, xy, first_point, *, offset_prime=None, seed=0, poly_index0=0,
-                        device="cuda", algorithm="reference") -> PolygonBatch:
+                        device="cuda", algorithm="reference", rings=None) -> PolygonBatch:
         """Batched create_polygon.  xy: [npts,2] f32 (numpy or cuda tensor); first_point: npoly+1 offsets.
-        algorithm: "reference" or "earclip" (see triangulate); ear clipping takes no offset_prime."""
+        algorithm: "reference" or "earclip" (see triangulate); ear clipping takes no offset_prime.
+        rings = (first_ring, ring_start): polygons with holes (earclip only), as mr_polygon_rings with ring_base
+        first_ring[0]; polygon i then gets N + 2H - 2 triangles."""
         _check_algorithm(algorithm, offset_prime)
+        if rings is not None and algorithm != "earclip":
+            raise ValueError("holes are triangulated by the earclip algorithm only")
         fp_host = np.ascontiguousarray(
             first_point.cpu().numpy() if _is_cuda(first_point) else first_point, dtype=np.uint64)
         npoly = len(fp_host) - 1
-        ft_host = polygon_offsets_host(fp_host)
+        rg = keep = None
+        if rings is None:
+            ft_host = polygon_offsets_host(fp_host)
+        else:
+            fr, rs = rings
+            fr_host = np.ascontiguousarray(fr.cpu().numpy() if _is_cuda(fr) else fr, dtype=np.uint64)
+            if len(fr_host) != npoly + 1:
+                raise ValueError("first_ring must hold npoly+1 offsets")
+            ft_host = polygon_offsets_rings_host(fp_host, fr_host)
+            keep = (torch.from_numpy(fr_host.view(np.int64)).to(torch.device(device)),
+                    rs if _is_cuda(rs) else torch.from_numpy(
+                        np.ascontiguousarray(rs, dtype=np.uint64).view(np.int64)).to(torch.device(device)))
+            rg = MrPolygonRings(_ptr(keep[0]), int(fr_host[0]), _ptr(keep[1]))
         dev = torch.device(device)
         xy_d = xy if _is_cuda(xy) else torch.from_numpy(np.ascontiguousarray(xy, dtype=np.float32)).to(dev)
         fp_d = torch.from_numpy(fp_host.view(np.int64)).to(dev)
@@ -358,32 +391,44 @@ class Polygon:
         nt = torch.empty(npoly, dtype=torch.int32, device=dev)
         self.triangulate(self.job(xy_d, fp_d, npoly, vtx_out=vtx, first_tri=ft_d, bbox_out=bbox,
                                   status_out=status, ntri_out=nt, offset_prime=op_d, seed=seed,
-                                  poly_index0=poly_index0, point_base=int(fp_host[0])), algorithm)
+                                  poly_index0=poly_index0, point_base=int(fp_host[0])), algorithm, rg)
         return PolygonBatch(npoly, fp_host, ft_host, vtx[: ntri * 3 * self.layout.stride], bbox, status, nt,
                             self.layout)
 
-    def create_polygon(self, vertices, *, offset_prime=None, seed=0, index=0, algorithm="reference") -> PolygonObj:
+    def create_polygon(self, vertices, *, offset_prime=None, seed=0, index=0, algorithm="reference",
+                       holes=None) -> PolygonObj:
         """Polygon.create_polygon(vertices): one polygon -> VertexBuffer of n-2 triangles + bbox.
 
         Like the reference (Polygon.zig:82-92: a mapped-at-creation buffer filled by the emit callback) the
         vertex range is HOST memory -- the stand-in for the mapped range -- so the call takes the library's
-        small-batch path: one copy in, one kernel, one copy out.  algorithm: as for create_polygons."""
+        small-batch path: one copy in, one kernel, one copy out.  algorithm: as for create_polygons.
+        holes: a list of point arrays, one per hole (earclip only); the polygon then gets N + 2H - 2 triangles."""
         _check_algorithm(algorithm, offset_prime)
+        if holes is not None and algorithm != "earclip":
+            raise ValueError("holes are triangulated by the earclip algorithm only")
         v = np.ascontiguousarray(vertices, dtype=np.float32).reshape(-1, 2)
+        rg = None
+        if holes is not None:
+            hs = [np.ascontiguousarray(h, dtype=np.float32).reshape(-1, 2) for h in holes]
+            rs = np.cumsum([0, len(v)] + [len(h) for h in hs[:-1]]).astype(np.uint64) if hs else np.zeros(1, np.uint64)
+            fr = np.array([0, len(hs) + 1], dtype=np.uint64)
+            v = np.concatenate([v] + hs).astype(np.float32) if hs else v
+            rg = MrPolygonRings(fr.ctypes.data, 0, rs.ctypes.data)
         n = len(v)
+        ntri_total = n - 2 + 2 * (len(holes) if holes else 0)
         if n < 2:  # Polygon.zig:82: vertices.len - 2 underflows
             raise ValueError("a polygon needs at least 2 vertices")
         op = None if offset_prime is None else np.ascontiguousarray(offset_prime, dtype=np.uint32).reshape(2)
         fp = np.array([0, n], dtype=np.uint64)
-        ft = np.array([0, n - 2], dtype=np.uint64)
-        mapped = np.zeros(max((n - 2) * 3 * self.layout.stride, 1), dtype=np.uint8)  # VertexBuffer.new: zeroed
+        ft = np.array([0, ntri_total], dtype=np.uint64)
+        mapped = np.zeros(max(ntri_total * 3 * self.layout.stride, 1), dtype=np.uint8)  # VertexBuffer.new: zeroed
         bb = np.zeros(4, dtype=np.float32)
         st = np.zeros(1, dtype=np.uint32)
         nt = np.zeros(1, dtype=np.uint32)
         self.triangulate(self.job(v, fp, 1, vtx_out=mapped, first_tri=ft, bbox_out=bb, status_out=st, ntri_out=nt,
-                                  offset_prime=op, seed=seed, poly_index0=index), algorithm)
+                                  offset_prime=op, seed=seed, poly_index0=index), algorithm, rg)
         buf = torch.from_numpy(mapped) if torch is not None else mapped
-        vb = VertexBuffer(buf, (n - 2) * 3, 1, 0, 0)
+        vb = VertexBuffer(buf, ntri_total * 3, 1, 0, 0)
         return PolygonObj(vb, (float(bb[0]), float(bb[1]), 0.0), (float(bb[2]), float(bb[3]), 0.0),
                           int(st[0]), int(nt[0]))
 

@@ -228,6 +228,40 @@ class Polygon {
         o.bounding_box_p1[1] = bbox[3];
         return o;
     }
+    // A polygon with holes (mr_triangulate_earclip_holes): N + 2H - 2 triangles, N the points of all rings.
+    PolygonObj create_polygon_earclip(const std::vector<Point>& outer, const std::vector<std::vector<Point>>& holes) {
+        std::vector<Point> pts(outer);
+        std::vector<uint64_t> ring_start{0};
+        for (const auto& h : holes) {
+            ring_start.push_back(pts.size());
+            pts.insert(pts.end(), h.begin(), h.end());
+        }
+        if (pts.size() < 2) throw Error(MR_E_BADARG, "create_polygon: vertices.len - 2 underflows (Polygon.zig:82)");
+        PolygonObj o;
+        const uint64_t n = pts.size(), ntri = n + 2 * holes.size() - 2;
+        o.vertex_buffer = VertexBuffer::create(0, static_cast<uint32_t>(ntri), layout_.native.stride);
+        const uint64_t first_point[2] = {0, n};
+        const uint64_t first_tri[2] = {0, ntri};
+        const uint64_t first_ring[2] = {0, ring_start.size()};
+        float bbox[4];
+        mr_polygon_job j{};
+        j.xy = reinterpret_cast<const float*>(pts.data());
+        j.first_point = first_point;
+        j.npoly = 1;
+        j.layout = layout_.native;
+        j.vtx_out = o.vertex_buffer.mapped.data();
+        j.first_tri = first_tri;
+        j.bbox_out = bbox;
+        j.status_out = &o.status;
+        j.ntri_out = &o.ntri;
+        const mr_polygon_rings rings{first_ring, 0, ring_start.data()};
+        ctx_.check(mr_triangulate_earclip_holes(ctx_.get(), &j, &rings), "mr_triangulate_earclip_holes");
+        o.bounding_box_p0[0] = bbox[0];
+        o.bounding_box_p0[1] = bbox[1];
+        o.bounding_box_p1[0] = bbox[2];
+        o.bounding_box_p1[1] = bbox[3];
+        return o;
+    }
     const VertexLayout& layout() const { return layout_; }
 
    private:

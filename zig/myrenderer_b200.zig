@@ -53,6 +53,13 @@ pub const PolygonJob = extern struct {
     ntri_out: ?[*]u32,
 };
 
+// mr_polygon_rings: the rings (outer boundary, then holes) of each polygon of a PolygonJob
+pub const PolygonRings = extern struct {
+    first_ring: [*]const u64,
+    ring_base: u64,
+    ring_start: [*]const u64,
+};
+
 pub extern fn mr_context_create(device: c_int, ctx_out: *?*Context) c_int;
 pub extern fn mr_context_destroy(ctx: ?*Context) c_int;
 pub extern fn mr_sync(ctx: ?*Context) c_int;
@@ -63,6 +70,7 @@ pub extern fn mr_terrain_build_full(ctx: ?*Context, height: *const anyopaque, he
 pub extern fn mr_terrain_describe(n: u32, params: ?*const TerrainParams, bbox_min: ?*[3]f32, bbox_max: ?*[3]f32, vertex_count: ?*u64, index_count: ?*u64) c_int;
 pub extern fn mr_triangulate_batch(ctx: ?*Context, job: *const PolygonJob) c_int;
 pub extern fn mr_triangulate_earclip(ctx: ?*Context, job: *const PolygonJob) c_int;
+pub extern fn mr_triangulate_earclip_holes(ctx: ?*Context, job: *const PolygonJob, rings: *const PolygonRings) c_int;
 pub extern fn mr_polygon_draw_range(first_tri_i: u64, first_tri_next: u64, tri_base: u64, out: *DrawRange) c_int;
 pub extern fn mr_unirand_seed_host(top: u32, seed: u64, index: u64, offset_out: *u32, prime_out: *u32) c_int;
 pub extern fn mr_context_trim(ctx: ?*Context) c_int;
