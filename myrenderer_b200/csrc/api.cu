@@ -273,24 +273,29 @@ int mr_terrain_build(mr_context* ctx, const mr_terrain_job* job) {
     mr_terrain_job d = j;
     if (!want_v) d.vtx_out = nullptr;
     if (!want_i) d.idx_out = nullptr;
+    mr_staging io(ctx);
     bool vs = false, is = false;
     void* vdev = nullptr;
-    void* idev = nullptr;
+    uint32_t* idev = nullptr;
     const size_t row_bytes = (size_t)j.n * j.layout.stride;
     const size_t qrow_bytes = 6u * (size_t)(j.n - 1u) * 4u;
-    int rc;
+    // a staged output holds its band only: rows [row_begin, row_end), quad rows [qrow_begin, qrow_end)
+    const size_t vbytes = (size_t)(j.row_end - j.row_begin) * row_bytes;
+    const size_t ibytes = (size_t)(j.qrow_end - j.qrow_begin) * qrow_bytes;
+    unsigned char* idst = nullptr;  // where a staged band goes in the caller's buffer
     // The index buffer does not depend on the heightmap.  When it has to travel to a host buffer, it is built and copied
     // on a side stream first, so that its device-to-host copy overlaps the heightmap's host-to-device copy (PCIe is full
     // duplex) and the vertex kernel, instead of both copies queueing behind both kernels.
     cudaStream_t idx_stream = ctx->stream;
     if (want_i) {
-        // staged output holds quad rows [qrow_begin, qrow_end) only (device outputs keep the caller's idx_qrow0 origin)
-        rc = mr_stage_out(ctx, 5, j.idx_out, (size_t)(j.qrow_end - j.qrow_begin) * qrow_bytes, &idev, &is);
-        if (rc) return rc;
+        // (device outputs keep the caller's idx_qrow0 origin)
+        idev = io.out(MR_SLOT_BBOX, j.idx_out, ibytes, &is);
+        if (io.rc) return io.rc;
         if (is) {
-            d.idx_out = static_cast<uint32_t*>(idev);
+            d.idx_out = idev;
             d.idx_qrow0 = j.qrow_begin;
-            if (want_v && !mr_is_device_ptr(j.vtx_out)) {
+            idst = reinterpret_cast<unsigned char*>(j.idx_out) + (size_t)(j.qrow_begin - j.idx_qrow0) * qrow_bytes;
+            if (want_v && !io.where(j.vtx_out).device) {
                 if (mr_aux_streams(ctx)) return mr_fail(ctx, MR_E_CUDA, "side streams");
                 MR_CUDA(ctx, cudaEventRecord(ctx->fork_ev, ctx->stream));  // order after earlier work on the context
                 MR_CUDA(ctx, cudaStreamWaitEvent(ctx->aux[0], ctx->fork_ev, 0));
@@ -298,24 +303,21 @@ int mr_terrain_build(mr_context* ctx, const mr_terrain_job* job) {
             }
         }
     }
+    int rc;
     if (idx_stream != ctx->stream) {
         mr_terrain_job di = d;
         di.vtx_out = nullptr;
         rc = mr_terrain_build_impl(ctx, &di, idx_stream);
         if (rc) return rc;
-        unsigned char* dst = reinterpret_cast<unsigned char*>(j.idx_out) + (size_t)(j.qrow_begin - j.idx_qrow0) * qrow_bytes;
-        MR_CUDA(ctx, cudaMemcpyAsync(dst, idev, (size_t)(j.qrow_end - j.qrow_begin) * qrow_bytes, cudaMemcpyDeviceToHost, idx_stream));
+        MR_CUDA(ctx, cudaMemcpyAsync(idst, idev, ibytes, cudaMemcpyDeviceToHost, idx_stream));
         MR_CUDA(ctx, cudaEventRecord(ctx->join_ev[0], idx_stream));
         d.idx_out = nullptr;
     }
     if (want_v) {
         const size_t texel = j.height_fmt == MR_HEIGHT_U16 ? 2 : 4;
-        const void* hdev = nullptr;
-        rc = mr_stage_in(ctx, 0, j.height, (size_t)j.height_rows * j.n * texel, &hdev);
-        if (rc) return rc;
-        d.height = hdev;
-        rc = mr_stage_out(ctx, 4, j.vtx_out, (size_t)(j.row_end - j.row_begin) * row_bytes, &vdev, &vs);
-        if (rc) return rc;
+        d.height = io.in(MR_SLOT_XY, j.height, (size_t)j.height_rows * j.n * texel);
+        vdev = io.out(MR_SLOT_VTX, j.vtx_out, vbytes, &vs);
+        if (io.rc) return io.rc;
         if (vs) {
             d.vtx_out = vdev;
             d.vtx_row0 = j.row_begin;
@@ -324,17 +326,12 @@ int mr_terrain_build(mr_context* ctx, const mr_terrain_job* job) {
     rc = mr_terrain_build_impl(ctx, &d, ctx->stream);
     if (rc) return rc;
     if (vs) {
-        rc = mr_copy_back(ctx, static_cast<unsigned char*>(j.vtx_out) + (size_t)(j.row_begin - j.vtx_row0) * row_bytes, vdev,
-                          (size_t)(j.row_end - j.row_begin) * row_bytes);
-        if (rc) return rc;
+        unsigned char* vdst = static_cast<unsigned char*>(j.vtx_out) + (size_t)(j.row_begin - j.vtx_row0) * row_bytes;
+        MR_CUDA(ctx, cudaMemcpyAsync(vdst, vdev, vbytes, cudaMemcpyDeviceToHost, ctx->stream));
     }
-    if (is && idx_stream == ctx->stream) {
-        rc = mr_copy_back(ctx, reinterpret_cast<unsigned char*>(j.idx_out) + (size_t)(j.qrow_begin - j.idx_qrow0) * qrow_bytes, idev,
-                          (size_t)(j.qrow_end - j.qrow_begin) * qrow_bytes);
-        if (rc) return rc;
-    }
+    if (is && idx_stream == ctx->stream) MR_CUDA(ctx, cudaMemcpyAsync(idst, idev, ibytes, cudaMemcpyDeviceToHost, ctx->stream));
     if (idx_stream != ctx->stream) MR_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->join_ev[0], 0));
-    return mr_finish_host_io(ctx);
+    return io.finish(MR_OK);
 }
 
 int mr_terrain_build_full(mr_context* ctx, const void* height, uint32_t height_fmt, uint32_t n, const mr_layout* layout,
@@ -377,21 +374,11 @@ int mr_terrain_tile_bounds(mr_context* ctx, const void* height, uint32_t height_
     mr_terrain_params p;
     if (params) p = *params; else mr_terrain_params_default(&p);
     MR_CUDA(ctx, cudaSetDevice(ctx->device));
-    const void* hdev = nullptr;
-    int rc = mr_stage_in(ctx, 0, height, (size_t)n * n * (height_fmt == MR_HEIGHT_U16 ? 2 : 4), &hdev);
-    if (rc) return rc;
-    void* bdev = nullptr;
-    bool st = false;
-    const size_t bytes = (size_t)tr * tc * 32;
-    rc = mr_stage_out(ctx, 4, bbox_out, bytes, &bdev, &st);
-    if (rc) return rc;
-    rc = mr_terrain_tile_bounds_impl(ctx, hdev, height_fmt, n, tile_rows, tile_cols, &p, static_cast<float*>(bdev));
-    if (rc) return rc;
-    if (st) {
-        rc = mr_copy_back(ctx, bbox_out, bdev, bytes);
-        if (rc) return rc;
-    }
-    return mr_finish_host_io(ctx);
+    mr_staging io(ctx);
+    const void* hdev = io.in(MR_SLOT_XY, height, (size_t)n * n * (height_fmt == MR_HEIGHT_U16 ? 2 : 4));
+    float* bdev = io.out(MR_SLOT_VTX, bbox_out, (size_t)tr * tc * 32);
+    if (io.rc) return io.rc;
+    return io.finish(mr_terrain_tile_bounds_impl(ctx, hdev, height_fmt, n, tile_rows, tile_cols, &p, bdev));
 }
 
 namespace {
@@ -404,37 +391,35 @@ int terrain_cull_common(mr_context* ctx, const float* bbox, uint32_t n, uint32_t
     if (idx_out && (reinterpret_cast<uintptr_t>(idx_out) & 7u)) return mr_fail(ctx, MR_E_BADARG, "cull: idx_out must be 8-byte aligned");
     const size_t ntiles = (size_t)tr * tc;
     MR_CUDA(ctx, cudaSetDevice(ctx->device));
-    const void* bdev = nullptr;
-    int rc = mr_stage_in(ctx, 0, bbox, ntiles * 32, &bdev);
-    if (rc) return rc;
-    void *vdev = nullptr, *idev = nullptr, *xdev = nullptr, *cdev = nullptr, *work = nullptr;
-    bool sv = false, si = false, sx = false, sc = false;
-    if (visible_out) { rc = mr_stage_out(ctx, 1, visible_out, ntiles * 4, &vdev, &sv); if (rc) return rc; }
-    // visible ids and per-slot first index are needed internally even when the caller does not ask for the ids
-    rc = mr_scratch(ctx, 10, ntiles * 12 + 16, &work);
+    mr_staging io(ctx);
+    const float* bdev = io.in(MR_SLOT_XY, bbox, ntiles * 32);
+    uint32_t* vdev = io.out(MR_SLOT_FP, visible_out, ntiles * 4);
+    if (io.rc) return io.rc;
+    // visible ids, per-slot first index and the counts are needed internally even when the caller does not ask for them
+    void *work = nullptr, *cdev = nullptr;
+    int rc = mr_scratch(ctx, MR_SLOT_MISC, ntiles * 12 + 16, &work);
+    if (!rc && !counts_out) rc = mr_scratch(ctx, MR_SLOT_OP, 16, &cdev);
     if (rc) return rc;
     unsigned long long* first_index = static_cast<unsigned long long*>(work);
     uint32_t* ids_scratch = reinterpret_cast<uint32_t*>(first_index + ntiles);
-    if (visible_ids_out) { rc = mr_stage_out(ctx, 2, visible_ids_out, ntiles * 4, &idev, &si); if (rc) return rc; }
-    else idev = ids_scratch;
-    const size_t max_idx_bytes = 24ull * (size_t)(n - 1u) * (n - 1u);
-    if (idx_out) { rc = mr_stage_out(ctx, 5, idx_out, max_idx_bytes, &xdev, &sx); if (rc) return rc; }
-    if (counts_out) { rc = mr_stage_out(ctx, 3, counts_out, 16, &cdev, &sc); if (rc) return rc; }
-    else { rc = mr_scratch(ctx, 3, 16, &cdev); if (rc) return rc; }
-    rc = mr_terrain_cull_impl(ctx, static_cast<const float*>(bdev), n, tile_rows, tile_cols, xform, frustum, static_cast<uint32_t*>(vdev),
-                              static_cast<uint32_t*>(idev), first_index, static_cast<uint32_t*>(xdev),
+    // host outputs of a length known after the kernel: only their filled prefixes travel back
+    bool si = false, sx = false, sc = false;
+    uint32_t* idev = visible_ids_out ? io.out(MR_SLOT_FT, visible_ids_out, ntiles * 4, &si) : ids_scratch;
+    uint32_t* xdev = io.out(MR_SLOT_BBOX, idx_out, 24ull * (size_t)(n - 1u) * (n - 1u), &sx);
+    if (counts_out) cdev = io.out(MR_SLOT_OP, counts_out, 16, &sc);
+    if (io.rc) return io.rc;
+    rc = mr_terrain_cull_impl(ctx, bdev, n, tile_rows, tile_cols, xform, frustum, vdev, idev, first_index, xdev,
                               static_cast<unsigned long long*>(cdev));
     if (rc) return rc;
-    if (sv) { rc = mr_copy_back(ctx, visible_out, vdev, ntiles * 4); if (rc) return rc; }
     uint64_t counts[2] = {0, 0};
-    if (si || sx || sc) {  // host outputs: only the filled prefixes travel
+    if (si || sx || sc) {
         MR_CUDA(ctx, cudaMemcpyAsync(counts, cdev, 16, cudaMemcpyDeviceToHost, ctx->stream));
         MR_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
         if (sc) memcpy(counts_out, counts, 16);
-        if (si && counts[0]) { rc = mr_copy_back(ctx, visible_ids_out, idev, (size_t)counts[0] * 4); if (rc) return rc; }
-        if (sx && counts[1]) { rc = mr_copy_back(ctx, idx_out, xdev, (size_t)counts[1] * 4); if (rc) return rc; }
+        if (si && counts[0]) MR_CUDA(ctx, cudaMemcpyAsync(visible_ids_out, idev, (size_t)counts[0] * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        if (sx && counts[1]) MR_CUDA(ctx, cudaMemcpyAsync(idx_out, xdev, (size_t)counts[1] * 4, cudaMemcpyDeviceToHost, ctx->stream));
     }
-    return mr_finish_host_io(ctx);
+    return io.finish(MR_OK);
 }
 }  // namespace
 
@@ -453,7 +438,7 @@ int mr_selftest_fastdiv(mr_context* ctx, float divisor, int force_fast, uint64_t
     if (!ctx || !mismatches_out) return MR_E_BADARG;
     MR_CUDA(ctx, cudaSetDevice(ctx->device));
     void* d = nullptr;
-    int rc = mr_scratch(ctx, 10, 8, &d);
+    int rc = mr_scratch(ctx, MR_SLOT_MISC, 8, &d);
     if (rc) return rc;
     MR_CUDA(ctx, cudaMemsetAsync(d, 0, 8, ctx->stream));
     rc = mr_selftest_fastdiv_impl(ctx, divisor, force_fast, static_cast<unsigned long long*>(d));
@@ -467,63 +452,33 @@ int mr_selftest_fastdiv(mr_context* ctx, float divisor, int force_fast, uint64_t
 int mr_heightmap_normalize(mr_context* ctx, const uint16_t* in, uint64_t count, float* out) {
     if (!ctx || (count && (!in || !out))) return MR_E_BADARG;
     MR_CUDA(ctx, cudaSetDevice(ctx->device));
-    const void* din = nullptr;
-    int rc = mr_stage_in(ctx, 0, in, (size_t)count * 2, &din);
-    if (rc) return rc;
-    void* dout = nullptr;
-    bool st = false;
-    rc = mr_stage_out(ctx, 4, out, (size_t)count * 4, &dout, &st);
-    if (rc) return rc;
-    rc = mr_heightmap_normalize_impl(ctx, static_cast<const uint16_t*>(din), count, static_cast<float*>(dout));
-    if (rc) return rc;
-    if (st) {
-        rc = mr_copy_back(ctx, out, dout, (size_t)count * 4);
-        if (rc) return rc;
-    }
-    return mr_finish_host_io(ctx);
+    mr_staging io(ctx);
+    const uint16_t* din = io.in(MR_SLOT_XY, in, (size_t)count * 2);
+    float* dout = io.out(MR_SLOT_VTX, out, (size_t)count * 4);
+    if (io.rc) return io.rc;
+    return io.finish(mr_heightmap_normalize_impl(ctx, din, count, dout));
 }
 
 int mr_polygon_offsets(mr_context* ctx, const uint64_t* first_point, uint32_t npoly, uint64_t* first_tri_out) {
     if (!ctx || !first_point || !first_tri_out) return MR_E_BADARG;
     MR_CUDA(ctx, cudaSetDevice(ctx->device));
-    const void* dfp = nullptr;
-    int rc = mr_stage_in(ctx, 1, first_point, (size_t)(npoly + 1) * 8, &dfp);
-    if (rc) return rc;
-    void* dft = nullptr;
-    bool st = false;
-    rc = mr_stage_out(ctx, 2, first_tri_out, (size_t)(npoly + 1) * 8, &dft, &st);
-    if (rc) return rc;
-    rc = mr_polygon_offsets_impl(ctx, static_cast<const uint64_t*>(dfp), npoly, static_cast<uint64_t*>(dft));
-    if (rc) return rc;
-    if (st) {
-        rc = mr_copy_back(ctx, first_tri_out, dft, (size_t)(npoly + 1) * 8);
-        if (rc) return rc;
-    }
-    return mr_finish_host_io(ctx);
+    mr_staging io(ctx);
+    const uint64_t* dfp = io.in(MR_SLOT_FP, first_point, (size_t)(npoly + 1) * 8);
+    uint64_t* dft = io.out(MR_SLOT_FT, first_tri_out, (size_t)(npoly + 1) * 8);
+    if (io.rc) return io.rc;
+    return io.finish(mr_polygon_offsets_impl(ctx, dfp, npoly, dft));
 }
 
 int mr_polygon_offsets_rings(mr_context* ctx, const uint64_t* first_point, const uint64_t* first_ring, uint32_t npoly,
                              uint64_t* first_tri_out) {
     if (!ctx || !first_point || !first_ring || !first_tri_out) return MR_E_BADARG;
     MR_CUDA(ctx, cudaSetDevice(ctx->device));
-    const void* dfp = nullptr;
-    int rc = mr_stage_in(ctx, 1, first_point, (size_t)(npoly + 1) * 8, &dfp);
-    if (rc) return rc;
-    const void* dfr = nullptr;
-    rc = mr_stage_in(ctx, 14, first_ring, (size_t)(npoly + 1) * 8, &dfr);
-    if (rc) return rc;
-    void* dft = nullptr;
-    bool st = false;
-    rc = mr_stage_out(ctx, 2, first_tri_out, (size_t)(npoly + 1) * 8, &dft, &st);
-    if (rc) return rc;
-    rc = mr_polygon_ring_counts(ctx, static_cast<const uint64_t*>(dfp), static_cast<const uint64_t*>(dfr), npoly, 2,
-                                static_cast<uint64_t*>(dft));
-    if (rc) return rc;
-    if (st) {
-        rc = mr_copy_back(ctx, first_tri_out, dft, (size_t)(npoly + 1) * 8);
-        if (rc) return rc;
-    }
-    return mr_finish_host_io(ctx);
+    mr_staging io(ctx);
+    const uint64_t* dfp = io.in(MR_SLOT_FP, first_point, (size_t)(npoly + 1) * 8);
+    const uint64_t* dfr = io.in(MR_SLOT_FR, first_ring, (size_t)(npoly + 1) * 8);
+    uint64_t* dft = io.out(MR_SLOT_FT, first_tri_out, (size_t)(npoly + 1) * 8);
+    if (io.rc) return io.rc;
+    return io.finish(mr_polygon_ring_counts(ctx, dfp, dfr, npoly, 2, dft));
 }
 
 int mr_polygon_draw_range(uint64_t first_tri_i, uint64_t first_tri_next, uint64_t tri_base, mr_draw_range* out) {
@@ -555,121 +510,75 @@ int triangulate_common(mr_context* ctx, const mr_polygon_job* job, bool earclip,
         if (mr_triangulate_small(ctx, &j, &rc_small)) return rc_small;
     }
 
-    mr_polygon_job d = j;
-    const bool fp_dev = mr_is_device_ptr(j.first_point);
-    const bool ft_dev = mr_is_device_ptr(j.first_tri);
-    // sizes of the data arrays: known from first_point/first_tri when those live on the host
-    uint64_t npts = 0, ntri = 0;
-    bool need_sizes = !mr_is_device_ptr(j.xy) || !mr_is_device_ptr(j.vtx_out);
+    mr_staging io(ctx);
+    // Host buffers need the sizes of their arrays: xy covers [point_base, first_point[npoly]), the vertex buffer
+    // [tri_base, first_tri[npoly]) and ring_start [ring_base, first_ring[npoly]).  Offsets that live on the device are
+    // read with one synchronisation, and all of them are checked before any data moves.
+    const bool need_sizes = !io.where(j.xy).device || !io.where(j.vtx_out).device;
+    const bool need_nrings = rings && !io.where(rings->ring_start).device;
+    uint64_t fp_ends[2] = {0, 0}, ft_ends[2] = {0, 0}, fr_end = 0;
+    bool enqueued = false;
+    cudaError_t e = cudaSuccess;
+    auto read = [&](const uint64_t* a, uint32_t i, uint64_t* v) {
+        if (!io.where(a).device) {
+            *v = a[i];
+        } else {
+            enqueued = true;
+            if (e == cudaSuccess) e = cudaMemcpyAsync(v, a + i, 8, cudaMemcpyDeviceToHost, ctx->stream);
+        }
+    };
     if (need_sizes) {
-        uint64_t fp_ends[2], ft_ends[2];
-        if (fp_dev) {
-            MR_CUDA(ctx, cudaMemcpyAsync(&fp_ends[0], j.first_point, 8, cudaMemcpyDeviceToHost, ctx->stream));
-            MR_CUDA(ctx, cudaMemcpyAsync(&fp_ends[1], j.first_point + j.npoly, 8, cudaMemcpyDeviceToHost, ctx->stream));
-        } else {
-            fp_ends[0] = j.first_point[0];
-            fp_ends[1] = j.first_point[j.npoly];
-        }
-        if (ft_dev) {
-            MR_CUDA(ctx, cudaMemcpyAsync(&ft_ends[0], j.first_tri, 8, cudaMemcpyDeviceToHost, ctx->stream));
-            MR_CUDA(ctx, cudaMemcpyAsync(&ft_ends[1], j.first_tri + j.npoly, 8, cudaMemcpyDeviceToHost, ctx->stream));
-        } else {
-            ft_ends[0] = j.first_tri[0];
-            ft_ends[1] = j.first_tri[j.npoly];
-        }
-        if (fp_dev || ft_dev) MR_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        if (fp_ends[0] < j.point_base || ft_ends[0] < j.tri_base) return mr_fail(ctx, MR_E_BADARG, "polygons: base beyond first offset");
-        npts = fp_ends[1] - j.point_base;   // xy covers [point_base, first_point[npoly])
-        ntri = ft_ends[1] - j.tri_base;
+        read(j.first_point, 0, &fp_ends[0]);
+        read(j.first_point, j.npoly, &fp_ends[1]);
+        read(j.first_tri, 0, &ft_ends[0]);
+        read(j.first_tri, j.npoly, &ft_ends[1]);
     }
-    const void* p = nullptr;
-    int rc;
-    rc = mr_stage_in(ctx, 0, j.xy, (size_t)npts * 8, &p);
-    if (rc) return rc;
-    d.xy = static_cast<const float*>(p);
-    rc = mr_stage_in(ctx, 1, j.first_point, (size_t)(j.npoly + 1) * 8, &p);
-    if (rc) return rc;
-    d.first_point = static_cast<const uint64_t*>(p);
-    rc = mr_stage_in(ctx, 2, j.first_tri, (size_t)(j.npoly + 1) * 8, &p);
-    if (rc) return rc;
-    d.first_tri = static_cast<const uint64_t*>(p);
-    d.offset_prime = nullptr;
-    if (j.offset_prime && !earclip) {
-        rc = mr_stage_in(ctx, 3, j.offset_prime, (size_t)j.npoly * 8, &p);
-        if (rc) return rc;
-        d.offset_prime = static_cast<const uint32_t*>(p);
-    }
+    if (need_nrings) read(rings->first_ring, j.npoly, &fr_end);
+    if (e != cudaSuccess) return mr_fail(ctx, MR_E_CUDA, "cudaMemcpyAsync", e);
+    if (enqueued) MR_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if (need_sizes && (fp_ends[0] < j.point_base || ft_ends[0] < j.tri_base))
+        return mr_fail(ctx, MR_E_BADARG, "polygons: base beyond first offset");
+    if (need_nrings && fr_end < rings->ring_base) return mr_fail(ctx, MR_E_BADARG, "polygons: ring_base beyond the last ring");
+    const uint64_t npts = need_sizes ? fp_ends[1] - j.point_base : 0;
+    const uint64_t ntri = need_sizes ? ft_ends[1] - j.tri_base : 0;
+    const uint64_t nrings = need_nrings ? fr_end - rings->ring_base : 0;
+
+    mr_polygon_job d = j;
+    d.xy = io.in(MR_SLOT_XY, j.xy, (size_t)npts * 8);
+    d.first_point = io.in(MR_SLOT_FP, j.first_point, (size_t)(j.npoly + 1) * 8);
+    d.first_tri = io.in(MR_SLOT_FT, j.first_tri, (size_t)(j.npoly + 1) * 8);
+    d.offset_prime = earclip ? nullptr : io.in(MR_SLOT_OP, j.offset_prime, (size_t)j.npoly * 8);
     mr_polygon_rings dr{};
     if (rings) {
-        // ring_start covers [ring_base, first_ring[npoly]): its size is needed only when it lives on the host
-        uint64_t nrings = 0;
-        if (!mr_is_device_ptr(rings->ring_start)) {
-            uint64_t fr_end = 0;
-            if (mr_is_device_ptr(rings->first_ring)) {
-                MR_CUDA(ctx, cudaMemcpyAsync(&fr_end, rings->first_ring + j.npoly, 8, cudaMemcpyDeviceToHost, ctx->stream));
-                MR_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-            } else {
-                fr_end = rings->first_ring[j.npoly];
-            }
-            if (fr_end < rings->ring_base) return mr_fail(ctx, MR_E_BADARG, "polygons: ring_base beyond the last ring");
-            nrings = fr_end - rings->ring_base;
-        }
+        dr.first_ring = io.in(MR_SLOT_FR, rings->first_ring, (size_t)(j.npoly + 1) * 8);
         dr.ring_base = rings->ring_base;
-        rc = mr_stage_in(ctx, 14, rings->first_ring, (size_t)(j.npoly + 1) * 8, &p);
-        if (rc) return rc;
-        dr.first_ring = static_cast<const uint64_t*>(p);
-        rc = mr_stage_in(ctx, 15, rings->ring_start, (size_t)nrings * 8, &p);
-        if (rc) return rc;
-        dr.ring_start = static_cast<const uint64_t*>(p);
+        dr.ring_start = io.in(MR_SLOT_RS, rings->ring_start, (size_t)nrings * 8);
     }
-    bool sv = false, sb = false, ss = false, sn = false;
-    void* q = nullptr;
+    bool sv = false;
     const size_t vbytes = (size_t)ntri * 3u * j.layout.stride;
     // The vertex range is written over the whole kernel run: into pinned host memory the kernels store
     // directly (zero-copy over PCIe, overlapping the transfer with the triangulation; measured 10.3 vs
     // 12.3 ms for the 100k batch); pageable host memory is staged and copied back.
-    if (void* alias = mr_pinned_device_alias(j.vtx_out)) {
-        q = alias;
+    if (void* alias = io.where(j.vtx_out).alias) {
+        d.vtx_out = alias;
         ctx->host_io = true;  // the kernels store into the caller's host buffer: the call returns after they finish
     } else {
-        rc = mr_stage_out(ctx, 4, j.vtx_out, vbytes, &q, &sv);
-        if (rc) return rc;
+        d.vtx_out = io.out(MR_SLOT_VTX, j.vtx_out, vbytes, &sv);
     }
-    d.vtx_out = q;
-    if (j.bbox_out) {
-        rc = mr_stage_out(ctx, 5, j.bbox_out, (size_t)j.npoly * 16, &q, &sb);
-        if (rc) return rc;
-        d.bbox_out = static_cast<float*>(q);
-    }
-    if (j.status_out) {
-        rc = mr_stage_out(ctx, 6, j.status_out, (size_t)j.npoly * 4, &q, &ss);
-        if (rc) return rc;
-        d.status_out = static_cast<uint32_t*>(q);
-    }
-    if (j.ntri_out) {
-        rc = mr_stage_out(ctx, 7, j.ntri_out, (size_t)j.npoly * 4, &q, &sn);
-        if (rc) return rc;
-        d.ntri_out = static_cast<uint32_t*>(q);
-    }
-    rc = rings     ? mr_triangulate_earclip_holes_impl(ctx, &d, &dr)
-         : earclip ? mr_triangulate_earclip_impl(ctx, &d)
-                   : mr_triangulate_impl(ctx, &d, fp_dev ? nullptr : j.first_point);
+    d.bbox_out = io.out(MR_SLOT_BBOX, j.bbox_out, (size_t)j.npoly * 16);
+    d.status_out = io.out(MR_SLOT_STATUS, j.status_out, (size_t)j.npoly * 4);
+    d.ntri_out = io.out(MR_SLOT_NTRI, j.ntri_out, (size_t)j.npoly * 4);
+    if (io.rc) return io.rc;
+    const int rc = rings     ? mr_triangulate_earclip_holes_impl(ctx, &d, &dr)
+                   : earclip ? mr_triangulate_earclip_impl(ctx, &d)
+                             : mr_triangulate_impl(ctx, &d, io.where(j.first_point).device ? nullptr : j.first_point);
     if (rc) return rc;
-    if (sv) {
-        // the polygons of this job own [first_tri[0], first_tri[npoly]) only
-        uint64_t ft0 = ft_dev ? 0 : j.first_tri[0];
-        if (ft_dev) {
-            MR_CUDA(ctx, cudaMemcpyAsync(&ft0, j.first_tri, 8, cudaMemcpyDeviceToHost, ctx->stream));
-            MR_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-        }
-        const size_t off = (size_t)(ft0 - j.tri_base) * 3u * j.layout.stride;
-        rc = mr_copy_back(ctx, static_cast<unsigned char*>(j.vtx_out) + off, static_cast<unsigned char*>(d.vtx_out) + off, vbytes - off);
-        if (rc) return rc;
+    if (sv) {  // the polygons of this job own [first_tri[0], first_tri[npoly]) only
+        const size_t off = (size_t)(ft_ends[0] - j.tri_base) * 3u * j.layout.stride;
+        MR_CUDA(ctx, cudaMemcpyAsync(static_cast<unsigned char*>(j.vtx_out) + off, static_cast<unsigned char*>(d.vtx_out) + off,
+                                     vbytes - off, cudaMemcpyDeviceToHost, ctx->stream));
     }
-    if (sb) { rc = mr_copy_back(ctx, j.bbox_out, d.bbox_out, (size_t)j.npoly * 16); if (rc) return rc; }
-    if (ss) { rc = mr_copy_back(ctx, j.status_out, d.status_out, (size_t)j.npoly * 4); if (rc) return rc; }
-    if (sn) { rc = mr_copy_back(ctx, j.ntri_out, d.ntri_out, (size_t)j.npoly * 4); if (rc) return rc; }
-    return mr_finish_host_io(ctx);
+    return io.finish(MR_OK);
 }
 }  // namespace
 
@@ -685,39 +594,21 @@ int mr_triangulate_earclip_holes(mr_context* ctx, const mr_polygon_job* job, con
 int mr_selftest_crossing(mr_context* ctx, const float* q, uint64_t count, int8_t* sign_out) {
     if (!ctx || (count && (!q || !sign_out))) return MR_E_BADARG;
     MR_CUDA(ctx, cudaSetDevice(ctx->device));
-    const void* din = nullptr;
-    int rc = mr_stage_in(ctx, 0, q, (size_t)count * 36, &din);
-    if (rc) return rc;
-    void* dout = nullptr;
-    bool st = false;
-    rc = mr_stage_out(ctx, 4, sign_out, (size_t)count, &dout, &st);
-    if (rc) return rc;
-    rc = mr_selftest_crossing_impl(ctx, static_cast<const float*>(din), count, static_cast<int8_t*>(dout));
-    if (rc) return rc;
-    if (st) {
-        rc = mr_copy_back(ctx, sign_out, dout, (size_t)count);
-        if (rc) return rc;
-    }
-    return mr_finish_host_io(ctx);
+    mr_staging io(ctx);
+    const float* din = io.in(MR_SLOT_XY, q, (size_t)count * 36);
+    int8_t* dout = io.out(MR_SLOT_VTX, sign_out, (size_t)count);
+    if (io.rc) return io.rc;
+    return io.finish(mr_selftest_crossing_impl(ctx, din, count, dout));
 }
 
 int mr_selftest_orient(mr_context* ctx, const float* abc, uint64_t count, int8_t* sign_out) {
     if (!ctx || (count && (!abc || !sign_out))) return MR_E_BADARG;
     MR_CUDA(ctx, cudaSetDevice(ctx->device));
-    const void* din = nullptr;
-    int rc = mr_stage_in(ctx, 0, abc, (size_t)count * 24, &din);
-    if (rc) return rc;
-    void* dout = nullptr;
-    bool st = false;
-    rc = mr_stage_out(ctx, 4, sign_out, (size_t)count, &dout, &st);
-    if (rc) return rc;
-    rc = mr_selftest_orient_impl(ctx, static_cast<const float*>(din), count, static_cast<int8_t*>(dout));
-    if (rc) return rc;
-    if (st) {
-        rc = mr_copy_back(ctx, sign_out, dout, (size_t)count);
-        if (rc) return rc;
-    }
-    return mr_finish_host_io(ctx);
+    mr_staging io(ctx);
+    const float* din = io.in(MR_SLOT_XY, abc, (size_t)count * 24);
+    int8_t* dout = io.out(MR_SLOT_VTX, sign_out, (size_t)count);
+    if (io.rc) return io.rc;
+    return io.finish(mr_selftest_orient_impl(ctx, din, count, dout));
 }
 
 int mr_triangulate_tier_counts(mr_context* ctx, uint32_t out[8]) {
@@ -760,38 +651,20 @@ int mr_unirand_seed_batch(mr_context* ctx, const uint64_t* first_point, uint32_t
                           uint64_t poly_index0, uint32_t* offset_prime_out) {
     if (!ctx || !first_point || !offset_prime_out) return MR_E_BADARG;
     MR_CUDA(ctx, cudaSetDevice(ctx->device));
-    const void* dfp = nullptr;
-    int rc = mr_stage_in(ctx, 1, first_point, (size_t)(npoly + 1) * 8, &dfp);
-    if (rc) return rc;
-    void* dout = nullptr;
-    bool st = false;
-    rc = mr_stage_out(ctx, 3, offset_prime_out, (size_t)npoly * 8, &dout, &st);
-    if (rc) return rc;
-    rc = mr_unirand_seed_batch_impl(ctx, static_cast<const uint64_t*>(dfp), npoly, seed, poly_index0,
-                                    static_cast<uint32_t*>(dout));
-    if (rc) return rc;
-    if (st) {
-        rc = mr_copy_back(ctx, offset_prime_out, dout, (size_t)npoly * 8);
-        if (rc) return rc;
-    }
-    return mr_finish_host_io(ctx);
+    mr_staging io(ctx);
+    const uint64_t* dfp = io.in(MR_SLOT_FP, first_point, (size_t)(npoly + 1) * 8);
+    uint32_t* dout = io.out(MR_SLOT_OP, offset_prime_out, (size_t)npoly * 8);
+    if (io.rc) return io.rc;
+    return io.finish(mr_unirand_seed_batch_impl(ctx, dfp, npoly, seed, poly_index0, dout));
 }
 
 int mr_synth_heightmap_u16(mr_context* ctx, uint64_t seed, uint32_t n, uint32_t row0, uint32_t rows, uint16_t* out) {
     if (!ctx || !out) return MR_E_BADARG;
     MR_CUDA(ctx, cudaSetDevice(ctx->device));
-    void* dout = nullptr;
-    bool st = false;
-    const size_t bytes = (size_t)rows * n * 2;
-    int rc = mr_stage_out(ctx, 4, out, bytes, &dout, &st);
-    if (rc) return rc;
-    rc = mr_synth_heightmap_u16_impl(ctx, seed, n, row0, rows, static_cast<uint16_t*>(dout));
-    if (rc) return rc;
-    if (st) {
-        rc = mr_copy_back(ctx, out, dout, bytes);
-        if (rc) return rc;
-    }
-    return mr_finish_host_io(ctx);
+    mr_staging io(ctx);
+    uint16_t* dout = io.out(MR_SLOT_VTX, out, (size_t)rows * n * 2);
+    if (io.rc) return io.rc;
+    return io.finish(mr_synth_heightmap_u16_impl(ctx, seed, n, row0, rows, dout));
 }
 
 int mr_synth_polygons(mr_context* ctx, uint64_t seed, uint64_t poly_index0, const uint64_t* first_point,
@@ -805,25 +678,16 @@ int mr_synth_polygons_family(mr_context* ctx, int family, uint64_t seed, uint64_
     if (family != MR_FAMILY_STAR && family != MR_FAMILY_ELLIPSE && family != MR_FAMILY_ZIPPER)
         return mr_fail(ctx, MR_E_BADARG, "synth_polygons: unknown family");
     MR_CUDA(ctx, cudaSetDevice(ctx->device));
-    const void* dfp = nullptr;
-    int rc = mr_stage_in(ctx, 1, first_point, (size_t)(npoly + 1) * 8, &dfp);
-    if (rc) return rc;
-    void* dout = nullptr;
-    bool st = false;
+    mr_staging io(ctx);
     size_t bytes = 0;
-    if (!mr_is_device_ptr(xy_out)) {
-        if (mr_is_device_ptr(first_point)) return mr_fail(ctx, MR_E_BADARG, "synth_polygons: host xy_out needs host first_point");
+    if (!io.where(xy_out).device) {
+        if (io.where(first_point).device) return mr_fail(ctx, MR_E_BADARG, "synth_polygons: host xy_out needs host first_point");
         bytes = (size_t)(first_point[npoly] - first_point[0]) * 8;
     }
-    rc = mr_stage_out(ctx, 0, xy_out, bytes, &dout, &st);
-    if (rc) return rc;
-    rc = mr_synth_polygons_impl(ctx, family, seed, poly_index0, static_cast<const uint64_t*>(dfp), npoly, static_cast<float*>(dout));
-    if (rc) return rc;
-    if (st) {
-        rc = mr_copy_back(ctx, xy_out, dout, bytes);
-        if (rc) return rc;
-    }
-    return mr_finish_host_io(ctx);
+    const uint64_t* dfp = io.in(MR_SLOT_FP, first_point, (size_t)(npoly + 1) * 8);
+    float* dout = io.out(MR_SLOT_XY, xy_out, bytes);
+    if (io.rc) return io.rc;
+    return io.finish(mr_synth_polygons_impl(ctx, family, seed, poly_index0, dfp, npoly, dout));
 }
 
 int mr_ipc_export(mr_context* ctx, void* dev, unsigned char handle_out[MR_IPC_HANDLE_BYTES]) {

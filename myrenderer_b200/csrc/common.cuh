@@ -10,7 +10,32 @@
 #include <vector>
 #include "../../include/myrenderer_b200.h"
 
-#define MR_NUM_SCRATCH 16
+// ---- scratch slots -----------------------------------------------------------------------------------------
+// The growing device buffers of mr_context (mr_scratch), by what they hold.  Rule: within one call, no two live buffers
+// share a slot; a slot that several entry points use holds one buffer of whichever call is running.
+enum mr_slot {
+    MR_SLOT_XY,      // polygon points (triangulation in, mr_synth_polygons_family out); the heightmap (terrain build, tile
+                     // bounds, mr_heightmap_normalize); the tile boxes (cull); the self-test inputs
+    MR_SLOT_FP,      // first_point (triangulation, offsets, unirand seeds, polygon synthesis); the cull's visible flags
+    MR_SLOT_FT,      // first_tri (triangulation in, offsets out); the cull's visible tile ids
+    MR_SLOT_OP,      // offset_prime (triangulation in, mr_unirand_seed_batch out); the cull's two counts
+    MR_SLOT_VTX,     // vertex buffers (triangulation, terrain build); tile bounds; normalised heights; self-test signs;
+                     // the synthetic heightmap
+    MR_SLOT_BBOX,    // polygon bounding boxes; terrain index buffers (build, cull)
+    MR_SLOT_STATUS,  // polygon status
+    MR_SLOT_NTRI,    // polygon triangle counts
+    MR_SLOT_WORK,    // reference-path work list; its header outlives the call (mr_triangulate_tier_counts)
+    MR_SLOT_TIER1,   // general-path workspaces of polygons handed over by the fast path
+    MR_SLOT_MISC,    // prefix-sum temporary (mr_polygon_offsets_impl, mr_polygon_ring_counts); the cull's work list;
+                     // the fast-division self-test's counter
+    MR_SLOT_TIER1B,  // general-path workspaces of the 1025..MR_MAX_POLYGON_POINTS class
+    MR_SLOT_PAR,     // parallel-search scratch of the n <= 64 kernel
+    MR_SLOT_EC_WORK, // ear-clip work list (apart from MR_SLOT_WORK, so the tier counts survive an ear-clip call)
+    MR_SLOT_FR,      // first_ring
+    MR_SLOT_RS,      // ring_start
+    MR_NUM_SCRATCH
+};
+static_assert(MR_NUM_SCRATCH == 16, "scratch slot count");
 
 constexpr int MR_NUM_AUX = 12;
 
@@ -78,32 +103,7 @@ inline int mr_fail(mr_context* ctx, int code, const char* what, cudaError_t e = 
         (ctx)->launches++;                                              \
     } while (0)
 
-// true when the pointer can be dereferenced by a kernel on ctx->device
-inline bool mr_is_device_ptr(const void* p) {
-    if (!p) return false;
-    cudaPointerAttributes a;
-    cudaError_t e = cudaPointerGetAttributes(&a, p);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        return false;
-    }
-    return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
-}
-
-// Pinned (page-locked) host memory is reachable from kernels under UVA: returns its device alias, or
-// nullptr when `p` is not pinned host memory.  Used for outputs that are produced over a long kernel,
-// where storing straight over PCIe overlaps the transfer with the compute.
-inline void* mr_pinned_device_alias(void* p) {
-    if (!p) return nullptr;
-    cudaPointerAttributes a;
-    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
-        cudaGetLastError();
-        return nullptr;
-    }
-    return a.type == cudaMemoryTypeHost ? a.devicePointer : nullptr;
-}
-
-inline int mr_scratch(mr_context* ctx, int slot, size_t bytes, void** out) {
+inline int mr_scratch(mr_context* ctx, mr_slot slot, size_t bytes, void** out) {
     if (bytes == 0) bytes = 16;
     if (ctx->scratch_bytes[slot] < bytes) {
         if (ctx->scratch[slot]) {
@@ -121,37 +121,6 @@ inline int mr_scratch(mr_context* ctx, int slot, size_t bytes, void** out) {
     return MR_OK;
 }
 
-// Input staging: returns a device pointer holding `bytes` of src (src itself when already device).
-inline int mr_stage_in(mr_context* ctx, int slot, const void* src, size_t bytes, const void** dev) {
-    if (!src || bytes == 0 || mr_is_device_ptr(src)) {
-        *dev = src;
-        return MR_OK;
-    }
-    ctx->host_io = true;  // a pinned source is copied asynchronously: the call must not return before it is read
-    void* d = nullptr;
-    int rc = mr_scratch(ctx, slot, bytes, &d);
-    if (rc) return rc;
-    MR_CUDA(ctx, cudaMemcpyAsync(d, src, bytes, cudaMemcpyHostToDevice, ctx->stream));
-    *dev = d;
-    return MR_OK;
-}
-
-// Output staging: device buffer to produce into; *staged says a copy-back is needed.
-inline int mr_stage_out(mr_context* ctx, int slot, void* dst, size_t bytes, void** dev, bool* staged) {
-    *staged = false;
-    if (!dst || bytes == 0 || mr_is_device_ptr(dst)) {
-        *dev = dst;
-        return MR_OK;
-    }
-    ctx->host_io = true;
-    void* d = nullptr;
-    int rc = mr_scratch(ctx, slot, bytes, &d);
-    if (rc) return rc;
-    *dev = d;
-    *staged = true;
-    return MR_OK;
-}
-
 // End of an entry point: if the call touched caller host memory in any way, wait for the stream, so that inputs may
 // be reused and outputs read as soon as the call returns (the header's contract for host pointers).
 inline int mr_finish_host_io(mr_context* ctx) {
@@ -162,10 +131,82 @@ inline int mr_finish_host_io(mr_context* ctx) {
     return MR_OK;
 }
 
-inline int mr_copy_back(mr_context* ctx, void* dst, const void* dev, size_t bytes) {
-    MR_CUDA(ctx, cudaMemcpyAsync(dst, dev, bytes, cudaMemcpyDeviceToHost, ctx->stream));
-    return MR_OK;
-}
+// Where a caller buffer lives: device (or managed) memory that kernels use as it is, pinned host memory, which kernels
+// reach through its device alias under UVA, or pageable host memory.  A null pointer counts as device memory.
+struct mr_loc {
+    bool device;
+    void* alias;  // pinned host memory: its device alias
+};
+
+// The caller buffers of one entry point: validate the arguments first, then stage inputs and outputs, run the work on
+// ctx->stream, and end with finish().  Each caller pointer is classified once (one cudaPointerGetAttributes).  Host
+// inputs are copied into scratch slot `slot`; host outputs are produced in it and copied back over the whole range by
+// finish(), or by the caller when it asks for `staged` (a part of the buffer, or on another stream).  The first failure
+// is kept in rc and turns every later step into a no-op returning null, so a caller checks rc once before its work.
+struct mr_staging {
+    mr_context* ctx;
+    int rc = MR_OK;
+
+    explicit mr_staging(mr_context* c) : ctx(c) {}
+
+    mr_loc where(const void* p) {
+        if (!p) return {true, nullptr};
+        for (int i = 0; i < nseen; ++i)
+            if (seen[i].p == p) return seen[i].loc;
+        mr_loc l{false, nullptr};
+        cudaPointerAttributes a;
+        if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+            cudaGetLastError();  // not known to CUDA: pageable host memory
+        } else {
+            l.device = a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
+            l.alias = a.type == cudaMemoryTypeHost ? a.devicePointer : nullptr;
+        }
+        if (nseen < MR_NUM_SCRATCH) seen[nseen++] = {p, l};
+        return l;
+    }
+
+    // a device pointer holding `bytes` of src (src itself when kernels can read it)
+    template <class T>
+    const T* in(mr_slot slot, const T* src, size_t bytes) {
+        if (rc) return nullptr;
+        if (bytes == 0 || where(src).device) return src;
+        ctx->host_io = true;  // a pinned source is copied asynchronously: the call must not return before it is read
+        void* d = nullptr;
+        if ((rc = mr_scratch(ctx, slot, bytes, &d))) return nullptr;
+        const cudaError_t e = cudaMemcpyAsync(d, src, bytes, cudaMemcpyHostToDevice, ctx->stream);
+        if (e != cudaSuccess) rc = mr_fail(ctx, MR_E_CUDA, "cudaMemcpyAsync", e);
+        return rc ? nullptr : static_cast<const T*>(d);
+    }
+
+    // the device buffer to produce output dst in (dst itself when kernels can write it)
+    template <class T>
+    T* out(mr_slot slot, T* dst, size_t bytes, bool* staged = nullptr) {
+        if (staged) *staged = false;
+        if (rc) return nullptr;
+        if (bytes == 0 || where(dst).device) return dst;
+        ctx->host_io = true;
+        void* d = nullptr;
+        if ((rc = mr_scratch(ctx, slot, bytes, &d))) return nullptr;
+        if (staged) *staged = true;
+        else back[nback++] = {dst, d, bytes};  // one per slot at most, by the slot rule
+        return static_cast<T*>(d);
+    }
+
+    // the end of a call whose work returned work_rc: the whole-range copy-backs in the order of their out() calls, then
+    // the synchronisation of mr_finish_host_io
+    int finish(int work_rc) {
+        if (work_rc) return work_rc;
+        for (int i = 0; i < nback; ++i)
+            MR_CUDA(ctx, cudaMemcpyAsync(back[i].dst, back[i].dev, back[i].bytes, cudaMemcpyDeviceToHost, ctx->stream));
+        return mr_finish_host_io(ctx);
+    }
+
+private:
+    struct { const void* p; mr_loc loc; } seen[MR_NUM_SCRATCH];  // (pointers past the last entry are asked again)
+    int nseen = 0;
+    struct { void* dst; const void* dev; size_t bytes; } back[MR_NUM_SCRATCH];
+    int nback = 0;
+};
 
 // ---- shared device helpers ------------------------------------------------------------
 __host__ __device__ __forceinline__ uint64_t mr_mix64(uint64_t z) {

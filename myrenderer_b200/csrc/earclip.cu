@@ -650,7 +650,7 @@ int earclip_run(mr_context* ctx, const mr_polygon_job* j, const mr_polygon_rings
     constexpr size_t ZERO_WORDS = 2 * (size_t)MR_SIZE_BINS + 64 + EC_CLASSES;
     const size_t order_bytes = ((ZERO_WORDS + npoly) * 4 + 7) / 8 * 8;
     void* work = nullptr;
-    int rc = mr_scratch(ctx, 13, order_bytes + (rings ? ((size_t)npoly + 1) * 8 : 0), &work);
+    int rc = mr_scratch(ctx, MR_SLOT_EC_WORK, order_bytes + (rings ? ((size_t)npoly + 1) * 8 : 0), &work);
     if (rc) return rc;
     uint32_t* w = static_cast<uint32_t*>(work);
     uint32_t* hist = w;
@@ -680,13 +680,7 @@ int earclip_run(mr_context* ctx, const mr_polygon_job* j, const mr_polygon_rings
     a.bbox_out = j->bbox_out;
     a.status_out = j->status_out;
     a.ntri_out = j->ntri_out;
-    a.stride = j->layout.stride;
-    a.off_x = j->layout.attr[0].offset;
-    a.off_c = j->layout.nattr > 1 ? j->layout.attr[1].offset : 0xFFFFFFFFu;
-    a.fast32 = (a.stride == 32 && j->layout.nattr == 2 && ((a.off_x == 0 && a.off_c == 16) || (a.off_x == 16 && a.off_c == 0)) &&
-                reinterpret_cast<uintptr_t>(a.vtx_out) % 32 == 0)
-                   ? 1
-                   : 0;
+    sink_layout(a, j->layout, a.vtx_out);
     a.order = order;
     a.cursor = cursor;
     a.queue_head = heads;

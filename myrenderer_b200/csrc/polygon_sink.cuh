@@ -104,3 +104,17 @@ struct Sink {
 
 __device__ __forceinline__ float fmin_acc(float acc, float v) { return v < acc ? v : acc; }
 __device__ __forceinline__ float fmax_acc(float acc, float v) { return v > acc ? v : acc; }
+
+// host: the sink fields of a polygon path's kernel arguments from the job's vertex layout and (device) vertex buffer.
+// fast32 selects the single 32-byte store, which needs stride 32, position and colour at offsets 0 and 16 in either
+// order, and a 32-byte-aligned buffer.
+template <class Args>
+inline void sink_layout(Args& a, const mr_layout& L, const void* vtx_out) {
+    a.stride = L.stride;
+    a.off_x = L.attr[0].offset;
+    a.off_c = L.nattr > 1 ? L.attr[1].offset : 0xFFFFFFFFu;
+    a.fast32 = (a.stride == 32 && L.nattr == 2 && ((a.off_x == 0 && a.off_c == 16) || (a.off_x == 16 && a.off_c == 0)) &&
+                reinterpret_cast<uintptr_t>(vtx_out) % 32 == 0)
+                   ? 1
+                   : 0;
+}

@@ -1264,8 +1264,6 @@ __global__ void unirand_seed_batch_k(const uint64_t* __restrict__ first_point, u
 enum { HDR_CLASS_BEGIN = 0, HDR_CLASS_END = CLASS_SLOTS, HDR_QUEUE_HEAD = 2 * CLASS_SLOTS, HDR_SPEC_COUNT = 5 * CLASS_SLOTS,
        HDR_GENERAL_COUNT = 6 * CLASS_SLOTS, HEADER_WORDS = 8 * CLASS_SLOTS };
 static_assert(NUM_CLASSES <= CLASS_SLOTS && 2 * NUM_CLASSES + 2 <= 3 * CLASS_SLOTS, "work-list header too small");
-enum { SLOT_XY = 0, SLOT_FP = 1, SLOT_FT = 2, SLOT_OP = 3, SLOT_VTX = 4, SLOT_BBOX = 5, SLOT_STATUS = 6, SLOT_NTRI = 7,
-       SLOT_WORK = 8, SLOT_TIER1 = 9, SLOT_MISC = 10, SLOT_TIER1B = 11, SLOT_PAR = 12 };
 
 int mr_polygon_size_sort(mr_context* ctx, const uint64_t* first_point, uint32_t npoly, uint32_t* hist, uint32_t* cursor,
                          uint32_t* class_begin, uint32_t* class_end, uint32_t* order) {
@@ -1284,7 +1282,7 @@ int mr_polygon_offsets_impl(mr_context* ctx, const uint64_t* first_point_dev, ui
                             uint64_t* first_tri_dev) {
     // counts are written into first_tri_dev[0..npoly) then scanned in place via a temp
     void* tmp = nullptr;
-    int rc = mr_scratch(ctx, SLOT_MISC, (size_t)(npoly + 1) * 8, &tmp);
+    int rc = mr_scratch(ctx, MR_SLOT_MISC, (size_t)(npoly + 1) * 8, &tmp);
     if (rc) return rc;
     const unsigned blocks = (unsigned)std::min<uint64_t>(((uint64_t)npoly + 255) / 256 + 1, 1024);
     polygon_offsets_k<<<blocks, 256, 0, ctx->stream>>>(first_point_dev, npoly, static_cast<uint64_t*>(tmp));
@@ -1297,7 +1295,7 @@ int mr_polygon_offsets_impl(mr_context* ctx, const uint64_t* first_point_dev, ui
 int mr_polygon_ring_counts(mr_context* ctx, const uint64_t* first_point, const uint64_t* first_ring, uint32_t npoly,
                            uint32_t sub, uint64_t* out) {
     void* tmp = nullptr;
-    int rc = mr_scratch(ctx, SLOT_MISC, (size_t)(npoly + 1) * 8, &tmp);
+    int rc = mr_scratch(ctx, MR_SLOT_MISC, (size_t)(npoly + 1) * 8, &tmp);
     if (rc) return rc;
     const unsigned blocks = (unsigned)std::min<uint64_t>(((uint64_t)npoly + 255) / 256 + 1, 1024);
     polygon_ring_counts_k<<<blocks, 256, 0, ctx->stream>>>(first_point, first_ring, npoly, sub, static_cast<uint64_t*>(tmp));
@@ -1454,14 +1452,7 @@ void fill_batch_args(BatchArgs& a, const mr_polygon_job* j, uint32_t* header, ui
     a.bbox_out = j->bbox_out;
     a.status_out = j->status_out;
     a.ntri_out = j->ntri_out;
-    a.stride = j->layout.stride;
-    a.off_x = j->layout.attr[0].offset;
-    a.off_c = j->layout.nattr > 1 ? j->layout.attr[1].offset : 0xFFFFFFFFu;
-    a.fast32 = (a.stride == 32 && j->layout.nattr == 2 &&
-                ((a.off_x == 0 && a.off_c == 16) || (a.off_x == 16 && a.off_c == 0)) &&
-                reinterpret_cast<uintptr_t>(a.vtx_out) % 32 == 0)
-                   ? 1
-                   : 0;
+    sink_layout(a, j->layout, a.vtx_out);
     a.order = order;
     a.class_begin = header + HDR_CLASS_BEGIN;
     a.class_end = header + HDR_CLASS_END;
@@ -1479,7 +1470,7 @@ void fill_batch_args(BatchArgs& a, const mr_polygon_job* j, uint32_t* header, ui
 int class0_scratch(mr_context* ctx, const PolyPlan& plan, BatchArgs& a) {
     void* pw = nullptr;
     const ClassLaunch& L0 = plan.first[0];
-    const int rc = mr_scratch(ctx, SLOT_PAR, (size_t)ctx->sm_count * L0.per_sm * L0.wpb * PAR_GL_BYTES, &pw);
+    const int rc = mr_scratch(ctx, MR_SLOT_PAR, (size_t)ctx->sm_count * L0.per_sm * L0.wpb * PAR_GL_BYTES, &pw);
     if (rc) return rc;
     a.par_ws = static_cast<unsigned char*>(pw);
     return MR_OK;
@@ -1496,7 +1487,7 @@ int launch_general(mr_context* ctx, BatchArgs& a, int which, uint32_t units) {
     const uint64_t need = ((uint64_t)units + wpb - 1) / wpb;
     if (need < blocks) blocks = need ? need : 1;
     void* t1 = nullptr;
-    const int rc = mr_scratch(ctx, which == 0 ? SLOT_TIER1 : SLOT_TIER1B, (size_t)blocks * wpb * L1.total, &t1);
+    const int rc = mr_scratch(ctx, which == 0 ? MR_SLOT_TIER1 : MR_SLOT_TIER1B, (size_t)blocks * wpb * L1.total, &t1);
     if (rc) return rc;
     a.tier1_ws = static_cast<unsigned char*>(t1);
     a.tier1_ws_stride = L1.total;
@@ -1522,7 +1513,7 @@ int mr_triangulate_impl(mr_context* ctx, const mr_polygon_job* j, const uint64_t
     // work-list memory: header | hist[NBINS] | cursor[NBINS] | order[npoly] | spec_list[npoly] | general_list[npoly]
     const size_t header_words = HEADER_WORDS;
     void* work = nullptr;
-    rc = mr_scratch(ctx, SLOT_WORK, (header_words + 2 * (size_t)NBINS + 3 * (size_t)npoly) * 4, &work);
+    rc = mr_scratch(ctx, MR_SLOT_WORK, (header_words + 2 * (size_t)NBINS + 3 * (size_t)npoly) * 4, &work);
     if (rc) return rc;
     uint32_t* w = static_cast<uint32_t*>(work);
     uint32_t* hist = w + header_words;
