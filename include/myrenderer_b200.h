@@ -417,6 +417,48 @@ typedef struct mr_polygon_rings {
                                    first_point[i] and is its outer boundary, the others are holes */
 } mr_polygon_rings;
 int mr_triangulate_earclip_holes(mr_context* ctx, const mr_polygon_job* job, const mr_polygon_rings* rings);
+/* ---- indexed ear clipping ------------------------------------------------------------------------------------
+ * mr_triangulate_earclip_indexed writes the triangles of mr_triangulate_earclip (rings == NULL) or of
+ * mr_triangulate_earclip_holes (rings != NULL) as point indices: three u32 per triangle into idx_out, so that the
+ * caller's own xy array, bound as a float32x2 vertex buffer, is drawn with drawIndexed (12 bytes per triangle instead
+ * of three vertices).  Bit for bit:
+ *   Same polygons, same rules: the status rules, checks, triangles, their corner order, the OVERFLOW / UNDERFILL rule,
+ *     bbox_out, status_out and ntri_out are those of the entry point named above.  With vtx_out, everything the call
+ *     writes besides idx_out is byte-identical to what that entry point writes for the same job.
+ *   Indices: polygon i's index range is idx_out[3*(first_tri[i]-tri_base) .. 3*(first_tri[i+1]-tri_base)).  For
+ *     triangle t < ntri_out[i], entries 3t, 3t+1, 3t+2 of the range are its three corners in the order its vertices are
+ *     emitted, corner k (the polygon's k-th point, k < N) as the low 32 bits of first_point[i] + k - index_base.  With
+ *     holes, k is the input point a merged-ring position was taken from, so both copies of a bridge endpoint carry the
+ *     same index.  The value is always defined; it is unambiguous while the points indexed stay below 2^32 apart.
+ *   index_base selects what the indices point into: point_base indexes the rows of xy; 0 gives absolute point numbers,
+ *     so that a job over a sub-range (a rank's shard) writes the same indices as the whole batch does, straight into a
+ *     global index buffer.
+ *   Zeros: the rest of each range is 0 -- an UNDERFILL tail, and the whole range of a DEGENERATE / TOO_LARGE /
+ *     NONFINITE polygon.  A (0, 0, 0) triangle rasterises nothing, as zeroed vertices draw nothing.
+ *   vtx_out may be NULL here (in this entry point only): the layout is then not read, and bbox_out, status_out and
+ *     ntri_out are still written.  NULL indices or idx_out, or an idx_out that is not 4-byte aligned: MR_E_BADARG.
+ *     Every check runs before any kernel, so a rejected call writes nothing.
+ *   idx_out may be a device or a host pointer like the other outputs: pinned host memory is stored into directly, a
+ *     pageable one is staged and only the job's range, [3*(first_tri[0]-tri_base), 3*(first_tri[npoly]-tri_base)), is
+ *     copied back.
+ *   Like mr_triangulate_earclip, the call leaves mr_triangulate_tier_counts and the reference path's state as they were.
+ * mr_polygon_draw_indexed_range is the indexed sibling of mr_polygon_draw_range (drawIndexed's arguments, IndexedDraw.zig's
+ * IndexBuffer): index_count = 3*(first_tri_next - first_tri_i), first_index = 3*(first_tri_i - tri_base),
+ * instance_count 1, base_vertex 0, first_instance 0; MR_E_BADARG when a range is negative or a field does not fit its
+ * u32. */
+typedef struct mr_polygon_indices {
+    uint32_t* idx_out;   /* 3 per triangle of the first_tri ranges: idx_out[3*(first_tri[i]-tri_base) ...] */
+    uint64_t index_base; /* index of point k of polygon i = (uint32_t)(first_point[i] + k - index_base)       */
+} mr_polygon_indices;
+int mr_triangulate_earclip_indexed(mr_context* ctx, const mr_polygon_job* job, const mr_polygon_rings* rings,
+                                   const mr_polygon_indices* indices);
+typedef struct mr_draw_indexed_range { /* mirror of drawIndexed's arguments / IndexedDraw.zig's IndexBuffer */
+    uint32_t index_count, instance_count, first_index;
+    int32_t base_vertex;
+    uint32_t first_instance;
+} mr_draw_indexed_range;
+int mr_polygon_draw_indexed_range(uint64_t first_tri_i, uint64_t first_tri_next, uint64_t tri_base,
+                                  mr_draw_indexed_range* out);
 /* Self-test used by the test-suite: sign_out[i] = cross(a1, b1, a2, b2, My) above for q[9i..9i+8] =
  * (a1x, a1y, b1x, b1y, a2x, a2y, b2x, b2y, My), as mr_triangulate_earclip_holes evaluates it (-1, 0, +1). */
 int mr_selftest_crossing(mr_context* ctx, const float* q /* 9 per case */, uint64_t count, int8_t* sign_out);

@@ -100,6 +100,20 @@ class MrPolygonRings(C.Structure):
     _fields_ = [("first_ring", C.c_void_p), ("ring_base", C.c_uint64), ("ring_start", C.c_void_p)]
 
 
+class MrPolygonIndices(C.Structure):
+    _fields_ = [("idx_out", C.c_void_p), ("index_base", C.c_uint64)]
+
+
+class MrDrawIndexedRange(C.Structure):
+    _fields_ = [
+        ("index_count", C.c_uint32),
+        ("instance_count", C.c_uint32),
+        ("first_index", C.c_uint32),
+        ("base_vertex", C.c_int32),
+        ("first_instance", C.c_uint32),
+    ]
+
+
 class MrError(RuntimeError):
     def __init__(self, code: int, where: str, detail: str = ""):
         self.code = code
@@ -147,6 +161,10 @@ SIGNATURES = {
     "mr_triangulate_earclip": (C.c_int, [C.c_void_p, C.POINTER(MrPolygonJob)]),
     "mr_selftest_orient": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
     "mr_triangulate_earclip_holes": (C.c_int, [C.c_void_p, C.POINTER(MrPolygonJob), C.POINTER(MrPolygonRings)]),
+    "mr_triangulate_earclip_indexed": (
+        C.c_int, [C.c_void_p, C.POINTER(MrPolygonJob), C.POINTER(MrPolygonRings), C.POINTER(MrPolygonIndices)]),
+    "mr_polygon_draw_indexed_range": (
+        C.c_int, [C.c_uint64, C.c_uint64, C.c_uint64, C.POINTER(MrDrawIndexedRange)]),
     "mr_selftest_crossing": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
     "mr_polygon_offsets_rings": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]),
     "mr_polygon_offsets": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p]),

@@ -492,18 +492,34 @@ int mr_polygon_draw_range(uint64_t first_tri_i, uint64_t first_tri_next, uint64_
     return MR_OK;
 }
 
+int mr_polygon_draw_indexed_range(uint64_t first_tri_i, uint64_t first_tri_next, uint64_t tri_base, mr_draw_indexed_range* out) {
+    if (!out || first_tri_next < first_tri_i || first_tri_i < tri_base) return MR_E_BADARG;
+    const uint64_t prims = first_tri_next - first_tri_i, off = first_tri_i - tri_base;
+    if (prims > 0xFFFFFFFFull / 3 || off > 0xFFFFFFFFull / 3) return MR_E_BADARG;  // drawIndexed's fields are u32
+    out->index_count = (uint32_t)(prims * 3);
+    out->instance_count = 1;
+    out->first_index = (uint32_t)(off * 3);
+    out->base_vertex = 0;
+    out->first_instance = 0;
+    return MR_OK;
+}
+
 namespace {
-// mr_triangulate_batch, mr_triangulate_earclip and mr_triangulate_earclip_holes (rings != nullptr): the same checks,
+// mr_triangulate_batch, mr_triangulate_earclip, mr_triangulate_earclip_holes (rings != nullptr) and
+// mr_triangulate_earclip_indexed (indices != nullptr, checked by the caller; vtx_out may then be null): the same checks,
 // staging and copy-back; ear clipping takes no edge order and has no small-batch path.
-int triangulate_common(mr_context* ctx, const mr_polygon_job* job, bool earclip, const mr_polygon_rings* rings = nullptr) {
+int triangulate_common(mr_context* ctx, const mr_polygon_job* job, bool earclip, const mr_polygon_rings* rings = nullptr,
+                       const mr_polygon_indices* indices = nullptr) {
     if (!ctx || !job) return MR_E_BADARG;
     if (rings && (!rings->first_ring || !rings->ring_start) && job->npoly) return mr_fail(ctx, MR_E_BADARG, "polygons: null ring pointer");
     const mr_polygon_job& j = *job;
     if (j.npoly == 0) return MR_OK;
-    if (!j.xy || !j.first_point || !j.first_tri || !j.vtx_out) return mr_fail(ctx, MR_E_BADARG, "polygons: null pointer");
-    if (!layout_ok(&j.layout, 1, 2)) return mr_fail(ctx, MR_E_BADARG, "polygons: bad vertex layout");
-    if (j.layout.nattr > 1 && j.layout.attr[1].ncomp < 3) return mr_fail(ctx, MR_E_BADARG, "polygons: colour needs 3 components");
-    if (reinterpret_cast<uintptr_t>(j.vtx_out) & 3u) return mr_fail(ctx, MR_E_BADARG, "polygons: vtx_out must be 4-byte aligned");
+    if (!j.xy || !j.first_point || !j.first_tri || (!j.vtx_out && !indices)) return mr_fail(ctx, MR_E_BADARG, "polygons: null pointer");
+    if (j.vtx_out) {
+        if (!layout_ok(&j.layout, 1, 2)) return mr_fail(ctx, MR_E_BADARG, "polygons: bad vertex layout");
+        if (j.layout.nattr > 1 && j.layout.attr[1].ncomp < 3) return mr_fail(ctx, MR_E_BADARG, "polygons: colour needs 3 components");
+        if (reinterpret_cast<uintptr_t>(j.vtx_out) & 3u) return mr_fail(ctx, MR_E_BADARG, "polygons: vtx_out must be 4-byte aligned");
+    }
     MR_CUDA(ctx, cudaSetDevice(ctx->device));
     if (!earclip) {  // the reference's own call shape (Polygon.create_polygon: one small polygon, everything in host memory)
         int rc_small = MR_OK;
@@ -511,10 +527,10 @@ int triangulate_common(mr_context* ctx, const mr_polygon_job* job, bool earclip,
     }
 
     mr_staging io(ctx);
-    // Host buffers need the sizes of their arrays: xy covers [point_base, first_point[npoly]), the vertex buffer
-    // [tri_base, first_tri[npoly]) and ring_start [ring_base, first_ring[npoly]).  Offsets that live on the device are
-    // read with one synchronisation, and all of them are checked before any data moves.
-    const bool need_sizes = !io.where(j.xy).device || !io.where(j.vtx_out).device;
+    // Host buffers need the sizes of their arrays: xy covers [point_base, first_point[npoly]), the vertex and index
+    // buffers [tri_base, first_tri[npoly]) and ring_start [ring_base, first_ring[npoly]).  Offsets that live on the device
+    // are read with one synchronisation, and all of them are checked before any data moves.
+    const bool need_sizes = !io.where(j.xy).device || !io.where(j.vtx_out).device || (indices && !io.where(indices->idx_out).device);
     const bool need_nrings = rings && !io.where(rings->ring_start).device;
     uint64_t fp_ends[2] = {0, 0}, ft_ends[2] = {0, 0}, fr_end = 0;
     bool enqueued = false;
@@ -555,7 +571,7 @@ int triangulate_common(mr_context* ctx, const mr_polygon_job* job, bool earclip,
         dr.ring_start = io.in(MR_SLOT_RS, rings->ring_start, (size_t)nrings * 8);
     }
     bool sv = false;
-    const size_t vbytes = (size_t)ntri * 3u * j.layout.stride;
+    const size_t vbytes = j.vtx_out ? (size_t)ntri * 3u * j.layout.stride : 0;
     // The vertex range is written over the whole kernel run: into pinned host memory the kernels store
     // directly (zero-copy over PCIe, overlapping the transfer with the triangulation; measured 10.3 vs
     // 12.3 ms for the 100k batch); pageable host memory is staged and copied back.
@@ -568,8 +584,21 @@ int triangulate_common(mr_context* ctx, const mr_polygon_job* job, bool earclip,
     d.bbox_out = io.out(MR_SLOT_BBOX, j.bbox_out, (size_t)j.npoly * 16);
     d.status_out = io.out(MR_SLOT_STATUS, j.status_out, (size_t)j.npoly * 4);
     d.ntri_out = io.out(MR_SLOT_NTRI, j.ntri_out, (size_t)j.npoly * 4);
+    // the index range like the vertex range: pinned memory stored into directly, pageable memory staged
+    mr_polygon_indices di{};
+    bool si = false;
+    if (indices) {
+        di.index_base = indices->index_base;
+        if (void* alias = io.where(indices->idx_out).alias) {
+            di.idx_out = static_cast<uint32_t*>(alias);
+            ctx->host_io = true;
+        } else {
+            di.idx_out = io.out(MR_SLOT_IDX, indices->idx_out, (size_t)ntri * 12u, &si);
+        }
+    }
     if (io.rc) return io.rc;
-    const int rc = rings     ? mr_triangulate_earclip_holes_impl(ctx, &d, &dr)
+    const int rc = indices   ? mr_triangulate_earclip_indexed_impl(ctx, &d, rings ? &dr : nullptr, &di)
+                   : rings   ? mr_triangulate_earclip_holes_impl(ctx, &d, &dr)
                    : earclip ? mr_triangulate_earclip_impl(ctx, &d)
                              : mr_triangulate_impl(ctx, &d, io.where(j.first_point).device ? nullptr : j.first_point);
     if (rc) return rc;
@@ -577,6 +606,11 @@ int triangulate_common(mr_context* ctx, const mr_polygon_job* job, bool earclip,
         const size_t off = (size_t)(ft_ends[0] - j.tri_base) * 3u * j.layout.stride;
         MR_CUDA(ctx, cudaMemcpyAsync(static_cast<unsigned char*>(j.vtx_out) + off, static_cast<unsigned char*>(d.vtx_out) + off,
                                      vbytes - off, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    if (si) {
+        const size_t off = (size_t)(ft_ends[0] - j.tri_base) * 3u;
+        MR_CUDA(ctx, cudaMemcpyAsync(indices->idx_out + off, di.idx_out + off, ((size_t)ntri * 3u - off) * 4u,
+                                     cudaMemcpyDeviceToHost, ctx->stream));
     }
     return io.finish(MR_OK);
 }
@@ -589,6 +623,13 @@ int mr_triangulate_earclip(mr_context* ctx, const mr_polygon_job* job) { return 
 int mr_triangulate_earclip_holes(mr_context* ctx, const mr_polygon_job* job, const mr_polygon_rings* rings) {
     if (!rings) return MR_E_BADARG;
     return triangulate_common(ctx, job, true, rings);
+}
+
+int mr_triangulate_earclip_indexed(mr_context* ctx, const mr_polygon_job* job, const mr_polygon_rings* rings,
+                                   const mr_polygon_indices* indices) {
+    if (!ctx || !job || !indices || !indices->idx_out) return MR_E_BADARG;
+    if (reinterpret_cast<uintptr_t>(indices->idx_out) & 3u) return mr_fail(ctx, MR_E_BADARG, "polygons: idx_out must be 4-byte aligned");
+    return triangulate_common(ctx, job, true, rings, indices);
 }
 
 int mr_selftest_crossing(mr_context* ctx, const float* q, uint64_t count, int8_t* sign_out) {

@@ -33,9 +33,10 @@ enum mr_slot {
     MR_SLOT_EC_WORK, // ear-clip work list (apart from MR_SLOT_WORK, so the tier counts survive an ear-clip call)
     MR_SLOT_FR,      // first_ring
     MR_SLOT_RS,      // ring_start
+    MR_SLOT_IDX,     // polygon index buffers (mr_triangulate_earclip_indexed)
     MR_NUM_SCRATCH
 };
-static_assert(MR_NUM_SCRATCH == 16, "scratch slot count");
+static_assert(MR_NUM_SCRATCH == 17, "scratch slot count");
 
 constexpr int MR_NUM_AUX = 12;
 
@@ -236,6 +237,9 @@ int mr_triangulate_earclip_impl(mr_context* ctx, const mr_polygon_job* job);
 int mr_selftest_orient_impl(mr_context* ctx, const float* abc, uint64_t count, int8_t* sign_out);
 int mr_triangulate_earclip_holes_impl(mr_context* ctx, const mr_polygon_job* job, const mr_polygon_rings* rings);
 int mr_selftest_crossing_impl(mr_context* ctx, const float* q, uint64_t count, int8_t* sign_out);
+// rings == nullptr: the polygons of mr_triangulate_earclip; job->vtx_out may be null
+int mr_triangulate_earclip_indexed_impl(mr_context* ctx, const mr_polygon_job* job, const mr_polygon_rings* rings,
+                                        const mr_polygon_indices* indices);
 // out[0..npoly]: exclusive prefix sum of max(N + 2H - sub, 0) with H as for mr_polygon_offsets_rings (triangulate.cu;
 // sub 2: first_tri, sub 0: the merged ring sizes the ear-clip size classes key on); device pointers
 int mr_polygon_ring_counts(mr_context* ctx, const uint64_t* first_point, const uint64_t* first_ring, uint32_t npoly,

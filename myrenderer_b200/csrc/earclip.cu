@@ -6,6 +6,8 @@
 // is warp-uniform (every lane holds the same cursor); the blocker scan of a candidate runs lane-parallel over the list
 // of non-convex vertices, behind an exact bounding-box reject.  mr_triangulate_earclip_holes first bridges a polygon's
 // holes into its outer ring in the same workspace (merge_holes) and then runs the same ring walk on the merged ring.
+// mr_triangulate_earclip_indexed runs the same walks in instantiations of their own that also (or, without a vertex
+// buffer, only) store each triangle's three point indices.
 #include "common.cuh"
 
 namespace {
@@ -15,8 +17,10 @@ constexpr int EC_CLASSES = 4;
 __host__ __device__ constexpr uint32_t ec_nmax(int c) { return c == 0 ? 64u : c == 1 ? 256u : c == 2 ? 1024u : MR_MAX_POLYGON_POINTS; }
 // warps per block: the 4096-point class fits three 61 KB workspaces per SM
 __host__ __device__ constexpr int ec_wpb(int c) { return c == EC_CLASSES - 1 ? 3 : 4; }
-// per warp: xy 8 B | prev 2 B | next 2 B | blocker list 2 B | flags 1 B, per point (15 * nmax is a multiple of 16)
-__host__ __device__ constexpr size_t ec_ws_bytes(uint32_t nmax) { return (size_t)nmax * 15u; }
+// per warp: xy 8 B | prev 2 B | next 2 B | blocker list 2 B [| position -> point id map 2 B] | flags 1 B, per point (15
+// and 17 times nmax are multiples of 16).  Only the indexed holes instantiation keeps the map: there the clip reuses the
+// blocker list that merge_holes built the merged ring's point ids in; in every other one position = id.
+__host__ __device__ constexpr size_t ec_ws_bytes(uint32_t nmax, bool map = false) { return (size_t)nmax * (map ? 17u : 15u); }
 
 constexpr uint8_t F_NONCONVEX = 1;  // s * orient(prev, v, next) <= 0 in the current ring
 constexpr uint8_t F_REMOVED = 2;    // clipped
@@ -44,6 +48,12 @@ struct RingArgs {
     const uint64_t* first_ring;
     uint64_t ring_base;
     const uint64_t* ring_start;
+};
+
+// index output of mr_triangulate_earclip_indexed (device pointer)
+struct IdxArgs {
+    uint32_t* idx_out;
+    uint64_t index_base;
 };
 
 // ---- exact orientation ---------------------------------------------------------------------------------------
@@ -138,23 +148,52 @@ __device__ bool is_ear(const Ring& R, uint32_t p, uint32_t c, uint32_t q, int s,
     return true;
 }
 
-struct Emit {
+// What the indexed instantiations add to Emit: the polygon's index range, the index of its point 0, the position ->
+// point id map of a merged ring (null: position = id) and whether there is a vertex buffer (warp-uniform).  Empty
+// otherwise, so that Emit<false> is the plain emitter.
+template <bool IDX>
+struct EmitIdx {
+    static constexpr bool vtx = true;
+};
+template <>
+struct EmitIdx<true> {
+    uint32_t* idx;
+    uint32_t ibase;
+    MR_SPAN(uint16_t) map;
+    bool vtx;
+};
+
+template <bool IDX>
+struct Emit : EmitIdx<IDX> {
     Sink sink;
     uint32_t cap_tri, t;
     float mn, mx, lasty;
-    // triangle (x0, x1, x2) as the next one of the polygon; lanes 0..2 store its vertices
+    // triangle (x0, x1, x2) as the next one of the polygon; lanes 0..2 store its vertices and indices
     __device__ __forceinline__ void tri(const Ring& R, uint32_t x0, uint32_t x1, uint32_t x2, uint32_t lane) {
         const float2 v0 = R.P[x0], v1 = R.P[x1], v2 = R.P[x2];
         mn = fmin_acc(fmin_acc(fmin_acc(mn, v0.x), v1.x), v2.x);
         mx = fmax_acc(fmax_acc(fmax_acc(mx, v0.x), v1.x), v2.x);
         lasty = v2.y;
-        if (t < cap_tri && lane < 3u) sink.write(3u * t + lane, lane == 0u ? v0 : lane == 1u ? v1 : v2);
+        if (t < cap_tri && lane < 3u) {
+            if (this->vtx) sink.write(3u * t + lane, lane == 0u ? v0 : lane == 1u ? v1 : v2);
+            if constexpr (IDX) {
+                const uint32_t x = lane == 0u ? x0 : lane == 1u ? x1 : x2;
+                this->idx[3u * t + lane] = this->ibase + (MR_SPAN_IS_NULL(this->map) ? x : (uint32_t)this->map[x]);
+            }
+        }
         ++t;
+    }
+    // zero the range from vertex / index k0 on
+    __device__ __forceinline__ void zero_from(uint32_t k0, uint32_t lane) {
+        if (this->vtx) sink.zero(k0, sink.cap_vtx, lane);
+        if constexpr (IDX)
+            for (uint32_t k = k0 + lane; k < sink.cap_vtx; k += 32) this->idx[k] = 0u;
     }
 };
 
 // Runs the ring walk of one valid polygon (3 <= n, finite points loaded into R.P); returns MR_POLY_NO_EAR or 0.
-__device__ uint32_t clip_ring(const Ring& R, uint32_t n, Emit& em, uint32_t lane) {
+template <class EM>
+__device__ uint32_t clip_ring(const Ring& R, uint32_t n, EM& em, uint32_t lane) {
     // winding s from the lowest point (first index smallest in (y, x)) and its nearest distinct neighbours
     uint32_t m = 0;
     for (uint32_t i = lane; i < n; i += 32)
@@ -495,16 +534,24 @@ __device__ uint32_t ring_status(const EcArgs& a, const RingArgs& rg, uint32_t pi
     return __all_sync(0xFFFFFFFFu, ok) ? MR_POLY_OK : MR_POLY_DEGENERATE;
 }
 
-// One polygon of mr_triangulate_earclip (HOLES false; rg unused) or mr_triangulate_earclip_holes.
-template <bool HOLES>
-__device__ void earclip_polygon(const EcArgs& a, const RingArgs& rg, uint32_t pi, const Ring& R, uint32_t lane) {
+// One polygon of mr_triangulate_earclip (HOLES false; rg unused) or mr_triangulate_earclip_holes; with IDX, of
+// mr_triangulate_earclip_indexed (map: the position -> point id map of the holes case; ix and map unused otherwise).
+template <bool HOLES, bool IDX>
+__device__ void earclip_polygon(const EcArgs& a, const RingArgs& rg, const IdxArgs& ix, MR_SPAN(uint16_t) map, uint32_t pi,
+                                const Ring& R, uint32_t lane) {
     const uint64_t p0 = a.first_point[pi] - a.point_base;
     const uint64_t np64 = a.first_point[pi + 1] - a.first_point[pi];
     const uint64_t t0 = a.first_tri[pi] - a.tri_base;
     const uint32_t cap_tri = (uint32_t)(a.first_tri[pi + 1] - a.first_tri[pi]);
     const uint32_t n = (uint32_t)(np64 > 0xFFFFFFFFull ? 0xFFFFFFFFull : np64);
 
-    Emit em;
+    Emit<IDX> em;
+    if constexpr (IDX) {
+        em.idx = ix.idx_out + t0 * 3u;
+        em.ibase = (uint32_t)(a.first_point[pi] - ix.index_base);
+        em.map = HOLES ? map : MR_SPAN_NULL(uint16_t);
+        em.vtx = a.vtx_out != nullptr;
+    }
     em.sink.base = a.vtx_out + t0 * 3u * a.stride;
     em.sink.cap_vtx = cap_tri * 3u;
     em.sink.stride = a.stride;
@@ -547,6 +594,10 @@ __device__ void earclip_polygon(const EcArgs& a, const RingArgs& rg, uint32_t pi
                     status = merge_holes(R, src, n, H, hs, lane);
                     L = n + 2u * H;
                 }
+                if constexpr (IDX) {  // keep the merged ring's point ids through the clip, which reuses R.lst
+                    for (uint32_t k = lane; k < L; k += 32) map[k] = H ? R.lst[k] : (uint16_t)k;
+                    __syncwarp();
+                }
             }
             status |= clip_ring(R, L, em, lane);
             const uint32_t T = L - 2u;
@@ -554,13 +605,13 @@ __device__ void earclip_polygon(const EcArgs& a, const RingArgs& rg, uint32_t pi
             if (T > cap_tri) status |= MR_POLY_OVERFLOW;
             if (T < cap_tri) {
                 status |= MR_POLY_UNDERFILL;
-                em.sink.zero(3u * T, em.sink.cap_vtx, lane);
+                em.zero_from(3u * T, lane);
             }
             b1y = fmin_acc(em.mn, em.lasty);
             b2y = fmax_acc(em.mx, em.lasty);
         }
     }
-    if (status & (MR_POLY_DEGENERATE | MR_POLY_TOO_LARGE | MR_POLY_NONFINITE)) em.sink.zero(0, em.sink.cap_vtx, lane);
+    if (status & (MR_POLY_DEGENERATE | MR_POLY_TOO_LARGE | MR_POLY_NONFINITE)) em.zero_from(0, lane);
     if (lane == 0) {
         if (a.status_out) a.status_out[pi] = status;
         if (a.ntri_out) a.ntri_out[pi] = ntri;
@@ -570,18 +621,20 @@ __device__ void earclip_polygon(const EcArgs& a, const RingArgs& rg, uint32_t pi
 
 // size class C: polygons of ec_nmax(C-1)+1 .. ec_nmax(C) points (class 0 also takes every invalid size); with holes the
 // size is that of the merged ring, N + 2H
-template <bool HOLES, int C>
-__device__ __forceinline__ void earclip_class(const EcArgs& a, const RingArgs& rg) {
+template <bool HOLES, bool IDX, int C>
+__device__ __forceinline__ void earclip_class(const EcArgs& a, const RingArgs& rg, const IdxArgs& ix) {
     extern __shared__ __align__(16) unsigned char smem[];
     constexpr uint32_t NMAX = ec_nmax(C);
+    constexpr bool MAP = HOLES && IDX;
     const uint32_t lane = threadIdx.x & 31u;
-    unsigned char* ws = smem + (size_t)(threadIdx.x >> 5) * ec_ws_bytes(NMAX);
+    unsigned char* ws = smem + (size_t)(threadIdx.x >> 5) * ec_ws_bytes(NMAX, MAP);
     Ring R;
     R.P = MR_MAKE_SPAN(float2, reinterpret_cast<float2*>(ws), NMAX);
     R.prv = MR_MAKE_SPAN(uint16_t, reinterpret_cast<uint16_t*>(ws + 8u * NMAX), NMAX);
     R.nxt = MR_MAKE_SPAN(uint16_t, reinterpret_cast<uint16_t*>(ws + 10u * NMAX), NMAX);
     R.lst = MR_MAKE_SPAN(uint16_t, reinterpret_cast<uint16_t*>(ws + 12u * NMAX), NMAX);
-    R.flg = MR_MAKE_SPAN(uint8_t, ws + 14u * NMAX, NMAX);
+    R.flg = MR_MAKE_SPAN(uint8_t, ws + (MAP ? 16u : 14u) * NMAX, NMAX);
+    MR_SPAN(uint16_t) map = MAP ? MR_MAKE_SPAN(uint16_t, reinterpret_cast<uint16_t*>(ws + 14u * NMAX), NMAX) : MR_SPAN_NULL(uint16_t);
     const uint32_t begin = C == EC_CLASSES - 1 ? 0u : a.cursor[NMAX + 1u];
     const uint32_t end = a.cursor[C == 0 ? 0u : ec_nmax(C - 1) + 1u];
     for (;;) {
@@ -589,17 +642,29 @@ __device__ __forceinline__ void earclip_class(const EcArgs& a, const RingArgs& r
         if (lane == 0) idx = atomicAdd(&a.queue_head[C], 1u);
         idx = __shfl_sync(0xFFFFFFFFu, idx, 0);
         if (idx >= end - begin) break;
-        earclip_polygon<HOLES>(a, rg, a.order[begin + idx], R, lane);
+        earclip_polygon<HOLES, IDX>(a, rg, ix, map, a.order[begin + idx], R, lane);
         __syncwarp();
     }
 }
 
 template <int C>
-__global__ void __launch_bounds__(ec_wpb(C) * 32) earclip_k(const EcArgs a) { earclip_class<false, C>(a, RingArgs{}); }
+__global__ void __launch_bounds__(ec_wpb(C) * 32) earclip_k(const EcArgs a) { earclip_class<false, false, C>(a, RingArgs{}, IdxArgs{}); }
 
 template <int C>
 __global__ void __launch_bounds__(ec_wpb(C) * 32) earclip_holes_k(const EcArgs a, const RingArgs rg) {
-    earclip_class<true, C>(a, rg);
+    earclip_class<true, false, C>(a, rg, IdxArgs{});
+}
+
+// at the 72 registers earclip_k<0..2> compiles to, 7 blocks per SM (the occupancy the latency-bound ring walk needs);
+// class 3 is held to one block per SM by its workspace
+template <int C>
+__global__ void __launch_bounds__(ec_wpb(C) * 32, C == EC_CLASSES - 1 ? 1 : 7) earclip_idx_k(const EcArgs a, const IdxArgs ix) {
+    earclip_class<false, true, C>(a, RingArgs{}, ix);
+}
+
+template <int C>
+__global__ void __launch_bounds__(ec_wpb(C) * 32) earclip_holes_idx_k(const EcArgs a, const RingArgs rg, const IdxArgs ix) {
+    earclip_class<true, true, C>(a, rg, ix);
 }
 
 __global__ void __launch_bounds__(256) selftest_orient_k(const float* __restrict__ abc, uint64_t count, int8_t* __restrict__ out) {
@@ -617,19 +682,26 @@ __global__ void __launch_bounds__(256) selftest_crossing_k(const float* __restri
     }
 }
 
-// rg == nullptr: mr_triangulate_earclip
+// rg == nullptr: without holes; ix == nullptr: without indices
 template <int C>
-int launch_class(mr_context* ctx, const EcArgs& a, const RingArgs* rg, uint32_t npoly) {
+int launch_class(mr_context* ctx, const EcArgs& a, const RingArgs* rg, const IdxArgs* ix, uint32_t npoly) {
     const int wpb = ec_wpb(C);
-    const size_t smem = (size_t)wpb * ec_ws_bytes(ec_nmax(C));
-    const void* fn = rg ? reinterpret_cast<const void*>(earclip_holes_k<C>) : reinterpret_cast<const void*>(earclip_k<C>);
+    const size_t smem = (size_t)wpb * ec_ws_bytes(ec_nmax(C), rg && ix);
+    const void* fn = ix ? (rg ? reinterpret_cast<const void*>(earclip_holes_idx_k<C>) : reinterpret_cast<const void*>(earclip_idx_k<C>))
+                        : (rg ? reinterpret_cast<const void*>(earclip_holes_k<C>) : reinterpret_cast<const void*>(earclip_k<C>));
     MR_CUDA(ctx, cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 0;
     MR_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, wpb * 32, smem));
     uint64_t grid = (uint64_t)ctx->sm_count * (per_sm < 1 ? 1 : per_sm);
     const uint64_t need = ((uint64_t)npoly + wpb - 1) / wpb;
     if (need < grid) grid = need;
-    if (rg) {
+    if (ix && rg) {
+        earclip_holes_idx_k<C><<<(unsigned)grid, wpb * 32, smem, ctx->stream>>>(a, *rg, *ix);
+        MR_LAUNCH_CHECK(ctx, "earclip_holes_idx_k");
+    } else if (ix) {
+        earclip_idx_k<C><<<(unsigned)grid, wpb * 32, smem, ctx->stream>>>(a, *ix);
+        MR_LAUNCH_CHECK(ctx, "earclip_idx_k");
+    } else if (rg) {
         earclip_holes_k<C><<<(unsigned)grid, wpb * 32, smem, ctx->stream>>>(a, *rg);
         MR_LAUNCH_CHECK(ctx, "earclip_holes_k");
     } else {
@@ -641,8 +713,8 @@ int launch_class(mr_context* ctx, const EcArgs& a, const RingArgs* rg, uint32_t 
 }  // namespace
 
 namespace {
-int earclip_run(mr_context* ctx, const mr_polygon_job* j, const mr_polygon_rings* rings) {
-    // all pointers in *j and *rings are device pointers here (staging happened in api.cu)
+int earclip_run(mr_context* ctx, const mr_polygon_job* j, const mr_polygon_rings* rings, const mr_polygon_indices* indices) {
+    // all pointers in *j, *rings and *indices are device pointers here (staging happened in api.cu)
     const uint32_t npoly = j->npoly;
     if (npoly == 0) return MR_OK;
     // work list: hist | cursor | class ranges of the reference path (unused) | queue heads | order [| merged sizes].  A
@@ -680,25 +752,39 @@ int earclip_run(mr_context* ctx, const mr_polygon_job* j, const mr_polygon_rings
     a.bbox_out = j->bbox_out;
     a.status_out = j->status_out;
     a.ntri_out = j->ntri_out;
-    sink_layout(a, j->layout, a.vtx_out);
+    if (a.vtx_out) {
+        sink_layout(a, j->layout, a.vtx_out);
+    } else {  // indices only: the layout is not read
+        a.stride = a.off_x = 0;
+        a.off_c = 0xFFFFFFFFu;
+        a.fast32 = 0;
+    }
     a.order = order;
     a.cursor = cursor;
     a.queue_head = heads;
     RingArgs rg{};
     if (rings) rg = RingArgs{rings->first_ring, rings->ring_base, rings->ring_start};
     const RingArgs* rp = rings ? &rg : nullptr;
+    IdxArgs ix{};
+    if (indices) ix = IdxArgs{indices->idx_out, indices->index_base};
+    const IdxArgs* xp = indices ? &ix : nullptr;
     // largest class first
-    if ((rc = launch_class<3>(ctx, a, rp, npoly))) return rc;
-    if ((rc = launch_class<2>(ctx, a, rp, npoly))) return rc;
-    if ((rc = launch_class<1>(ctx, a, rp, npoly))) return rc;
-    return launch_class<0>(ctx, a, rp, npoly);
+    if ((rc = launch_class<3>(ctx, a, rp, xp, npoly))) return rc;
+    if ((rc = launch_class<2>(ctx, a, rp, xp, npoly))) return rc;
+    if ((rc = launch_class<1>(ctx, a, rp, xp, npoly))) return rc;
+    return launch_class<0>(ctx, a, rp, xp, npoly);
 }
 }  // namespace
 
-int mr_triangulate_earclip_impl(mr_context* ctx, const mr_polygon_job* j) { return earclip_run(ctx, j, nullptr); }
+int mr_triangulate_earclip_impl(mr_context* ctx, const mr_polygon_job* j) { return earclip_run(ctx, j, nullptr, nullptr); }
 
 int mr_triangulate_earclip_holes_impl(mr_context* ctx, const mr_polygon_job* j, const mr_polygon_rings* rings) {
-    return earclip_run(ctx, j, rings);
+    return earclip_run(ctx, j, rings, nullptr);
+}
+
+int mr_triangulate_earclip_indexed_impl(mr_context* ctx, const mr_polygon_job* j, const mr_polygon_rings* rings,
+                                        const mr_polygon_indices* indices) {
+    return earclip_run(ctx, j, rings, indices);
 }
 
 int mr_selftest_crossing_impl(mr_context* ctx, const float* q, uint64_t count, int8_t* sign_out) {

@@ -23,7 +23,8 @@ from typing import Callable, Optional, Sequence
 import numpy as np
 
 from . import _capi as capi
-from ._capi import MrError, MrLayout, MrPolygonJob, MrPolygonRings, MrTerrainJob, MrTerrainParams
+from ._capi import (MrDrawIndexedRange, MrError, MrLayout, MrPolygonIndices, MrPolygonJob, MrPolygonRings, MrTerrainJob,
+                    MrTerrainParams)
 
 try:  # torch is plumbing (device memory, streams); numpy host arrays work without it
     import torch
@@ -270,16 +271,27 @@ class PolygonBatch:
     npoly: int
     first_point: np.ndarray         # host copy, npoly+1
     first_tri: np.ndarray           # host copy, npoly+1
-    vertex_buffer: object           # device bytes, 3*first_tri[-1]*stride
+    vertex_buffer: object           # device bytes, 3*first_tri[-1]*stride (None for output="indices")
     bbox: object                    # device f32 [npoly,4]
     status: object                  # device u32 [npoly]
     ntri: object                    # device u32 [npoly]
     layout: VertexLayout
+    index_buffer: object = None     # device u32 [3*first_tri[-1]] (output="indices" / "both"): rows of xy
+    index_base: int = 0             # first_point[0]: index k is row k of the xy the batch was made from
 
     def draw_range(self, i: int) -> VertexBuffer:
         """VertexBuffer.new(offset, primitive_count) for polygon i inside the packed buffer."""
         prims = int(self.first_tri[i + 1] - self.first_tri[i])
         return VertexBuffer(self.vertex_buffer, prims * 3, 1, int(self.first_tri[i]) * 3, 0)
+
+    def draw_indexed_range(self, i: int) -> MrDrawIndexedRange:
+        """drawIndexed's arguments for polygon i inside index_buffer (mr_polygon_draw_indexed_range)."""
+        out = MrDrawIndexedRange()
+        rc = capi.load().mr_polygon_draw_indexed_range(int(self.first_tri[i]), int(self.first_tri[i + 1]),
+                                                       int(self.first_tri[0]), C.byref(out))
+        if rc != 0:
+            raise MrError(rc, "mr_polygon_draw_indexed_range")
+        return out
 
 
 @dataclass
@@ -309,6 +321,7 @@ def polygon_offsets_rings_host(first_point: np.ndarray, first_ring: np.ndarray) 
 
 
 _ALGORITHMS = {"reference": "mr_triangulate_batch", "earclip": "mr_triangulate_earclip"}
+_OUTPUTS = ("vertices", "indices", "both")
 
 
 def _check_algorithm(algorithm, offset_prime):
@@ -335,11 +348,20 @@ class Polygon:
         j.bbox_out, j.status_out, j.ntri_out = _ptr(bbox_out), _ptr(status_out), _ptr(ntri_out)
         return j
 
-    def triangulate(self, job: MrPolygonJob, algorithm: str = "reference", rings: Optional[MrPolygonRings] = None):
+    def triangulate(self, job: MrPolygonJob, algorithm: str = "reference", rings: Optional[MrPolygonRings] = None,
+                    indices: Optional[MrPolygonIndices] = None):
         """algorithm "reference": mr_triangulate_batch (the reference's triangulator, for parity); "earclip":
         mr_triangulate_earclip (correct on every simple polygon, same output format), or with `rings`
-        mr_triangulate_earclip_holes (polygons with holes)."""
+        mr_triangulate_earclip_holes (polygons with holes).  With `indices` (earclip only):
+        mr_triangulate_earclip_indexed, which also writes point indices and takes a NULL vtx_out."""
         _check_algorithm(algorithm, None)
+        if indices is not None:
+            if algorithm != "earclip":
+                raise ValueError("indexed output is written by the earclip algorithm only")
+            self.ctx.check(self.ctx.lib.mr_triangulate_earclip_indexed(
+                self.ctx.handle, C.byref(job), None if rings is None else C.byref(rings), C.byref(indices)),
+                "mr_triangulate_earclip_indexed")
+            return
         if rings is not None:
             if algorithm != "earclip":
                 raise ValueError("holes are triangulated by the earclip algorithm only")
@@ -350,14 +372,20 @@ class Polygon:
         self.ctx.check(getattr(self.ctx.lib, name)(self.ctx.handle, C.byref(job)), name)
 
     def create_polygons(self, xy, first_point, *, offset_prime=None, seed=0, poly_index0=0,
-                        device="cuda", algorithm="reference", rings=None) -> PolygonBatch:
+                        device="cuda", algorithm="reference", rings=None, output="vertices") -> PolygonBatch:
         """Batched create_polygon.  xy: [npts,2] f32 (numpy or cuda tensor); first_point: npoly+1 offsets.
         algorithm: "reference" or "earclip" (see triangulate); ear clipping takes no offset_prime.
         rings = (first_ring, ring_start): polygons with holes (earclip only), as mr_polygon_rings with ring_base
-        first_ring[0]; polygon i then gets N + 2H - 2 triangles."""
+        first_ring[0]; polygon i then gets N + 2H - 2 triangles.
+        output: "vertices" (vertex_buffer), "indices" (index_buffer: three u32 per triangle, rows of xy, so xy itself
+        is the vertex buffer to draw them with) or "both"; anything but "vertices" needs the earclip algorithm."""
         _check_algorithm(algorithm, offset_prime)
         if rings is not None and algorithm != "earclip":
             raise ValueError("holes are triangulated by the earclip algorithm only")
+        if output not in _OUTPUTS:
+            raise ValueError(f"output must be one of {_OUTPUTS}, not {output!r}")
+        if output != "vertices" and algorithm != "earclip":
+            raise ValueError("indexed output is written by the earclip algorithm only")
         fp_host = np.ascontiguousarray(
             first_point.cpu().numpy() if _is_cuda(first_point) else first_point, dtype=np.uint64)
         npoly = len(fp_host) - 1
@@ -385,15 +413,20 @@ class Polygon:
                 raise ValueError("offset_prime must hold 2*npoly values")
             op_d = torch.from_numpy(op.view(np.int32)).to(dev)
         ntri = int(ft_host[-1])
-        vtx = torch.empty(max(ntri * 3 * self.layout.stride, 32), dtype=torch.uint8, device=dev)
+        vtx = idx = ix = None
+        if output != "indices":
+            vtx = torch.empty(max(ntri * 3 * self.layout.stride, 32), dtype=torch.uint8, device=dev)
+        if output != "vertices":
+            idx = torch.empty(max(ntri * 3, 1), dtype=torch.uint32, device=dev)
+            ix = MrPolygonIndices(_ptr(idx), int(fp_host[0]))
         bbox = torch.empty((npoly, 4), dtype=torch.float32, device=dev)
         status = torch.empty(npoly, dtype=torch.int32, device=dev)
         nt = torch.empty(npoly, dtype=torch.int32, device=dev)
         self.triangulate(self.job(xy_d, fp_d, npoly, vtx_out=vtx, first_tri=ft_d, bbox_out=bbox,
                                   status_out=status, ntri_out=nt, offset_prime=op_d, seed=seed,
-                                  poly_index0=poly_index0, point_base=int(fp_host[0])), algorithm, rg)
-        return PolygonBatch(npoly, fp_host, ft_host, vtx[: ntri * 3 * self.layout.stride], bbox, status, nt,
-                            self.layout)
+                                  poly_index0=poly_index0, point_base=int(fp_host[0])), algorithm, rg, ix)
+        return PolygonBatch(npoly, fp_host, ft_host, None if vtx is None else vtx[: ntri * 3 * self.layout.stride],
+                            bbox, status, nt, self.layout, None if idx is None else idx[: ntri * 3], int(fp_host[0]))
 
     def create_polygon(self, vertices, *, offset_prime=None, seed=0, index=0, algorithm="reference",
                        holes=None) -> PolygonObj:

@@ -168,6 +168,15 @@ struct PolygonObj {
     uint32_t status = 0, ntri = 0;
 };
 
+// A polygon as points plus an index buffer (mr_triangulate_earclip_indexed): bind `points` as a float32x2 vertex buffer
+// and draw `indices` with drawIndexed.
+struct IndexedPolygonObj {
+    std::vector<Point> points;      // the outer ring, then each hole
+    std::vector<uint32_t> indices;  // three per triangle, into points
+    float bounding_box_p0[3]{}, bounding_box_p1[3]{};
+    uint32_t status = 0, ntri = 0;
+};
+
 class Polygon {
    public:
     explicit Polygon(Context& ctx) : ctx_(ctx), layout_(gpu_vertex_layout()) {}
@@ -256,6 +265,39 @@ class Polygon {
         j.ntri_out = &o.ntri;
         const mr_polygon_rings rings{first_ring, 0, ring_start.data()};
         ctx_.check(mr_triangulate_earclip_holes(ctx_.get(), &j, &rings), "mr_triangulate_earclip_holes");
+        o.bounding_box_p0[0] = bbox[0];
+        o.bounding_box_p0[1] = bbox[1];
+        o.bounding_box_p1[0] = bbox[2];
+        o.bounding_box_p1[1] = bbox[3];
+        return o;
+    }
+    // The same polygon with holes as points plus indices (mr_triangulate_earclip_indexed, no vertex buffer).
+    IndexedPolygonObj create_polygon_earclip_indexed(const std::vector<Point>& outer, const std::vector<std::vector<Point>>& holes) {
+        IndexedPolygonObj o;
+        o.points = outer;
+        std::vector<uint64_t> ring_start{0};
+        for (const auto& h : holes) {
+            ring_start.push_back(o.points.size());
+            o.points.insert(o.points.end(), h.begin(), h.end());
+        }
+        if (o.points.size() < 2) throw Error(MR_E_BADARG, "create_polygon: vertices.len - 2 underflows (Polygon.zig:82)");
+        const uint64_t n = o.points.size(), ntri = n + 2 * holes.size() - 2;
+        o.indices.assign(3 * ntri, 0);
+        const uint64_t first_point[2] = {0, n};
+        const uint64_t first_tri[2] = {0, ntri};
+        const uint64_t first_ring[2] = {0, ring_start.size()};
+        float bbox[4];
+        mr_polygon_job j{};
+        j.xy = reinterpret_cast<const float*>(o.points.data());
+        j.first_point = first_point;
+        j.npoly = 1;
+        j.first_tri = first_tri;
+        j.bbox_out = bbox;
+        j.status_out = &o.status;
+        j.ntri_out = &o.ntri;
+        const mr_polygon_rings rings{first_ring, 0, ring_start.data()};
+        const mr_polygon_indices indices{o.indices.data(), 0};
+        ctx_.check(mr_triangulate_earclip_indexed(ctx_.get(), &j, &rings, &indices), "mr_triangulate_earclip_indexed");
         o.bounding_box_p0[0] = bbox[0];
         o.bounding_box_p0[1] = bbox[1];
         o.bounding_box_p1[0] = bbox[2];

@@ -60,6 +60,15 @@ pub const PolygonRings = extern struct {
     ring_start: [*]const u64,
 };
 
+// mr_polygon_indices: where mr_triangulate_earclip_indexed writes three u32 point indices per triangle
+pub const PolygonIndices = extern struct {
+    idx_out: [*]u32,
+    index_base: u64,
+};
+
+// mr_draw_indexed_range: drawIndexed's arguments for one polygon (IndexedDraw.zig's IndexBuffer)
+pub const DrawIndexedRange = extern struct { index_count: u32, instance_count: u32, first_index: u32, base_vertex: i32, first_instance: u32 };
+
 pub extern fn mr_context_create(device: c_int, ctx_out: *?*Context) c_int;
 pub extern fn mr_context_destroy(ctx: ?*Context) c_int;
 pub extern fn mr_sync(ctx: ?*Context) c_int;
@@ -72,6 +81,8 @@ pub extern fn mr_triangulate_batch(ctx: ?*Context, job: *const PolygonJob) c_int
 pub extern fn mr_triangulate_earclip(ctx: ?*Context, job: *const PolygonJob) c_int;
 pub extern fn mr_triangulate_earclip_holes(ctx: ?*Context, job: *const PolygonJob, rings: *const PolygonRings) c_int;
 pub extern fn mr_polygon_draw_range(first_tri_i: u64, first_tri_next: u64, tri_base: u64, out: *DrawRange) c_int;
+pub extern fn mr_triangulate_earclip_indexed(ctx: ?*Context, job: *const PolygonJob, rings: ?*const PolygonRings, indices: *const PolygonIndices) c_int;
+pub extern fn mr_polygon_draw_indexed_range(first_tri_i: u64, first_tri_next: u64, tri_base: u64, out: *DrawIndexedRange) c_int;
 pub extern fn mr_unirand_seed_host(top: u32, seed: u64, index: u64, offset_out: *u32, prime_out: *u32) c_int;
 pub extern fn mr_context_trim(ctx: ?*Context) c_int;
 pub extern fn mr_pinned_alloc(ctx: ?*Context, bytes: usize, host_out: *?*anyopaque) c_int;
